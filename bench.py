@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — policy-update throughput of the B200-native GeometryRL hot path.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config NAME]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config NAME] [--dump-outputs DIR]
 
 A "step" is one minibatch iteration of examples/torchrl/train.py:259-316 on synthetic rollout frames of the
 config's graph shape: policy forward (graph features -> EMPN/HEPi/transformer -> Gaussian head), TRPL
@@ -12,11 +12,22 @@ step fed from pinned HOST memory with a loss read back, `roofline` = the dominan
 8(d) accounting) / CUDA-event duration against MEASURED_PEAKS.json, `cpu_baseline` = the CPU oracle port of the same
 step on this box's host cores (bounded sample), `configs` = the other message-passing workloads, device-timed.
 
+The minibatches are drawn from fixed seeds on the host without running the model (`nominal_policy_output`), so every
+build of the project times and computes on the same inputs.  The starting parameters are seeded too, then calibrated
+by the policy's first training-mode forward, which runs the kernels under test (the reference's conv.py:104-105 rule).
+
+`--dump-outputs DIR` writes, as .npy files, the parameters the timed path started from right after that calibration
+(`init.<actor|critic>.<parameter>.npy`) and what its last timed step produced: the losses and metrics it returns
+(`out.<name>.npy`), the gradients it applied (`grad.<actor|critic>.<parameter>.npy`) and the parameters it left
+(`param.<actor|critic>.<parameter>.npy`).  Two builds run with the same arguments can be compared file by file; equal
+`init.*` files confirm that they started from the same state.
+
 `--impl reference` times that CPU port alone (the reference itself is pure Python on top of torchrl / PyG /
 ITPAL wheels that are not installable offline, so it cannot run unmodified here; see DESIGN.md)."""
 import argparse
 import json
 import os
+import re
 import subprocess
 import sys
 import threading
@@ -25,6 +36,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 # BASELINE.json's metric is "HEPi fwd+bwd+TRPL update samples/sec" and BASELINE.md section 4 names config 1
@@ -41,7 +53,6 @@ DEFAULT_MINIBATCH = {"rigid_insertion_multi_hepi_trpl_cfg": 8192, "rigid_pushing
 SIDE_WORKLOADS = [("rigid_insertion_multi_hepi_trpl_cfg", 1000), ("rigid_pushing_multi_empn_trpl_cfg", 4096),
                   ("cloth_hanging_multi_hepi_trpl_cfg", 8192), ("rope_shaping_hepi_trpl_cfg", 2048),
                   ("rigid_insertion_two_agents_multi_transformer_trpl_cfg", 1000)]
-MIN_TIMED_STEPS = 200  # the K-step timed region is repeated until at least this many steps were timed; median region reported
 METRIC = "fwd+bwd+TRPL update samples/sec (policy fwd+bwd, TRPL projection, losses, critic, Adam)"  # BASELINE.json metric
 N_ROTATE = 8  # distinct minibatches cycled through the timed region
 _emit = print
@@ -50,13 +61,13 @@ _emit = print
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=200, help="timed steps per region")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--config", default=DEFAULT_CONFIG)
     ap.add_argument("--minibatch", type=int, default=0, help="samples per GPU per step (default: DEFAULT_MINIBATCH, else the config's)")
     ap.add_argument("--no-side-workloads", action="store_true", help="skip the other configs reported under \"configs\"")
-    ap.add_argument("--repeats", type=int, default=0, help="timed regions of --steps steps each (default: enough for 200 steps)")
+    ap.add_argument("--repeats", type=int, default=1, help="timed regions of --steps steps each; the median region is reported")
     ap.add_argument("--cpu-sample", type=int, default=256, help="samples per CPU-baseline step")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-graph", action="store_true", help="launch the step eagerly instead of replaying a CUDA graph")
@@ -69,7 +80,14 @@ def parse():
     ap.add_argument("--precision", default="bf16", choices=["fp32", "bf16"],
                     help="nn.Linear contractions of the message-passing kernels: fp32 FFMA (parity 1e-5) or bf16 tcgen05 "
                          "tensor cores (parity 1e-2)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step of the headline workload to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1 or args.repeats < 1 or args.warmup < 0:
+        ap.error("--steps and --repeats must be at least 1, --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------
@@ -218,8 +236,49 @@ def config_block(args, cfg_name, cfg, B, world):
     """The `config` object of the JSON line; identical for our arm and the reference arm (same workload, same sizes)."""
     return {"workload": cfg_name, "body": cfg.model, "minibatch_per_gpu": B, "global_minibatch": B * world,
             "parallelism": f"dp{world}",
-            "inputs": f"{N_ROTATE} distinct synthetic minibatches rotated through the timed region; the per-step working "
-                      f"set (hundreds of MB of latents) exceeds the 126 MB L2"}
+            "inputs": f"{N_ROTATE} distinct synthetic minibatches (fixed seeds, independent of the kernels) rotated through "
+                      f"the timed region; the per-step working set (hundreds of MB of latents) exceeds the 126 MB L2"}
+
+
+def nominal_policy_output(cfg, B):
+    """(mean, variance, value) the synthetic old distribution drifts from: the freshly initialised Gaussian head's output
+    (mean 0, variance init_std**2 = 1: the initial policy's means are O(1e-2) and its variances within 2 % of 1) and a
+    zero value, as the initial critic's values are O(1e-3).  Taken from the initialisation rather than from a forward
+    pass, so that the minibatches do not depend on the kernels being measured."""
+    k = cfg.total_action_dim
+    return torch.zeros(B, k), torch.ones(B, k), torch.zeros(B, 1)
+
+
+DUMP_MAX_BYTES = 64 << 20
+
+
+def named_parameters(lrn, prefix):
+    return {f"{prefix}.{net_name}.{k}": v for net_name, net in (("actor", lrn.actor), ("critic", lrn.critic))
+            for k, v in net.named_parameters()}
+
+
+def host_arrays(tensors):
+    """Host copies keyed by `--dump-outputs` file names (float64 stays float64, everything else becomes float32)."""
+    arrays = {}
+    for k, v in tensors.items():
+        v = v.detach().cpu()
+        arrays[re.sub(r"[^A-Za-z0-9_.-]", "_", k)] = (v if v.dtype == torch.float64 else v.float()).numpy().copy()
+    if len(arrays) != len(tensors):
+        raise RuntimeError("--dump-outputs: two outputs map to the same file name")
+    return arrays
+
+
+def dump_outputs(path, arrays):
+    """DIR/<name>.npy for every array.  Above DUMP_MAX_BYTES in all, every array keeps the same fraction of its elements:
+    a fixed sample (flattened indices drawn by numpy.random.default_rng(0), in ascending order)."""
+    budget = DUMP_MAX_BYTES - 128 * len(arrays)  # .npy headers
+    frac = min(1.0, budget / sum(a.nbytes for a in arrays.values()))
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        if frac < 1.0:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, max(1, int(a.size * frac)), replace=False))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(path, f"{name}.npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -360,6 +419,7 @@ def measure(args, cfg_name, B, precision, dev, dp, rank, world, local, steps, fu
     actor, critic, projection, loss_module, adv_module = learner.build_agent(cfg, dev, seed=0)  # same init on all ranks
     lrn = learner.Learner(cfg, actor, critic, loss_module, dp=dp)
 
+    dump = full and rank == 0 and args.dump_outputs
     # ---- synthetic minibatches of this rank's environments (weak scaling: B samples per GPU) -----------
     gen = torch.Generator().manual_seed(1234 + rank)
     host_batches = []
@@ -369,10 +429,8 @@ def measure(args, cfg_name, B, precision, dev, dp, rank, world, local, steps, fu
         obs = synthetic_obs(cfg, B, gen, env_ids=env_ids)
         if i == 0:
             lrn.calibrate(to_device(obs, dev))  # one-time kernel calibration (global statistics under DP)
-        with torch.no_grad():
-            dist_ = actor.get_dist(to_device(obs, dev))
-            v = critic.module(*[obs[k].to(dev) for k in critic.in_keys])
-        mb = synthetic_minibatch(obs, dist_.mean, dist_.var_diag, v, gen)
+            init = host_arrays(named_parameters(lrn, "init")) if dump else None
+        mb = synthetic_minibatch(obs, *nominal_policy_output(cfg, B), gen)
         host_batches.append({k: t.pin_memory() for k, t in mb.items()})
     dev_batches = [to_device(b, dev) for b in host_batches]
     h2d_bytes = sum(t.numel() * t.element_size() for t in host_batches[0].values())
@@ -403,9 +461,7 @@ def measure(args, cfg_name, B, precision, dev, dp, rank, world, local, steps, fu
         step = lrn.update
     for i in range(args.warmup):
         step(dev_batches[i % N_ROTATE])
-    repeats = args.repeats or max(1, -(-MIN_TIMED_STEPS // steps))
-    if not full:
-        repeats = min(repeats, 3)
+    repeats = args.repeats if full else min(args.repeats, 3)
     sampler = ClockSampler(list(range(world)) if world > 1 else local)
     barrier()
     if rank == 0 and full:
@@ -425,10 +481,17 @@ def measure(args, cfg_name, B, precision, dev, dp, rank, world, local, steps, fu
         barrier()
         regions.append(max_over_ranks(e0.elapsed_time(e1)))
     torch.cuda.profiler.stop()
+    # the later passes below run more updates: take the timed path's last outputs now
+    outputs = None
+    if dump:
+        outputs = host_arrays({**{f"out.{k}": v for k, v in out.items() if torch.is_tensor(v)},
+                               **{f"grad.{k}": v for k, v in lrn.flat_grads().items()}, **named_parameters(lrn, "param")})
+        outputs.update(init)
     launches = launches_per_step * steps if use_graph else (_lib.launch_count - launches0) // repeats
     clocks = sampler.stop() if (rank == 0 and full) else None
     ms = sorted(regions)[len(regions) // 2]  # median K-step region (each region is exactly K steps, max over ranks)
     res = {"precision": precision, "value": B * world * steps / (ms * 1e-3), "ms_per_step": ms / steps, "steps": steps,
+           "outputs": outputs,
            "clocks": clocks, "gpu_launches": launches, "cuda_graph": use_graph, "B": B, "model": cfg.model,
            "regions_ms": [round(x, 3) for x in regions],
            # host-side cost of enqueueing one step (max over ranks of the median region): close to ms_per_step means the
@@ -577,6 +640,8 @@ def run_ours(args):
     B = resolve_minibatch(args, args.config, cfg)
 
     main_res = measure(args, args.config, B, args.precision, dev, dp, rank, world, local, args.steps)
+    if main_res["outputs"] is not None:
+        dump_outputs(args.dump_outputs, main_res["outputs"])
     # the other precision mode of the same path, measured in the same run (one region; no per-kernel pass)
     other = "fp32" if args.precision == "bf16" else "bf16"
     other_res = None

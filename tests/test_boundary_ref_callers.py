@@ -1,7 +1,7 @@
-"""CPU (build container only: needs /root/reference): the reference's OWN wrapper classes accept the repo's bodies and
-data builders — the duck-typed drop-in INTEGRATION.md section 1 describes.
+"""CPU, optional (needs a thobotics/geometry_rl checkout named by $GRL_REFERENCE): the reference's OWN wrapper classes
+accept the repo's bodies and data builders — the duck-typed drop-in INTEGRATION.md section 1 describes.
 
-The unmodified `GNNGaussianPolicyDiag` / `GNNVFNet` are imported from /root/reference through oracle/ref_shims and
+The unmodified `GNNGaussianPolicyDiag` / `GNNVFNet` are imported from that checkout through oracle/ref_shims and
 constructed around the repo's `HEPi` / `DeepSets` / `RigidTasksData` objects.  There is no GPU here, so the bodies cannot
 execute; what is checked is everything the wrapper itself touches: constructor contract (`gnn.device`), parameter
 registration (state_dict keys equal the ones the all-reference wrapper saved in the fixture), and the call protocol
@@ -14,10 +14,10 @@ import sys
 import pytest
 import torch
 
-REF = os.environ.get("GRL_REFERENCE", "/root/reference")
+REF = os.environ.get("GRL_REFERENCE", "")
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "geometry_rl")),
-                                reason="the reference checkout only exists in the build container")
+pytestmark = pytest.mark.skipif(not REF or not os.path.isdir(os.path.join(REF, "geometry_rl")),
+                                reason="set GRL_REFERENCE to a thobotics/geometry_rl checkout to run the reference's own wrappers")
 
 
 @pytest.fixture(scope="module")
