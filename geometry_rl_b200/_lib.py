@@ -98,6 +98,7 @@ class GrlReadoutDesc(C.Structure):
 
 
 READOUT_MAX_OUT = 8
+MAX_KNN = 8  # GRL_MAX_KNN: k of grl_knn_graph, max_neighbors of the radius graph
 LOSS_TERMS = 8
 LOSS_SCALARS = 16
 LOSS_STATS = 8
@@ -117,6 +118,8 @@ SIGNATURES = {
     "grl_knn_edge_ptr": (C.c_int, [_fp, C.c_int, C.c_int, C.c_int, _fp, _fp]),
     "grl_knn_graph": (C.c_int, [_fp, _fp, _fp, C.c_int, C.c_int, C.c_int, _fp, C.c_int64, _fp]),
     "grl_radius_neighbors": (C.c_int, [_fp, _fp, C.c_int, C.c_int, C.c_float, C.c_int, _fp, _fp, _fp]),
+    "grl_radius_edge_ptr": (C.c_int, [_fp, C.c_int, C.c_int, C.c_int64, _fp, _fp]),
+    "grl_radius_graph": (C.c_int, [_fp, _fp, _fp, C.c_int, C.c_int, C.c_int, _fp, C.c_int64, C.c_int64, _fp]),
     "grl_dense_edges": (C.c_int, [C.c_int, _fp, _fp, C.c_int, C.c_int, C.c_int, _fp, C.c_int64, _fp]),
     "grl_csr_build": (C.c_int, [_fp, C.c_int64, _fp, C.c_int, C.c_int, C.c_int, _fp, _fp, _fp, _fp]),
     "grl_embed_fwd": (C.c_int, [C.POINTER(GrlEmbedDesc), _fp]),

@@ -48,6 +48,8 @@ class GNNGaussianPolicyDiag(nn.Module):
         self.num_actuators = num_actuators
         self.hyper_data = hyper_data
         self.gnn = gnn
+        # fixed-capacity, in-place refreshed topology (BaseData.refresh_in_place) only for a model that consumes it
+        hyper_data.consumer_accepts_capacity = bool(getattr(gnn, "accepts_capacity_edge_sets", False))
 
     # ---- forward ---------------------------------------------------------------------------------
     def gnn_forward(self, *args, train=True):

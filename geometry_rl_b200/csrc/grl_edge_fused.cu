@@ -156,8 +156,9 @@ __global__ void __launch_bounds__(kThreads, 3) edge_fused_fwd_kernel(const GrlFu
   stage_w1_b1_b2(s.W1b, d.w1, d.b1, d.b2);
   tc::stage_weight_f16(s.W2h, d.w2, kC, kC, kC);
   tc::stage_weight_f16(s.Wkh, d.wk, kC, kC, kC);
-  // this CTA's key (dst) node range: equal cost shares
-  const long long W = 8ll * d.n_edges + d.n_key;
+  // this CTA's key (dst) node range: equal cost shares.  The edge count is read from rowptr[n_key], not n_edges: an edge
+  // set of fixed capacity (refreshed in place on the device) has n_edges = capacity and its real count only there.
+  const long long W = 8ll * __ldg(d.rowptr + d.n_key) + d.n_key;
   const int n_lo = blockIdx.x == 0 ? 0 : fused_lower_bound(d.rowptr, d.n_key, W * blockIdx.x / gridDim.x);
   const int n_hi = blockIdx.x + 1 == gridDim.x ? d.n_key : fused_lower_bound(d.rowptr, d.n_key, W * (blockIdx.x + 1) / gridDim.x);
   const int p0 = d.rowptr[n_lo], p1 = d.rowptr[n_hi];
@@ -425,7 +426,7 @@ edge_fused_bwd_ws3_kernel(const GrlFusedEdgeDesc d, const __grid_constant__ CUte
   tc::stage_weight_bf16(s.Wkb, d.wk, kC, kC, kC);
   if (tid < kC) s.b2[tid] = __ldg(d.b2 + tid);
   if (tid < 4 * kC) (&s.acc_gb2[0][0])[tid] = 0.f;
-  const long long W = 8ll * d.n_edges + d.n_key;
+  const long long W = 8ll * __ldg(d.rowptr + d.n_key) + d.n_key;  // real edge count, as in the forward
   const int n_lo = blockIdx.x == 0 ? 0 : fused_lower_bound(d.rowptr, d.n_key, W * blockIdx.x / gridDim.x);
   const int n_hi = blockIdx.x + 1 == gridDim.x ? d.n_key : fused_lower_bound(d.rowptr, d.n_key, W * (blockIdx.x + 1) / gridDim.x);
   const int p0 = d.rowptr[n_lo], p1 = d.rowptr[n_hi];

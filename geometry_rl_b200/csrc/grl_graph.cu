@@ -150,6 +150,79 @@ __global__ void __launch_bounds__(128) radius_neighbors_kernel(const float* __re
   }
 }
 
+// edge_ptr of a radius graph: count[b] = sum of cnt over graph b's P rows (rows past num_valid[b] hold 0), exclusive
+// prefix sum, every entry clamped to `capacity` (the edges of the COO buffer; the last graphs lose what does not fit).
+__global__ void radius_edge_ptr_kernel(const int32_t* __restrict__ cnt, int B, int P, int64_t capacity,
+                                       int64_t* __restrict__ edge_ptr) {
+  __shared__ long long part[1024];
+  const int tid = threadIdx.x, nt = blockDim.x;
+  const int per = (B + nt - 1) / nt;
+  const int b0 = tid * per, b1 = min(b0 + per, B);
+  long long s = 0;
+  for (int b = b0; b < b1; ++b)
+    for (int i = 0; i < P; ++i) s += cnt[(size_t)b * P + i];
+  part[tid] = s;
+  __syncthreads();
+  if (tid == 0) {
+    long long run = 0;
+    for (int i = 0; i < nt; ++i) { const long long t = part[i]; part[i] = run; run += t; }
+    edge_ptr[B] = min(run, (long long)capacity);
+  }
+  __syncthreads();
+  long long run = part[tid];
+  for (int b = b0; b < b1; ++b) {
+    edge_ptr[b] = min(run, (long long)capacity);
+    for (int i = 0; i < P; ++i) run += cnt[(size_t)b * P + i];
+  }
+}
+
+// Coalesced COO of a radius graph from the padded neighbour lists of radius_neighbors_kernel: per graph, sorted by
+// (source = neighbour j, target = centre i), like knn_graph_kernel.  Entries [edge_ptr[B], capacity) are set to 0, so
+// a gather over the whole buffer stays in bounds.
+__global__ void __launch_bounds__(128) radius_graph_kernel(const int32_t* __restrict__ nbr, const int32_t* __restrict__ cnt,
+                                                          const int64_t* __restrict__ edge_ptr, int B, int P, int max_nb,
+                                                          int64_t* __restrict__ coo, int64_t row_stride, int64_t capacity) {
+  __shared__ short snb[kMaxP * GRL_MAX_KNN];
+  __shared__ int off[kMaxP + 1];
+  const int tid = threadIdx.x;
+  for (int g = blockIdx.x; g < B; g += gridDim.x) {
+    __syncthreads();
+    for (int q = tid; q < P * max_nb; q += blockDim.x) {
+      const int i = q / max_nb, s = q - i * max_nb;
+      snb[q] = (short)(s < cnt[(size_t)g * P + i] ? nbr[(size_t)g * P * max_nb + q] : -1);
+    }
+    __syncthreads();
+    for (int j = tid; j < P; j += blockDim.x) {
+      int c = 0;
+      for (int q = 0; q < P * max_nb; ++q) c += (snb[q] == j);
+      off[j + 1] = c;
+    }
+    __syncthreads();
+    if (tid == 0) {
+      off[0] = 0;
+      for (int j = 0; j < P; ++j) off[j + 1] += off[j];
+    }
+    __syncthreads();
+    const int64_t base = edge_ptr[g], end = edge_ptr[g + 1];
+    for (int j = tid; j < P; j += blockDim.x) {
+      int64_t w = base + off[j];
+      for (int i = 0; i < P && w < end; ++i) {
+        bool hit = false;
+        for (int s = 0; s < max_nb; ++s) hit |= (snb[i * max_nb + s] == j);
+        if (hit) {
+          coo[w] = (int64_t)g * P + j;
+          coo[row_stride + w] = (int64_t)g * P + i;
+          ++w;
+        }
+      }
+    }
+  }
+  for (int64_t e = edge_ptr[B] + (int64_t)blockIdx.x * blockDim.x + tid; e < capacity; e += (int64_t)gridDim.x * blockDim.x) {
+    coo[e] = 0;
+    coo[row_stride + e] = 0;
+  }
+}
+
 __global__ void __launch_bounds__(128) dense_edges_kernel(int mode, const int32_t* __restrict__ num_valid,
                                                          const int64_t* __restrict__ edge_ptr, int B, int n_src, int n_dst,
                                                          int64_t* __restrict__ coo, int64_t row_stride) {
@@ -245,6 +318,25 @@ int grl_radius_neighbors(const float* pos, const int32_t* num_valid, int B, int 
   grl::radius_neighbors_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>(pos, num_valid, B, P, radius * radius,
                                                                        max_neighbors, nbr, cnt);
   return grl::check_launch("grl_radius_neighbors");
+}
+
+int grl_radius_edge_ptr(const int32_t* cnt, int B, int P, int64_t capacity, int64_t* edge_ptr, grl_stream_t stream) {
+  GRL_REQUIRE(cnt && edge_ptr && B > 0 && P > 0 && capacity >= 0, GRL_EINVAL, "grl_radius_edge_ptr: bad arguments");
+  grl::radius_edge_ptr_kernel<<<1, 1024, 0, (cudaStream_t)stream>>>(cnt, B, P, capacity, edge_ptr);
+  return grl::check_launch("grl_radius_edge_ptr");
+}
+
+int grl_radius_graph(const int32_t* nbr, const int32_t* cnt, const int64_t* edge_ptr, int B, int P, int max_neighbors,
+                     int64_t* coo, int64_t coo_row_stride, int64_t capacity, grl_stream_t stream) {
+  GRL_REQUIRE(nbr && cnt && edge_ptr && coo && B > 0 && P > 0 && capacity >= 1 && coo_row_stride >= capacity, GRL_EINVAL,
+              "grl_radius_graph: bad arguments");
+  GRL_REQUIRE(max_neighbors >= 1 && max_neighbors <= GRL_MAX_KNN, GRL_EUNSUPPORTED,
+              "grl_radius_graph: max_neighbors=%d not in [1,%d]", max_neighbors, GRL_MAX_KNN);
+  GRL_REQUIRE(P <= grl::kMaxP, GRL_EUNSUPPORTED, "grl_radius_graph: P=%d > %d", P, grl::kMaxP);
+  int grid = B < 16 * grl::sm_count() ? B : 16 * grl::sm_count();
+  grl::radius_graph_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>(nbr, cnt, edge_ptr, B, P, max_neighbors, coo,
+                                                                   coo_row_stride, capacity);
+  return grl::check_launch("grl_radius_graph");
 }
 
 int grl_dense_edges(int mode, const int32_t* num_valid, const int64_t* edge_ptr, int B, int n_src, int n_dst, int64_t* coo,

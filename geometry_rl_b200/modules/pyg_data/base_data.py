@@ -9,11 +9,13 @@ not in results:
   * `HeteroCartesian` / `HeteroDistance` edge attributes (recomputed every call by the reference,
     rigid_tasks_data.py:250, but read by none of HEPi / EMPN / DeepSets / transformer) are not produced.
 """
+import math
 from typing import Dict, List, Optional, Sequence, Tuple
 
 import torch
 
 from ... import ops
+from ..._lib import MAX_KNN as MAX_NUM_NEIGHBORS
 from .graph import GraphBatch
 
 
@@ -35,7 +37,8 @@ class BaseData:
     def __init__(self, observation_dim: Dict, observation_names: Dict, full_graph_obs: bool = False,
                  dist_as_pos: bool = False, output_mask_key: Optional[str] = None, training_noise: bool = False,
                  training_noise_std: float = 1e-2, concat_input_vector: bool = True, angular_velocity: bool = True,
-                 knn_k: int = 3, knn_to_actuators_k: int = -1, build_edges: bool = True, **kwargs):
+                 knn_k: int = 3, knn_to_actuators_k: int = -1, build_edges: bool = True, internal_edges: str = "knn",
+                 radius: Optional[float] = None, max_num_neighbors: int = MAX_NUM_NEIGHBORS, **kwargs):
         self._output_mask_key = output_mask_key
         self.training_noise = training_noise
         self.training_noise_std = training_noise_std
@@ -54,6 +57,24 @@ class BaseData:
             # the reference's own kNN-to-actuator branch never assigns TASK edges for rigid tasks
             # (rigid_tasks_data.py:302-312) and no shipped config selects it
             raise NotImplementedError("knn_to_actuators_k > 0 is not reachable with the shipped configs")
+        # INTERNAL edges of the kNN tasks (rigid, rope): "knn" (the reference's knn_graph, k = knn_k) or "radius" (every
+        # point within `radius`, at most the `max_num_neighbors` nearest; ops.radius_graph).  Cloth's are "full".
+        if internal_edges not in ("knn", "radius"):
+            raise ValueError(f"internal_edges must be 'knn' or 'radius', not {internal_edges!r}")
+        if internal_edges == "radius":
+            if self.INTERNAL_MODE != "knn":
+                raise ValueError(f"{type(self).__name__}: INTERNAL edges are '{self.INTERNAL_MODE}'; internal_edges="
+                                 "'radius' applies to the kNN tasks (rigid, rope)")
+            if isinstance(radius, bool) or not isinstance(radius, (int, float)) or not math.isfinite(radius) or radius <= 0:
+                raise ValueError(f"internal_edges='radius' needs a finite radius > 0, got {radius!r}")
+            if (isinstance(max_num_neighbors, bool) or not isinstance(max_num_neighbors, int)
+                    or not 1 <= max_num_neighbors <= MAX_NUM_NEIGHBORS):
+                raise ValueError(f"max_num_neighbors must be an int in [1, {MAX_NUM_NEIGHBORS}], got {max_num_neighbors!r}")
+        elif radius is not None:
+            raise ValueError("radius is only used with internal_edges='radius'")
+        self.internal_edges = internal_edges
+        self.radius = None if radius is None else float(radius)
+        self.max_num_neighbors = max_num_neighbors
         self.node_type_list = self._kept_node_types()
         # The reference keeps ONE placeholder and rebuilds it whenever the incoming batch size differs from the last one
         # (rigid_tasks_data.py:254-255), i.e. at every rollout <-> minibatch size alternation.  Same rule here: the dict
@@ -63,9 +84,15 @@ class BaseData:
         self.cache_all_sizes = False
         # Extension (BASELINE configs[3], SURVEY 3.4): rebuild the kNN / task topology from the CURRENT positions on every
         # `build_data` call instead of re-using the placeholder of the first batch (rope_tasks_data.py:224-225,251 builds
-        # once).  Off by default - parity runs use the reference's build-once rule; never on inside a CUDA-graph capture
-        # (the pruned row sets are derived with host-visible sizes).
+        # once).  Off by default - parity runs use the reference's build-once rule.  Two ways (see `refresh_in_place`):
+        #   * in place: radius INTERNAL edges, consumed by the fused 16-bit path - the placeholder of the batch size is
+        #     kept and its position- / num_valid-dependent edge types are rewritten on the device, no host sync, so a
+        #     captured CUDA graph (Learner.capture) rebuilds the topology on every replay;
+        #   * eagerly (any other combination, kNN included): the placeholder is dropped and rebuilt at exact size, with
+        #     host syncs - not capturable.
         self.rebuild_every_call = False
+        # set by the policy wrapper: True when the model consumes fixed-capacity edge sets (HEPi)
+        self.consumer_accepts_capacity = False
         self._placeholders: Dict[int, GraphBatch] = {}
         self._example_data: Optional[GraphBatch] = None
 
@@ -84,23 +111,34 @@ class BaseData:
         return slice(None)
 
     # ---- public entry point (base_data.py:45-55) ----------------------------------------------------
+    def refresh_in_place(self) -> bool:
+        """True when `rebuild_every_call` rewrites the topology in place on the device (capturable): radius INTERNAL
+        edges, edges built, a model that accepts fixed-capacity edge sets, and the fused 16-bit edge path."""
+        return (self.rebuild_every_call and self.internal_edges == "radius" and self.build_edges
+                and self.consumer_accepts_capacity and ops.fused_edge_enabled())
+
     def build_data(self, *args, **kwargs):
         inputs = self._preprocess_input(*args, **kwargs)
         if self._should_reconstruct_placeholders(**inputs):
             self._construct_placeholders(**inputs)
+        elif self.refresh_in_place():
+            self._refresh_topology(**inputs)
         with torch.no_grad():
             data = self._update_placeholders(**inputs)
             input_vector = self.construct_input_vector(data, **inputs)
         return data, input_vector
 
     def _should_reconstruct_placeholders(self, batch_size, **ignored) -> bool:
-        if self.rebuild_every_call:
+        refresh = self.refresh_in_place()
+        if self.rebuild_every_call and not refresh:
             self._placeholders.clear()
             return True
         cached = self._placeholders.get(batch_size)
-        if cached is not None:
+        if cached is not None and bool(cached.refreshed_edge_types) == refresh:
             self._example_data = cached
             return False
+        if cached is not None:  # built for the other rebuild mode (exact <-> fixed capacity)
+            del self._placeholders[batch_size]
         if not self.cache_all_sizes:
             self._placeholders.clear()  # `len(self.example_data) != batch_size` -> rebuild, the old one is dropped
         return True
@@ -145,12 +183,17 @@ class BaseData:
         e_int, e_agent, e_task = self.EDGE_TYPES
         P, A = npg[self.PARTICLE_TYPE], npg[self.ACTUATOR_TYPE]
         pts = position_vectors[self.PARTICLE_TYPE]
+        refresh = self.refresh_in_place()
         for et in self.EDGE_TYPES:  # insertion order INTERNAL, AGENT, TASK (rigid_tasks_data.py:285-319)
             src, _, dst = et
             if src not in kept or dst not in kept or not self.build_edges:
                 continue
+            # fixed capacity for what depends on the positions (INTERNAL) or on num_valid (TASK of the rigid tasks)
+            refreshed = refresh and (et == e_int or (et == e_task and num_valid is not None))
             if et == e_int:
-                if self.INTERNAL_MODE == "knn":
+                if self.INTERNAL_MODE == "knn" and self.internal_edges == "radius":
+                    coo, ptr = self._radius_edges(pts, num_valid, refreshed)
+                elif self.INTERNAL_MODE == "knn":
                     coo, ptr = ops.knn_graph(pts, num_valid, self.knn_k)
                 else:
                     coo, ptr = ops.dense_edges(0, B, P, P, device)
@@ -161,8 +204,8 @@ class BaseData:
                     coo = torch.empty(2, 0, dtype=torch.int64, device=device)
                     ptr = torch.zeros(B + 1, dtype=torch.int64, device=device)
             else:
-                coo, ptr = ops.dense_edges(1, B, P, A, device, num_valid=num_valid)
-            g.add_edge_type(et, coo, ptr)
+                coo, ptr = ops.dense_edges(1, B, P, A, device, num_valid=num_valid, capacity=refreshed)
+            g.add_edge_type(et, coo, ptr, refreshed=refreshed)
         for t in kept:  # HeteroNodeCategorical: one-hot over the PRE-subgraph type list (transforms.py:43-76)
             oh = torch.zeros(B * npg[t], len(self.ALL_NODE_TYPES), device=device)
             oh[:, list(self.ALL_NODE_TYPES).index(t)] = 1
@@ -171,6 +214,30 @@ class BaseData:
         g.output_mask = self.output_mask(g, self._output_mask_key)
         self._example_data = g
         self._placeholders[B] = g
+
+    def _radius_edges(self, pts, num_valid, capacity: bool):
+        B, P, _ = pts.shape
+        return ops.radius_graph(pts, num_valid, self.radius, self.max_num_neighbors,
+                                capacity=B * P * self.max_num_neighbors if capacity else None)
+
+    def _refresh_topology(self, position_vectors, infos, batch_size, device, **ignored):
+        """Rewrite the refreshed edge types of the cached placeholder from this batch, in place, on the device.
+
+        An edge type with no edge in the whole batch still runs its convolution here (its set has a fixed capacity, so
+        emptiness is not visible on the host): every destination row gets the update of an empty neighbourhood, as an
+        isolated node does in any batch.  Exact topology (build-once, eager rebuild) skips such an edge type instead,
+        as the reference does (hetero_fiber_conv.py:48-49)."""
+        g = self._example_data
+        num_valid = self._num_valid(infos, batch_size, device)
+        e_int = self.EDGE_TYPES[0]
+        pts = position_vectors[self.PARTICLE_TYPE]
+        for et in g.refreshed_edge_types:
+            if et == e_int:
+                coo, ptr = self._radius_edges(pts, num_valid, True)
+            else:
+                coo, ptr = ops.dense_edges(1, batch_size, pts.shape[1], position_vectors[self.ACTUATOR_TYPE].shape[1],
+                                           device, num_valid=num_valid, capacity=True)
+            ops.refresh_edge_set(g.edge_sets[et], coo, ptr)
 
     def _update_placeholders(self, position_vectors, norm_position_vectors, device, **ignored) -> GraphBatch:
         data = self._example_data.shallow_copy()

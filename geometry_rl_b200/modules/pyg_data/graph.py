@@ -66,6 +66,9 @@ class GraphBatch:
         self.output_mask_key: Optional[str] = None
         self.output_mask: slice = slice(None)
         self.homo_batch = None
+        # edge types held in fixed-capacity sets that the data builder refreshes in place from every batch's positions
+        # (BaseData.rebuild_every_call with radius edges on the fused 16-bit path); their row sets never enter pruning
+        self.refreshed_edge_types: set = set()
         self._homo_cache: Dict[str, ops.EdgeSet] = {}  # shared by every shallow copy of this topology
 
     # -- HeteroData-like surface ---------------------------------------------------------------
@@ -91,11 +94,14 @@ class GraphBatch:
             off += self.nodes_per_graph[t]
         return out
 
-    def add_edge_type(self, et: EdgeType, coo: torch.Tensor, edge_ptr: torch.Tensor):
+    def add_edge_type(self, et: EdgeType, coo: torch.Tensor, edge_ptr: torch.Tensor, refreshed: bool = False):
+        """`refreshed`: `coo` is a fixed-capacity buffer and the data builder rewrites the edge set in place later."""
         src, _, dst = et
         self.edge_types.append(et)
         self.edge_sets[et] = ops.build_edge_set(coo, edge_ptr, self.num_graphs, self.nodes_per_graph[src],
-                                                self.nodes_per_graph[dst])
+                                                self.nodes_per_graph[dst], exact=not refreshed)
+        if refreshed:
+            self.refreshed_edge_types.add(et)
 
     def shallow_copy(self) -> "GraphBatch":
         """`example_data.clone()` of the reference without copying the (immutable) topology."""
@@ -114,6 +120,8 @@ class GraphBatch:
         (node_types order); per graph the edges keep edge-type insertion order, as to_homogeneous()
         yields them, so the segmented sums see the same edge order as the reference."""
         if "homo" not in self._homo_cache:
+            for es in self.edge_sets.values():
+                ops.require_exact(es, "GraphBatch.homogeneous")
             B, dev = self.num_graphs, self.device
             n_tot = sum(self.nodes_per_graph.values())
             offs = self.node_offsets
@@ -168,11 +176,17 @@ class GraphBatch:
 
     # -- heterogeneous view without dead rows (HEPi) ---------------------------------------------------
     def hetero_pruned(self) -> PrunedHetero:
+        """Derived once per topology.  Every row of a node type that carries a refreshed edge type is live, so the live
+        set does not depend on edges that change from batch to batch; the pruned set of a refreshed edge type is then the
+        full `EdgeSet` itself (identity renumbering) and follows every in-place refresh."""
         if "hetero_pruned" not in self._homo_cache:
             dev = self.device
             touched = {t: torch.zeros(self._stores[t].num_nodes, dtype=torch.bool, device=dev) for t in self.node_types}
             for (src, _, dst), es in self.edge_sets.items():
-                if es.n_edges > 0:
+                if (src, _, dst) in self.refreshed_edge_types:
+                    touched[src][:] = True
+                    touched[dst][:] = True
+                elif es.n_edges > 0:
                     touched[src] |= (es.rowptr_src[1:] - es.rowptr_src[:-1]) > 0
                     touched[dst] |= (es.rowptr_dst[1:] - es.rowptr_dst[:-1]) > 0
             if self.output_mask_key is not None:
@@ -189,6 +203,9 @@ class GraphBatch:
             edge_sets = {}
             for et, es in self.edge_sets.items():
                 src, _, dst = et
+                if et in self.refreshed_edge_types:
+                    edge_sets[et] = es
+                    continue
                 if es.n_edges == 0 or src not in live_ids or dst not in live_ids:
                     continue
                 edge_sets[et] = ops.EdgeSet(

@@ -16,6 +16,10 @@ def _plain(s) -> str:
 
 
 class HEPi(nn.Module):
+    # On the fused 16-bit path every convolution walks the CSR row pointers, so it runs on fixed-capacity edge sets
+    # (ops.EdgeSet.exact False) as well; the other paths refuse them (ops.require_exact).
+    accepts_capacity_edge_sets = True
+
     def __init__(self, input_dim_node, input_dim_edge, hidden_dim, latent_dim, output_dim, output_dim_vec,
                  node_encoder_layers, edge_encoder_layers, node_decoder_layers, node_type_mapping, edge_type_mapping,
                  edge_level_mapping, message_passing, num_messages, concat_global=False, shared_processor=False,

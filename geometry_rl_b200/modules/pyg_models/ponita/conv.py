@@ -64,6 +64,14 @@ class FiberBundleConv(torch.nn.Module):
 
     @torch.no_grad()
     def _callibration_factors(self, x_src, x_dst, edge_attr, fk, edge_set):
+        if not edge_set.exact:
+            # fixed-capacity topology: statistics over the real edges only (one count read; the calibration is eager).
+            # A batch without any edge of this type leaves the convolution uncalibrated: the first batch with edges
+            # calibrates it, as with exact topology, where such a batch skips the convolution.
+            edge_set = ops.exact_edge_set(edge_set)
+            if edge_set.n_edges == 0:
+                return None
+            edge_attr = edge_attr.on(edge_set) if isinstance(edge_attr, ops.BasisSpec) else edge_attr
         x1 = ops.aggregate_messages(x_src, edge_attr, self.kernel.weight, edge_set)
         x2 = torch.einsum("boc,opc->bpc", x1, fk) / fk.shape[-2]
         std_in, std_1, std_2 = ops.calibration_std(x_dst), ops.calibration_std(x1), ops.calibration_std(x2)

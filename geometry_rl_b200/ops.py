@@ -90,6 +90,29 @@ class EdgeSet:
     src_eid: torch.Tensor  # [E] int32: src-sorted entry -> edge-order position
     s_src: Optional[torch.Tensor] = None  # [E] int32: source of the q-th src-sorted entry (lazy, see src_sorted_pairs)
     s_dst: Optional[torch.Tensor] = None  # [E] int32: destination of the q-th src-sorted entry
+    # False: a fixed-capacity set (refresh_edge_set rewrites it in place on the device, no host sync).  Every array is
+    # sized for `n_edges` = capacity; the real count is rowptr_dst[-1] (device only), and past it coo, edge_src, eid_coo and
+    # src_eid hold 0 (edge_dst, s_src, s_dst the node ids those zeros point at), so every gather stays in bounds.  Only
+    # the fused 16-bit kernels, which walk the CSR row pointers, accept such a set (`require_exact` guards the others).
+    exact: bool = True
+
+
+def require_exact(es: "EdgeSet", what: str) -> None:
+    """Refuse a fixed-capacity edge set in a consumer that visits all `n_edges` rows (strict fp32 kernels, the
+    materialised basis, the homogeneous view): the padding rows would enter its sums."""
+    if not es.exact:
+        raise ValueError(f"{what} needs an exact-size edge set; fixed-capacity (in-place refreshed) topology is consumed "
+                         "by the fused 16-bit edge kernels only (ops.set_precision('bf16'), fused edge path)")
+
+
+def exact_edge_set(es: "EdgeSet") -> "EdgeSet":
+    """The real-count prefix of a fixed-capacity edge set as an exact one (reads the count: one host sync).  Edges
+    [0, rowptr_dst[-1]) of the edge order are exactly the real ones, and the src-sorted entries point into them."""
+    if es.exact:
+        return es
+    E = int(es.rowptr_dst[-1].item())
+    return EdgeSet(es.n_src, es.n_dst, E, es.coo[:, :E], es.edge_ptr, es.rowptr_dst, es.edge_src[:E], es.edge_dst[:E],
+                   es.eid_coo[:E], es.rowptr_src, es.src_eid[:E])
 
 
 @dataclass
@@ -132,6 +155,7 @@ def src_sorted_pairs(es: "EdgeSet", sub: Optional[SubEdgeSet] = None):
 
 def build_sub_edge_set(es: "EdgeSet", out_ids: torch.Tensor) -> SubEdgeSet:
     assert es.n_src == es.n_dst, "sub edge sets are derived from homogeneous graphs"
+    require_exact(es, "build_sub_edge_set")
     dev = es.edge_src.device
     n_out = int(out_ids.numel())
     rank = torch.full((es.n_dst,), -1, dtype=torch.int64, device=dev)
@@ -187,8 +211,33 @@ def radius_neighbors(pos: torch.Tensor, num_valid: Optional[torch.Tensor], radiu
     return nbr, cnt
 
 
-def dense_edges(mode: int, B: int, n_src: int, n_dst: int, device, num_valid: Optional[torch.Tensor] = None):
-    """mode 0: ordered pairs j != k among n_src; mode 1: valid sources x all destinations."""
+def radius_graph(pos: torch.Tensor, num_valid: Optional[torch.Tensor], radius: float, max_num_neighbors: int,
+                 capacity: Optional[int] = None):
+    """pos [B,P,3] fp32 -> (coo [2,E] int64 coalesced, edge_ptr [B+1]): the radius graph of every point set.
+
+    Neighbours of centre i are the points j != i of the first num_valid[b] with sqdist <= radius^2 (the rounding of
+    knn_graph), at most `max_num_neighbors` nearest, ties to the lower index; row 0 = neighbour j (source), row 1 =
+    centre i (target), sorted by (j, i) per graph.  A point with a non-finite coordinate has no edges.
+    `capacity=None`: exact size (reads the count once, like knn_graph).  Otherwise no host sync: coo is
+    [2, capacity] with the entries past edge_ptr[B] set to 0, and edges that do not fit are dropped (edge_ptr is
+    clamped); `capacity=B * P * max_num_neighbors` can never drop one."""
+    pos = _f32c(pos)
+    B, P, _ = pos.shape
+    nbr, cnt = radius_neighbors(pos, num_valid, radius, max_num_neighbors)
+    edge_ptr = torch.empty(B + 1, dtype=torch.int64, device=pos.device)
+    bound = B * P * max_num_neighbors
+    L.call("grl_radius_edge_ptr", L.ptr(cnt), B, P, bound if capacity is None else int(capacity), L.ptr(edge_ptr))
+    E = int(edge_ptr[-1].item()) if capacity is None else int(capacity)
+    coo = torch.empty(2, max(E, 1), dtype=torch.int64, device=pos.device)
+    L.call("grl_radius_graph", L.ptr(nbr), L.ptr(cnt), L.ptr(edge_ptr), B, P, max_num_neighbors, L.ptr(coo),
+           coo.stride(0), coo.shape[1])
+    return coo[:, :E], edge_ptr
+
+
+def dense_edges(mode: int, B: int, n_src: int, n_dst: int, device, num_valid: Optional[torch.Tensor] = None,
+                capacity: bool = False):
+    """mode 0: ordered pairs j != k among n_src; mode 1: valid sources x all destinations.
+    `capacity` (mode 1): no host sync; coo is [2, B * n_src * n_dst] with the entries past edge_ptr[B] set to 0."""
     if mode == 0:
         counts = torch.full((B,), n_src * (n_src - 1), dtype=torch.int64, device=device)
     else:
@@ -197,20 +246,32 @@ def dense_edges(mode: int, B: int, n_src: int, n_dst: int, device, num_valid: Op
         counts = nv * n_dst
     edge_ptr = torch.zeros(B + 1, dtype=torch.int64, device=device)
     edge_ptr[1:] = torch.cumsum(counts, 0)
-    E = int(edge_ptr[-1].item())
-    coo = torch.empty(2, max(E, 1), dtype=torch.int64, device=device)
+    if capacity:
+        assert mode == 1, "fixed-capacity dense edges are the TASK edges (mode 1)"
+        E = B * n_src * n_dst
+        coo = torch.zeros(2, E, dtype=torch.int64, device=device)
+    else:
+        E = int(edge_ptr[-1].item())
+        coo = torch.empty(2, max(E, 1), dtype=torch.int64, device=device)
     if E > 0:
         nvp = num_valid.to(torch.int32).clamp(0, n_src).contiguous() if num_valid is not None else None
         L.call("grl_dense_edges", mode, L.ptr(nvp), L.ptr(edge_ptr), B, n_src, n_dst, L.ptr(coo), coo.stride(0))
     return coo[:, :E], edge_ptr
 
 
-def _csr(coo: torch.Tensor, edge_ptr: torch.Tensor, B: int, n_key: int, key_row: int):
+def _csr(coo: torch.Tensor, edge_ptr: torch.Tensor, B: int, n_key: int, key_row: int, out=None):
+    """`out` = (rowptr, other, eid) to rewrite in place; their entries past edge_ptr[B] are zeroed first (the kernel
+    writes the real edges only), so a gather through `other` / `eid` over the whole capacity stays in bounds."""
     E = coo.shape[1]
     dev = coo.device
-    rowptr = torch.zeros(B * n_key + 1, dtype=torch.int32, device=dev)
-    other = torch.empty(max(E, 1), dtype=torch.int32, device=dev)
-    eid = torch.empty(max(E, 1), dtype=torch.int32, device=dev)
+    if out is None:
+        rowptr = torch.zeros(B * n_key + 1, dtype=torch.int32, device=dev)
+        other = torch.empty(max(E, 1), dtype=torch.int32, device=dev)
+        eid = torch.empty(max(E, 1), dtype=torch.int32, device=dev)
+    else:
+        rowptr, other, eid = out
+        other.zero_()
+        eid.zero_()
     if E > 0:
         assert coo.stride(1) == 1
         L.call("grl_csr_build", L.ptr_any(coo), coo.stride(0), L.ptr(edge_ptr), B, n_key, key_row, L.ptr(rowptr),
@@ -219,17 +280,46 @@ def _csr(coo: torch.Tensor, edge_ptr: torch.Tensor, B: int, n_key: int, key_row:
 
 
 def build_edge_set(coo: torch.Tensor, edge_ptr: torch.Tensor, B: int, n_src_per_graph: int,
-                   n_dst_per_graph: int) -> EdgeSet:
-    """dst-sorted CSR (edge order) and src-sorted CSR of a batched, graph-major COO."""
+                   n_dst_per_graph: int, exact: bool = True) -> EdgeSet:
+    """dst-sorted CSR (edge order) and src-sorted CSR of a batched, graph-major COO.
+    `exact=False`: `coo` is a fixed-capacity buffer (radius_graph / dense_edges with a capacity); the set's `n_edges` is
+    the capacity, its real count rowptr_dst[-1], and it can be refreshed in place by `refresh_edge_set`."""
     E = coo.shape[1]
     if coo.stride(1) != 1:
         coo = coo.contiguous()
-    rowptr_dst, edge_src, eid_coo = _csr(coo, edge_ptr, B, n_dst_per_graph, 1)
+
+    def buffers(n_key):  # a capacity set gets zero tails (see _csr); a capacity is never 0
+        if exact:
+            return None
+        z = lambda n: torch.zeros(n, dtype=torch.int32, device=coo.device)  # noqa: E731
+        return z(B * n_key + 1), z(E), z(E)
+
+    rowptr_dst, edge_src, eid_coo = _csr(coo, edge_ptr, B, n_dst_per_graph, 1, buffers(n_dst_per_graph))
     edge_dst = coo[1][eid_coo.long()].to(torch.int32) if E > 0 else edge_src.clone()
     coo2 = torch.stack([edge_src.long(), edge_dst.long()]) if E > 0 else coo
-    rowptr_src, _, src_eid = _csr(coo2, edge_ptr, B, n_src_per_graph, 0)
+    rowptr_src, _, src_eid = _csr(coo2, edge_ptr, B, n_src_per_graph, 0, buffers(n_src_per_graph))
     return EdgeSet(B * n_src_per_graph, B * n_dst_per_graph, E, coo, edge_ptr, rowptr_dst, edge_src.contiguous(),
-                   edge_dst.contiguous(), eid_coo.contiguous(), rowptr_src, src_eid.contiguous())
+                   edge_dst.contiguous(), eid_coo.contiguous(), rowptr_src, src_eid.contiguous(), exact=exact)
+
+
+def refresh_edge_set(es: EdgeSet, coo: torch.Tensor, edge_ptr: torch.Tensor) -> None:
+    """Rewrite a fixed-capacity `EdgeSet` in place (same tensors, same addresses) from a new capacity COO / edge_ptr of
+    the same shape, cached src-sorted pairs included.  Device work only (no host sync): valid inside a CUDA-graph
+    capture, whose replays then rebuild the topology from whatever the inputs hold."""
+    assert not es.exact and tuple(coo.shape) == tuple(es.coo.shape) and edge_ptr.shape == es.edge_ptr.shape
+    B = es.edge_ptr.numel() - 1
+    es.coo.copy_(coo)
+    es.edge_ptr.copy_(edge_ptr)
+    _csr(es.coo, es.edge_ptr, B, es.n_dst // B, 1, (es.rowptr_dst, es.edge_src, es.eid_coo))
+    torch.index_select(es.coo[1], 0, es.eid_coo.long(), out=coo[1])  # coo is a scratch buffer from here on
+    es.edge_dst.copy_(coo[1])
+    coo[0].copy_(es.edge_src)
+    _csr(coo, es.edge_ptr, B, es.n_src // B, 0,
+         (es.rowptr_src, torch.empty_like(es.src_eid), es.src_eid))
+    if es.s_src is not None:
+        idx = es.src_eid.long()
+        torch.index_select(es.edge_src, 0, idx, out=es.s_src)
+        torch.index_select(es.edge_dst, 0, idx, out=es.s_dst)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -285,6 +375,7 @@ class EmbedFn(torch.autograd.Function):
 class EdgeBasisFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, pos_src, pos_dst, w1, b1, w2, b2, ori3, dim, es: EdgeSet):
+        require_exact(es, "the materialised edge basis")
         pos_src, pos_dst = _f32c(pos_src), _f32c(pos_dst)
         dev = pos_src.device
         w1t = torch.zeros(16, 64, dtype=torch.float32, device=dev)
@@ -350,6 +441,10 @@ class BasisSpec:
         self.pos_src, self.pos_dst = _f32c(pos_src.detach()), _f32c(pos_dst.detach())
         self.w1, self.b1, self.w2, self.b2 = w1, b1, w2, b2
         self.ori3, self.dim, self.es = ori3, dim, es
+
+    def on(self, es: EdgeSet) -> "BasisSpec":
+        """The same basis over another edge set (the exact view of a fixed-capacity one, see exact_edge_set)."""
+        return BasisSpec(self.pos_src, self.pos_dst, self.w1, self.b1, self.w2, self.b2, self.ori3, self.dim, es)
 
     def materialize(self) -> torch.Tensor:
         """The basis as a tensor (one-time calibration only, conv.py:151-157)."""
@@ -480,6 +575,7 @@ class FiberConvFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x_src, x_dst, basis, fk, wk, bias, ln_g, ln_b, w1, b1, w2, b2, es: EdgeSet,
                 sub: Optional[SubEdgeSet] = None):
+        require_exact(es, "FiberConvFn (strict fp32 / materialised-basis convolution)")
         homo = x_dst is None
         x_src = _f32c(x_src)
         if sub is not None:
@@ -634,6 +730,7 @@ def fiber_conv(x_src, x_dst, basis, fk, wk, bias, ln_g, ln_b, w1, b1, w2, b2, es
 
 def aggregate_messages(x_src, basis, wk, es: EdgeSet) -> torch.Tensor:
     """x1 only (no grad): used by the one-time calibration of conv.py:104-105,151-157."""
+    require_exact(es, "aggregate_messages")
     if isinstance(basis, BasisSpec):
         basis = basis.materialize()
     x_src, basis = _f32c(x_src.detach()), _f32c(basis.detach())

@@ -75,6 +75,18 @@ int grl_knn_graph(const float* pos, const int32_t* num_valid, const int64_t* edg
 int grl_radius_neighbors(const float* pos, const int32_t* num_valid, int B, int P, float radius, int max_neighbors,
                          int32_t* nbr, int32_t* cnt, grl_stream_t stream);
 
+/* Per-graph edge counts of a radius graph (the sum of cnt[b][0..P) from grl_radius_neighbors) and their exclusive
+ * prefix sum edge_ptr[B+1], every entry clamped to `capacity`.  Reads nothing on the host: usable inside a CUDA graph. */
+int grl_radius_edge_ptr(const int32_t* cnt, int B, int P, int64_t capacity, int64_t* edge_ptr, grl_stream_t stream);
+
+/* Coalesced COO of the radius graph given by nbr / cnt (grl_radius_neighbors) and edge_ptr (grl_radius_edge_ptr), in
+ * the convention of grl_knn_graph: row0 = neighbour (source), row1 = centre (target), sorted by (row0,row1) per graph,
+ * graph-major.  coo is [2][capacity] int64 (coo_row_stride >= capacity); entries [edge_ptr[B], capacity) are written
+ * with 0, so a gather over the whole buffer stays in bounds.  A point with a non-finite coordinate has no edges (a NaN
+ * distance never passes sqdist <= radius^2). */
+int grl_radius_graph(const int32_t* nbr, const int32_t* cnt, const int64_t* edge_ptr, int B, int P, int max_neighbors,
+                     int64_t* coo, int64_t coo_row_stride, int64_t capacity, grl_stream_t stream);
+
 /* Dense edge sets the reference builds with nested Python loops
  * (rigid_tasks_data.py:289-300,313-319): write the coalesced batched COO for
  *   mode 0: all ordered pairs j != k among n_src nodes per graph      (AGENT / cloth INTERNAL)
