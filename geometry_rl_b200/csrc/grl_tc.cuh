@@ -327,18 +327,21 @@ __device__ __forceinline__ __half2 gelu_h2(__half2 x) {
   const __half2 hx = __hmul2(x, half);
   return __hfma2(hx, t, hx);
 }
-// value and derivative with e = 0.5 (1 + t):  y = x e,  dy = e + x (1 - t^2) (k / 2 + 3 kc / 2 x^2)   (9 fma-pipe ops + 1 MUFU)
+// value and derivative with e = 0.5 (1 + t):  y = x e,  dy = e + x (1 - t^2) (k / 2 + 3 kc / 2 x^2)   (10 fma-pipe ops + 1 MUFU)
+// x^2 overflows fp16 for |x| > 256; there t = +-1 and the first factor of the derivative term is 0, so its second factor
+// takes min(x^2, 1024) (the exact x^2 below |x| = 32, where t is not yet +-1): 0 * inf would make dy NaN instead of e.
 __device__ __forceinline__ void gelu_h2(__half2 x, __half2& y, __half2& dy) {
   const __half2 k = __floats2half2_rn(0.7978845608028654f, 0.7978845608028654f);
   const __half2 kc = __floats2half2_rn(0.7978845608028654f * 0.044715f, 0.7978845608028654f * 0.044715f);
   const __half2 kh = __floats2half2_rn(0.5f * 0.7978845608028654f, 0.5f * 0.7978845608028654f);
   const __half2 k3h = __floats2half2_rn(1.5f * 0.7978845608028654f * 0.044715f, 1.5f * 0.7978845608028654f * 0.044715f);
   const __half2 half = __floats2half2_rn(0.5f, 0.5f), one = __floats2half2_rn(1.0f, 1.0f);
+  const __half2 x2max = __floats2half2_rn(1024.0f, 1024.0f);
   const __half2 x2 = __hmul2(x, x);
   const __half2 t = tanh_h2(__hmul2(x, __hfma2(x2, kc, k)));
   const __half2 e = __hfma2(t, half, half);
   y = __hmul2(x, e);
-  dy = __hfma2(__hmul2(x, __hfma2(__hneg2(t), t, one)), __hfma2(x2, k3h, kh), e);
+  dy = __hfma2(__hmul2(x, __hfma2(__hneg2(t), t, one)), __hfma2(__hmin2(x2, x2max), k3h, kh), e);
 }
 __device__ __forceinline__ uint4 pack_h8(const __half2 (&h)[4]) {
   uint4 o;
