@@ -97,6 +97,15 @@ class GrlReadoutDesc(C.Structure):
                 ("grad_latent", _fp), ("grad_partials", _fp), ("n_partials", _i32)]
 
 
+class GrlActDesc(C.Structure):
+    _fields_ = [("batch", _i32), ("num_rows", _i32), ("action_dim", _i32), ("hidden_dim", _i32), ("post_fc", _i32),
+                ("contextual_std", _i32), ("use_tanh_mean", _i32), ("deterministic", _i32), ("rank", _i32),
+                ("pre_shift", C.c_float), ("minimal_std", C.c_float), ("hidden", _fp), ("mean", _fp),
+                ("mean_weight", _fp), ("mean_bias", _fp), ("std_weight", _fp), ("std_bias", _fp), ("state", _fp),
+                ("loc", _fp), ("cov", _fp), ("action", _fp), ("log_prob", _fp), ("eps", _fp)]
+
+
+ACT_MAX_K = 32  # GRL_ACT_MAX_K
 READOUT_MAX_OUT = 8
 MAX_KNN = 8  # GRL_MAX_KNN: k of grl_knn_graph, max_neighbors of the radius graph
 LOSS_TERMS = 8
@@ -152,6 +161,8 @@ SIGNATURES = {
     "grl_absmax": (C.c_int, [_fp, C.c_int64, _fp, _fp]),
     "grl_reduce_partials": (C.c_int, [_fp, C.c_int, C.c_int64, _fp, C.c_int, _fp]),
     "grl_gae_scan": (C.c_int, [_fp, _fp, _fp, _fp, C.c_float, C.c_float, C.c_int, C.c_int, _fp, _fp, _fp]),
+    "grl_gaussian_act": (C.c_int, [C.POINTER(GrlActDesc), _fp]),
+    "grl_act_advance": (C.c_int, [_fp, _fp]),
     "grl_trpl_fwd": (C.c_int, [C.POINTER(GrlProjDesc), _fp]),
     "grl_trpl_bwd": (C.c_int, [C.POINTER(GrlProjDesc), _fp]),
     "grl_tc_selftest_gemm": (C.c_int, [_fp, _fp, _fp, C.c_int, C.c_int, _fp]),

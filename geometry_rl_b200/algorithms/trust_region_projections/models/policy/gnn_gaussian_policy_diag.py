@@ -10,6 +10,7 @@ import numpy as np
 import torch
 import torch.nn as nn
 
+from ..... import ops
 from ...utils.network_utils import initialize_weights
 from ...utils.torch_utils import inverse_softplus
 from ...utils.projection_utils import diag_of
@@ -79,6 +80,23 @@ class GNNGaussianPolicyDiag(nn.Module):
     def forward(self, *args, train=True):
         mean, var = self.forward_diag(*args, train=train)
         return mean, torch.diag_embed(var)
+
+    @torch.no_grad()
+    def act(self, *args, state, deterministic=False, rank=0, return_eps=False, train=True):
+        """`forward_diag`'s body call, then the head and the draw in one kernel (ops.gaussian_act) on the noise stream
+        `state` (not advanced here).  -> loc, covariance_matrix, action, sample_log_prob, eps (or None)."""
+        self.train(train)
+        batch_size = args[0].shape[0]
+        a_out = self.gnn_forward(*args, train=train)
+        mean, hidden = (None, a_out) if self.post_fc else a_out
+        std_w, std_b = (self._pre_std.weight, self._pre_std.bias) if self.contextual_std else (self._pre_std, None)
+        return ops.gaussian_act(state, batch=batch_size, num_rows=self.num_actuators, action_dim=self._mean.out_features,
+                                pre_shift=float(self._pre_activation_shift), minimal_std=float(self.minimal_std),
+                                std_weight=std_w, std_bias=std_b, hidden=hidden, mean=mean,
+                                mean_weight=self._mean.weight if self.post_fc else None,
+                                mean_bias=self._mean.bias if self.post_fc else None,
+                                use_tanh_mean=self.use_tanh_mean and self.post_fc, deterministic=deterministic,
+                                rank=rank, return_eps=return_eps)
 
     # ---- distribution helpers (std := second tuple element; diagonal or full layout) ----------------
     def sample(self, p, n=1):

@@ -9,6 +9,8 @@ from typing import Mapping, Sequence
 import torch
 from torch import nn
 
+from .... import ops
+
 LOG_2PI = math.log(2.0 * math.pi)
 
 
@@ -95,6 +97,97 @@ class PolicyOperator(nn.Module):
         td["loc"], td["covariance_matrix"] = dist.mean, dist.covariance_matrix
         td["action"], td["sample_log_prob"] = action, dist.log_prob(action)
         return td
+
+    # ---- rollout-time acting: fused head + on-device Philox noise (grl_gaussian_act), optionally one CUDA graph -----
+    # Opt-in path for the collector (`SyncDataCollector(policy=actor.act_graphed)`); `forward` and its torch RNG stay as
+    # they are.  The noise stream is an int64 device buffer {seed, call counter}: each sampling call draws from it and
+    # advances the counter on the device, so eager and replayed calls continue one stream.  Under data parallelism
+    # `act_rank` (set by DataParallel.attach) enters the key and ranks draw different noise.
+    act_rank = 0
+
+    def _act_state_buffer(self) -> torch.Tensor:
+        st = getattr(self, "_act_state", None)
+        if st is None:
+            st = torch.zeros(2, dtype=torch.int64, device=next(self.policy.parameters()).device)
+            self._act_state = st
+        return st
+
+    def act_state(self):
+        """(seed, call counter) of the acting noise stream (reads the device)."""
+        seed, counter = self._act_state_buffer().tolist()
+        return seed, counter
+
+    def set_act_state(self, seed: int, counter: int = 0) -> None:
+        """Restore the noise stream (in place: a captured act graph keeps reading the same buffer)."""
+        self._act_state_buffer().copy_(torch.tensor([int(seed), int(counter)], dtype=torch.int64))
+
+    def _act(self, obs, deterministic: bool, return_eps: bool = False):
+        state = self._act_state_buffer()
+        out = self.policy.act(*obs, state=state, deterministic=deterministic, rank=self.act_rank, return_eps=return_eps)
+        if not deterministic:
+            ops.act_advance(state)
+        return out
+
+    @staticmethod
+    def _write_act(td, out, copy: bool):
+        loc, cov, action, log_prob = out[:4]
+        if copy:
+            loc, cov, action, log_prob = loc.clone(), cov.clone(), action.clone(), log_prob.clone()
+        td["loc"], td["covariance_matrix"], td["action"], td["sample_log_prob"] = loc, cov, action, log_prob
+        return td
+
+    @torch.no_grad()
+    def act(self, td, *, deterministic: bool = False):
+        """The keys `forward` writes (loc, covariance_matrix, action, sample_log_prob), computed by one kernel after the
+        body, with noise from the device stream (`deterministic`: action = loc, nothing drawn)."""
+        return self._write_act(td, self._act([td_get(td, k) for k in self.in_keys], deterministic), copy=False)
+
+    def capture_act(self, example_td, *, seed: int, deterministic: bool = False, warmup: int = 2):
+        """Record `build_data -> body -> grl_gaussian_act -> advance` into one CUDA graph on static copies of the
+        example's observation keys (the batch size of every later `act_graphed` call), and start the noise stream at
+        (seed, 0).  A pending one-time FiberBundleConv calibration runs eagerly on the example first.  The graph holds the
+        topology of this batch size: re-capture after `hyper_data.invalidate()`.  With `hyper_data.rebuild_every_call`
+        the data builder must refresh its topology in place (`refresh_in_place()`): every replay then rebuilds the radius
+        graph from the static positions; any other rebuild mode is refused."""
+        hd = self.policy.hyper_data
+        if hd.rebuild_every_call and not hd.refresh_in_place():
+            raise ValueError(
+                "capture_act: the data builder rebuilds its topology eagerly on every call (rebuild_every_call with kNN "
+                "edges, the fp32 or unfused path, or a model other than HEPi), which reads sizes on the host and cannot "
+                "be replayed; a captured act rebuilds radius INTERNAL edges on the fused 16-bit path only "
+                "(internal_edges='radius', ops.set_precision('bf16')) - otherwise use `act`")
+        self._act_static = [td_get(example_td, k).clone() for k in self.in_keys]
+        with torch.no_grad():
+            self.get_dist(dict(zip(self.in_keys, self._act_static)))  # the one-time calibration, if still pending
+        self.set_act_state(seed, 0)
+        side = torch.cuda.Stream()
+        side.wait_stream(torch.cuda.current_stream())
+        with torch.cuda.stream(side), torch.no_grad():
+            for _ in range(warmup):  # draws without advancing: the stream is where set_act_state left it
+                self.policy.act(*self._act_static, state=self._act_state, deterministic=deterministic, rank=self.act_rank)
+        torch.cuda.current_stream().wait_stream(side)
+        self._act_graph = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(self._act_graph), torch.no_grad():
+            self._act_graph_out = self._act(self._act_static, deterministic)
+        # the replayed kernels read this batch size's topology tensors: keep them alive if the builder drops them
+        self._captured_topology = hd.example_data
+        return self
+
+    def act_static(self, td=None):
+        """Replay the captured act on whatever the static inputs hold; with `td`, write the graph's own output tensors
+        into it (no copy: the next replay overwrites them).  Returns the outputs keyed like `forward`'s."""
+        self._act_graph.replay()
+        out = dict(zip(self.out_keys, self._act_graph_out[:4]))
+        if td is not None:
+            self._write_act(td, self._act_graph_out, copy=False)
+        return out
+
+    def act_graphed(self, td):
+        """Copy td's observation keys into the static inputs, replay the captured act and write copies of its outputs."""
+        for s, k in zip(self._act_static, self.in_keys):
+            s.copy_(td_get(td, k), non_blocking=True)
+        self._act_graph.replay()
+        return self._write_act(td, self._act_graph_out, copy=True)
 
 
 class ValueOperator(nn.Module):

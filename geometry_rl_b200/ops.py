@@ -891,6 +891,49 @@ def gae(reward, value_T1, done, terminated, gamma: float, lmbda: float):
 
 
 # ------------------------------------------------------------------------------------------------
+# A1: rollout-time Gaussian head + on-device sampling
+# ------------------------------------------------------------------------------------------------
+def gaussian_act(state, *, batch: int, num_rows: int, action_dim: int, pre_shift: float, minimal_std: float,
+                 std_weight, std_bias=None, hidden=None, mean=None, mean_weight=None, mean_bias=None,
+                 use_tanh_mean: bool = False, deterministic: bool = False, rank: int = 0, return_eps: bool = False):
+    """One grl_gaussian_act launch (no autograd: acting only).  `state` is the int64 [2] {seed, call counter} buffer the
+    draw reads; it is not advanced here (`act_advance`).  post_fc is implied by `mean is None` (the head's `_mean`
+    Linear is applied to `hidden`), contextual std by `std_bias is not None` (`_pre_std` is a Linear).
+    -> loc [B,k], covariance_matrix [B,k,k], action [B,k], sample_log_prob [B], eps [B,k] (or None)."""
+    if state.dtype != torch.int64 or state.numel() != 2:
+        raise ValueError("gaussian_act: state must be an int64 tensor {seed, counter}")
+    post_fc, contextual = mean is None, std_bias is not None
+    B, A, a = int(batch), int(num_rows), int(action_dim)
+    k = A * a
+    dev = state.device
+    hidden = _f32c(hidden) if hidden is not None else None
+    mean = _f32c(mean) if mean is not None else None
+    if (post_fc or contextual) and (hidden is None or hidden.shape[0] != B * A):
+        raise ValueError(f"gaussian_act: hidden must have batch * num_rows = {B * A} rows")
+    if not post_fc and mean.numel() != B * k:
+        raise ValueError(f"gaussian_act: mean must hold batch * k = {B * k} values, got {mean.numel()}")
+    ws = [None if w is None else _f32c(w.detach()) for w in (mean_weight, mean_bias, std_weight, std_bias)]
+    loc = torch.empty(B, k, dtype=torch.float32, device=dev)
+    cov = torch.empty(B, k, k, dtype=torch.float32, device=dev)
+    action = torch.empty(B, k, dtype=torch.float32, device=dev)
+    log_prob = torch.empty(B, dtype=torch.float32, device=dev)
+    eps = torch.empty(B, k, dtype=torch.float32, device=dev) if return_eps else None
+    d = L.GrlActDesc(batch=B, num_rows=A, action_dim=a, hidden_dim=hidden.shape[-1] if hidden is not None else 64,
+                     post_fc=int(post_fc), contextual_std=int(contextual), use_tanh_mean=int(bool(use_tanh_mean)),
+                     deterministic=int(bool(deterministic)), rank=int(rank), pre_shift=float(pre_shift),
+                     minimal_std=float(minimal_std), hidden=L.ptr(hidden), mean=L.ptr(mean), mean_weight=L.ptr(ws[0]),
+                     mean_bias=L.ptr(ws[1]), std_weight=L.ptr(ws[2]), std_bias=L.ptr(ws[3]), state=L.ptr(state),
+                     loc=L.ptr(loc), cov=L.ptr(cov), action=L.ptr(action), log_prob=L.ptr(log_prob), eps=L.ptr(eps))
+    L.call("grl_gaussian_act", C.byref(d), shape=(B, k, 0))
+    return loc, cov, action, log_prob, eps
+
+
+def act_advance(state) -> None:
+    """state[1] += 1 on the device (the call counter of gaussian_act's noise stream)."""
+    L.call("grl_act_advance", L.ptr(state))
+
+
+# ------------------------------------------------------------------------------------------------
 # K4: trust-region projection
 # ------------------------------------------------------------------------------------------------
 class TrplProjectFn(torch.autograd.Function):

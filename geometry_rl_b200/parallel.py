@@ -162,6 +162,9 @@ class DataParallel:
         from .modules.pyg_models.pyg_compat import GraphLayerNorm
         from . import ops
         loss_module.dp = self
+        actor = getattr(loss_module, "actor_network", None)
+        if actor is not None:
+            actor.act_rank = self.rank  # rollout noise (PolicyOperator.act*): the rank enters the key, one stream per rank
         ops.set_calibration_std(self.global_std)  # conv.py:151-157 / ponita.py:178-192 statistics become global
         critic_dp = self.side if self.side is not None else self
         for m in loss_module.critic_network.modules():

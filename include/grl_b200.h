@@ -378,6 +378,44 @@ int grl_gae_scan(const float* reward, const float* value_T1, const uint8_t* done
                  float gamma, float lmbda, int B, int T, float* advantage, float* value_target, grl_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------
+ * A1  Rollout-time Gaussian head + sampling: replaces the eager ProbabilisticActor call of the collector
+ * (examples/torchrl/train.py, SyncDataCollector(policy=actor)): the head of
+ * models/policy/gnn_gaussian_policy_diag.py:26-87 (_mean, _pre_std, softplus, square), torch.randn, log_prob and
+ * diag_embed, one warp per sample.  Noise is counter-based Philox4x32-10 keyed by state[0] (seed) and the rank, with
+ * state[1] (the call counter) in the counter; grl_act_advance increments state[1].  The draw of a component depends
+ * on (seed, rank, call, sample, component) only.  Bit-level mapping: geometry_rl_b200/csrc/grl_act.cu.
+ * ------------------------------------------------------------------------------------------ */
+#define GRL_ACT_MAX_K 32 /* k = num_rows * action_dim components per sample */
+typedef struct {
+  int32_t batch;           /* B samples                                                                          */
+  int32_t num_rows;        /* A actuator rows per sample                                                         */
+  int32_t action_dim;      /* a components per row (k = A a <= GRL_ACT_MAX_K)                                     */
+  int32_t hidden_dim;      /* must be 64                                                                         */
+  int32_t post_fc;         /* 1: mean = hidden _mean.weight^T + _mean.bias; 0: mean given                          */
+  int32_t contextual_std;  /* 1: pre = hidden _pre_std.weight^T + _pre_std.bias; 0: pre = std_weight (shared)        */
+  int32_t use_tanh_mean;   /* loc = tanh(mean)                                                                   */
+  int32_t deterministic;   /* action = loc, eps = 0 (evaluation / play); draws nothing                             */
+  int32_t rank;            /* data-parallel rank: enters the Philox key                                           */
+  float pre_shift;         /* _pre_activation_shift                                                              */
+  float minimal_std;
+  const float* hidden;     /* [B*A][64] (post_fc or contextual std; else may be NULL)                              */
+  const float* mean;       /* [B][k] body mean rows (post_fc == 0)                                               */
+  const float* mean_weight;/* [a][64] (post_fc)                                                                  */
+  const float* mean_bias;  /* [a]     (post_fc)                                                                  */
+  const float* std_weight; /* [a][64] contextual, [a] shared _pre_std                                             */
+  const float* std_bias;   /* [a] (contextual)                                                                   */
+  const int64_t* state;    /* [2] {seed, call counter}                                                            */
+  float* loc;              /* [B][k]                                                                             */
+  float* cov;              /* [B][k][k]: diagonal var, off-diagonal entries exact zeros                            */
+  float* action;           /* [B][k]                                                                             */
+  float* log_prob;         /* [B]                                                                                */
+  float* eps;              /* optional [B][k]: the standard normals drawn                                          */
+} GrlActDesc;
+int grl_gaussian_act(const GrlActDesc* d, grl_stream_t stream);
+/* state[1] += 1 (one thread). */
+int grl_act_advance(int64_t* state, grl_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------
  * K4  TRPL projection of a diagonal Gaussian (mean + "std := cov" diagonal v):
  * replaces projections/kl_projection_layer.py:15-111,162-204 (ITPAL cpp_projection on the CPU),
  * projections/w2_projection_layer.py:15-68, base_projection_layer.py:71-100.
