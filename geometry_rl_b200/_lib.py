@@ -126,6 +126,8 @@ SIGNATURES = {
     "grl_reserve_sms": (C.c_int, [C.c_int]),
     "grl_knn_edge_ptr": (C.c_int, [_fp, C.c_int, C.c_int, C.c_int, _fp, _fp]),
     "grl_knn_graph": (C.c_int, [_fp, _fp, _fp, C.c_int, C.c_int, C.c_int, _fp, C.c_int64, _fp]),
+    "grl_knn_topology": (C.c_int, [_fp, _fp, _fp, C.c_int, C.c_int, C.c_int, C.c_int64, _fp, C.c_int64, _fp, _fp, _fp,
+                                   _fp, _fp, _fp, _fp, _fp, _fp]),
     "grl_radius_neighbors": (C.c_int, [_fp, _fp, C.c_int, C.c_int, C.c_float, C.c_int, _fp, _fp, _fp]),
     "grl_radius_edge_ptr": (C.c_int, [_fp, C.c_int, C.c_int, C.c_int64, _fp, _fp]),
     "grl_radius_graph": (C.c_int, [_fp, _fp, _fp, C.c_int, C.c_int, C.c_int, _fp, C.c_int64, C.c_int64, _fp]),

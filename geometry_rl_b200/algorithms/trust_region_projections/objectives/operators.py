@@ -147,15 +147,17 @@ class PolicyOperator(nn.Module):
         example's observation keys (the batch size of every later `act_graphed` call), and start the noise stream at
         (seed, 0).  A pending one-time FiberBundleConv calibration runs eagerly on the example first.  The graph holds the
         topology of this batch size: re-capture after `hyper_data.invalidate()`.  With `hyper_data.rebuild_every_call`
-        the data builder must refresh its topology in place (`refresh_in_place()`): every replay then rebuilds the radius
-        graph from the static positions; any other rebuild mode is refused."""
+        the data builder must refresh its topology in place (`refresh_in_place()`): every replay then rebuilds the kNN or
+        radius graph from the static positions; any other rebuild mode is refused."""
         hd = self.policy.hyper_data
         if hd.rebuild_every_call and not hd.refresh_in_place():
             raise ValueError(
                 "capture_act: the data builder rebuilds its topology eagerly on every call (rebuild_every_call with kNN "
-                "edges, the fp32 or unfused path, or a model other than HEPi), which reads sizes on the host and cannot "
-                "be replayed; a captured act rebuilds radius INTERNAL edges on the fused 16-bit path only "
-                "(internal_edges='radius', ops.set_precision('bf16')) - otherwise use `act`")
+                "edges without knn_in_place, a task with num_valid on the fp32 or unfused path, or a model other than "
+                "HEPi), which reads sizes on the host and cannot be replayed; a captured act rebuilds kNN INTERNAL edges "
+                "with `hyper_data.knn_in_place = True` (rope: any precision; rigid: fused 16-bit path) and radius "
+                "INTERNAL edges on the fused 16-bit path (internal_edges='radius', ops.set_precision('bf16')) - "
+                "otherwise use `act`")
         self._act_static = [td_get(example_td, k).clone() for k in self.in_keys]
         with torch.no_grad():
             self.get_dist(dict(zip(self.in_keys, self._act_static)))  # the one-time calibration, if still pending

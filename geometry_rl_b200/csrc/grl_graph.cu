@@ -4,6 +4,8 @@
 // rope_tasks_data.py:238-278, cloth_tasks_data.py:236-286; plus the graph-major batching of
 // Batch.from_data_list (rigid_tasks_data.py:324).  One CTA per graph; graphs have <= a few hundred
 // nodes, so everything is brute force in shared memory.  Integer outputs are bit-exact by construction.
+#include <algorithm>
+
 #include "grl_common.cuh"
 
 namespace grl {
@@ -109,6 +111,180 @@ __global__ void __launch_bounds__(128) knn_graph_kernel(const float* __restrict_
           ++w;
         }
       }
+    }
+  }
+}
+
+// Rank key of a squared distance: a sum of squares is +0, positive, +inf or NaN, and the bits of a non-negative float
+// order like the float.  NaN ranks as +inf, so the order (key, index) is total whatever the positions hold.
+__device__ __forceinline__ uint32_t dist_key(float d) { return d != d ? 0x7f800000u : __float_as_uint(d); }
+
+// The kk nearest neighbours of every valid centre of graph g (self excluded), ranked by (dist_key, index), written to
+// nbr[i * GRL_MAX_KNN + s], s < kk, in ascending INDEX order.  Every centre gets exactly kk neighbours; for finite
+// distances the set is the one knn_graph_kernel picks.  Ends with a block barrier.
+__device__ void knn_sorted_lists(const float* __restrict__ pos, int g, int P, int pv, int kk, float* sp, short* nbr) {
+  const int tid = threadIdx.x;
+  for (int i = tid; i < pv * 3; i += blockDim.x) sp[i] = pos[(size_t)g * P * 3 + i];
+  __syncthreads();
+  for (int i = tid; i < pv; i += blockDim.x) {
+    uint32_t bk[GRL_MAX_KNN];
+    int bj[GRL_MAX_KNN];
+#pragma unroll
+    for (int s = 0; s < GRL_MAX_KNN; ++s) { bk[s] = 0xffffffffu; bj[s] = 0x7fffffff; }  // empty: after every candidate
+    uint32_t worst = 0xffffffffu;  // bk[kk - 1]
+    for (int j = 0; j < pv; ++j) {
+      if (j == i) continue;
+      const uint32_t key = dist_key(sqdist(sp + 3 * i, sp + 3 * j));
+      if (key >= worst) continue;  // a tie keeps the lower index, which came first
+#pragma unroll
+      for (int u = GRL_MAX_KNN - 1; u >= 0; --u) {
+        if (u >= kk) continue;
+        if (u > 0 && bk[u - 1] > key) { bk[u] = bk[u - 1]; bj[u] = bj[u - 1]; }
+        else if (bk[u] > key) { bk[u] = key; bj[u] = j; }
+      }
+#pragma unroll
+      for (int s = 0; s < GRL_MAX_KNN; ++s) if (s == kk - 1) worst = bk[s];
+    }
+    // ascending index (odd-even transposition; the empty slots past kk sort last)
+#pragma unroll
+    for (int r = 0; r < GRL_MAX_KNN; ++r) {
+#pragma unroll
+      for (int s = r & 1; s + 1 < GRL_MAX_KNN; s += 2) {
+        const int a = bj[s], b = bj[s + 1];
+        bj[s] = min(a, b);
+        bj[s + 1] = max(a, b);
+      }
+    }
+#pragma unroll
+    for (int s = 0; s < GRL_MAX_KNN; ++s) if (s < kk) nbr[i * GRL_MAX_KNN + s] = (short)bj[s];
+  }
+  __syncthreads();
+}
+
+struct KnnTopoOut {
+  int64_t* coo;
+  int64_t row_stride;
+  int32_t *rowptr_dst, *edge_src, *edge_dst, *eid_coo, *rowptr_src, *src_eid, *s_src, *s_dst;
+};
+
+// Every layout of the kNN edge set in one pass (see grl_knn_topology).  CTAs [0, n_graph_ctas) own the graphs; the
+// others write the tail [edge_ptr[B], capacity).
+__global__ void __launch_bounds__(128) knn_topology_kernel(const float* __restrict__ pos,
+                                                          const int32_t* __restrict__ num_valid,
+                                                          const int64_t* __restrict__ edge_ptr, int B, int P, int k,
+                                                          int64_t capacity, int n_graph_ctas, KnnTopoOut o) {
+  __shared__ float sp[kMaxP * 3];
+  __shared__ short nbr[kMaxP * GRL_MAX_KNN];
+  __shared__ int cnt[kMaxP];
+  __shared__ int off[kMaxP + 1];
+  __shared__ int first_edge;
+  const int tid = threadIdx.x;
+  if ((int)blockIdx.x < n_graph_ctas) {
+    for (int g = blockIdx.x; g < B; g += n_graph_ctas) {
+      const int pv = valid_points(num_valid, g, P);
+      const int kk = max(0, min(k, pv - 1));
+      __syncthreads();  // the previous graph's shared arrays are no longer read
+      for (int j = tid; j < pv; j += blockDim.x) cnt[j] = 0;
+      knn_sorted_lists(pos, g, P, pv, kk, sp, nbr);
+      for (int q = tid; q < pv * kk; q += blockDim.x) atomicAdd(&cnt[nbr[(q / kk) * GRL_MAX_KNN + q % kk]], 1);
+      __syncthreads();
+      if (tid < 32) {  // off = exclusive prefix sum of cnt (off[j] = edges of the neighbours before j)
+        int carry = 0;
+        for (int b = 0; b < pv; b += 32) {
+          const int j = b + tid;
+          int v = j < pv ? cnt[j] : 0;
+#pragma unroll
+          for (int d = 1; d < 32; d <<= 1) {
+            const int t = __shfl_up_sync(0xffffffffu, v, d);
+            if (tid >= d) v += t;
+          }
+          if (j < pv) off[j + 1] = carry + v;
+          carry += __shfl_sync(0xffffffffu, v, 31);
+        }
+        if (tid == 0) off[0] = 0;
+      }
+      __syncthreads();
+      const int64_t e0 = edge_ptr[g], e1 = edge_ptr[g + 1];
+      const int64_t node0 = (int64_t)g * P;
+      // edge order = dst-sorted CSR: centre i, then its neighbours ascending
+      for (int i = tid; i < P; i += blockDim.x) {
+        if (i >= pv) {
+          o.rowptr_dst[node0 + i] = (int32_t)e1;
+          continue;
+        }
+        const int64_t e = e0 + (int64_t)i * kk;
+        o.rowptr_dst[node0 + i] = (int32_t)e;
+        for (int s = 0; s < kk; ++s) {
+          o.edge_src[e + s] = (int32_t)(node0 + nbr[i * GRL_MAX_KNN + s]);
+          o.edge_dst[e + s] = (int32_t)(node0 + i);
+        }
+      }
+      // COO order = src-sorted CSR: neighbour j, then the centres that chose it ascending
+      for (int j = tid; j < P; j += blockDim.x) {
+        if (j >= pv) {
+          o.rowptr_src[node0 + j] = (int32_t)e1;
+          continue;
+        }
+        int64_t w = e0 + off[j];
+        const int64_t w1 = e0 + off[j + 1];
+        o.rowptr_src[node0 + j] = (int32_t)w;
+        for (int i = 0; i < pv && w < w1; ++i) {
+          for (int s = 0; s < kk; ++s) {
+            if (nbr[i * GRL_MAX_KNN + s] != j) continue;
+            const int64_t e = e0 + (int64_t)i * kk + s;
+            o.coo[w] = node0 + j;
+            o.coo[o.row_stride + w] = node0 + i;
+            o.eid_coo[e] = (int32_t)w;
+            o.src_eid[w] = (int32_t)e;
+            if (o.s_src) {
+              o.s_src[w] = (int32_t)(node0 + j);
+              o.s_dst[w] = (int32_t)(node0 + i);
+            }
+            ++w;
+            break;  // a centre lists j at most once
+          }
+        }
+      }
+      if (g == B - 1 && tid == 0) {
+        o.rowptr_dst[(size_t)B * P] = (int32_t)e1;
+        o.rowptr_src[(size_t)B * P] = (int32_t)e1;
+      }
+    }
+    return;
+  }
+  // Tail: coo, edge_src, eid_coo and src_eid hold 0; edge_dst, s_src and s_dst hold what a gather through those zeros
+  // reads: coo[1][0], edge_src[0] and edge_dst[0].  They come from the first graph with edges, g0, whose kNN lists this
+  // CTA recomputes: edge 0 of the edge order is (nbr[0][0] -> centre 0), and COO entry 0 is the smallest (j, i).
+  const int64_t e_end = edge_ptr[B];
+  if (e_end >= capacity) return;
+  int v_dst = 0, v_ssrc = 0, v_sdst = 0;
+  if (e_end > 0) {
+    int lo = 0, hi = B - 1;  // smallest g with edge_ptr[g + 1] > 0 (edge_ptr is non-decreasing and edge_ptr[0] = 0)
+    while (lo < hi) {
+      const int mid = (lo + hi) / 2;
+      if (edge_ptr[mid + 1] > 0) hi = mid; else lo = mid + 1;
+    }
+    const int g0 = lo, pv = valid_points(num_valid, g0, P), kk = max(0, min(k, pv - 1));
+    if (tid == 0) first_edge = 0x7fffffff;
+    knn_sorted_lists(pos, g0, P, pv, kk, sp, nbr);
+    for (int i = tid; i < pv; i += blockDim.x) atomicMin(&first_edge, nbr[i * GRL_MAX_KNN] * kMaxP + i);
+    __syncthreads();
+    v_dst = (int)((int64_t)g0 * P + first_edge % kMaxP);
+    v_ssrc = (int)((int64_t)g0 * P + nbr[0]);
+    v_sdst = (int)((int64_t)g0 * P);
+  }
+  const int64_t n_tail = gridDim.x - n_graph_ctas;
+  for (int64_t e = e_end + (int64_t)(blockIdx.x - n_graph_ctas) * blockDim.x + tid; e < capacity;
+       e += n_tail * blockDim.x) {
+    o.coo[e] = 0;
+    o.coo[o.row_stride + e] = 0;
+    o.edge_src[e] = 0;
+    o.eid_coo[e] = 0;
+    o.src_eid[e] = 0;
+    o.edge_dst[e] = v_dst;
+    if (o.s_src) {
+      o.s_src[e] = v_ssrc;
+      o.s_dst[e] = v_sdst;
     }
   }
 }
@@ -306,6 +482,33 @@ int grl_knn_graph(const float* pos, const int32_t* num_valid, const int64_t* edg
   int grid = B < 16 * grl::sm_count() ? B : 16 * grl::sm_count();
   grl::knn_graph_kernel<<<grid, 128, 0, (cudaStream_t)stream>>>(pos, num_valid, edge_ptr, B, P, k, coo, coo_row_stride);
   return grl::check_launch("grl_knn_graph");
+}
+
+int grl_knn_topology(const float* pos, const int32_t* num_valid, const int64_t* edge_ptr, int B, int P, int k,
+                     int64_t capacity, int64_t* coo, int64_t coo_row_stride, int32_t* rowptr_dst, int32_t* edge_src,
+                     int32_t* edge_dst, int32_t* eid_coo, int32_t* rowptr_src, int32_t* src_eid, int32_t* s_src,
+                     int32_t* s_dst, grl_stream_t stream) {
+  // the per-edge arrays may be NULL for a set of no edges (capacity 0): nothing is written to them then
+  GRL_REQUIRE(pos && edge_ptr && rowptr_dst && rowptr_src && B > 0 && P > 0 && (s_src == nullptr) == (s_dst == nullptr) &&
+                  (capacity == 0 || (coo && edge_src && edge_dst && eid_coo && src_eid)),
+              GRL_EINVAL, "grl_knn_topology: bad arguments");
+  GRL_REQUIRE(k >= 1 && k <= GRL_MAX_KNN, GRL_EUNSUPPORTED, "grl_knn_topology: k=%d not in [1,%d]", k, GRL_MAX_KNN);
+  GRL_REQUIRE(P <= grl::kMaxP, GRL_EUNSUPPORTED, "grl_knn_topology: P=%d > %d", P, grl::kMaxP);
+  const int64_t bound = (int64_t)B * P * std::max(0, std::min(k, P - 1));  // edges of B graphs with every point valid
+  GRL_REQUIRE(capacity >= bound && coo_row_stride >= capacity, GRL_EINVAL,
+              "grl_knn_topology: capacity=%lld (row stride %lld) below the %lld edges B*P*min(k,P-1)",
+              (long long)capacity, (long long)coo_row_stride, (long long)bound);
+  GRL_REQUIRE(capacity <= INT32_MAX && (int64_t)B * P < INT32_MAX, GRL_EUNSUPPORTED,
+              "grl_knn_topology: capacity=%lld or B*P=%lld exceeds the int32 edge / node ids", (long long)capacity,
+              (long long)B * P);
+  const int graph_ctas = B < 16 * grl::sm_count() ? B : 16 * grl::sm_count();
+  // a tail can only exist when some graph has fewer than P valid points or the buffer is larger than every edge
+  const bool tail = num_valid != nullptr || capacity > bound;
+  const int tail_ctas = tail ? (int)std::min<int64_t>(grl::sm_count(), (capacity + 4095) / 4096) : 0;
+  grl::KnnTopoOut o{coo, coo_row_stride, rowptr_dst, edge_src, edge_dst, eid_coo, rowptr_src, src_eid, s_src, s_dst};
+  grl::knn_topology_kernel<<<graph_ctas + tail_ctas, 128, 0, (cudaStream_t)stream>>>(pos, num_valid, edge_ptr, B, P, k,
+                                                                                    capacity, graph_ctas, o);
+  return grl::check_launch("grl_knn_topology");
 }
 
 int grl_radius_neighbors(const float* pos, const int32_t* num_valid, int B, int P, float radius, int max_neighbors,

@@ -225,16 +225,18 @@ class Learner:
         `loss_module._global_steps`): lr annealing or an entropy schedule would be frozen, so capture refuses them.
         The graph also holds the topology tensors of this batch size: re-capture after `hyper_data.invalidate()`.  With
         `hyper_data.rebuild_every_call` the data builder must refresh its topology in place (`refresh_in_place()`): every
-        replay then rebuilds the radius graph from the static inputs' positions; any other rebuild mode is refused."""
+        replay then rebuilds the kNN or radius graph from the static inputs' positions; any other rebuild mode is refused."""
         for net in (self.actor, self.critic):
             for m in net.modules():
                 hd = getattr(m, "hyper_data", None)
                 if hd is not None and hd.rebuild_every_call and not hd.refresh_in_place():
                     raise ValueError(
                         "capture: the data builder rebuilds its topology eagerly on every call (rebuild_every_call with "
-                        "kNN edges, the fp32 or unfused path, or a model other than HEPi), which reads sizes on the host "
-                        "and cannot be replayed; a captured update rebuilds radius INTERNAL edges on the fused 16-bit "
-                        "path only (internal_edges='radius', ops.set_precision('bf16')) - otherwise use `update`")
+                        "kNN edges without knn_in_place, a task with num_valid on the fp32 or unfused path, or a model "
+                        "other than HEPi), which reads sizes on the host and cannot be replayed; a captured update "
+                        "rebuilds kNN INTERNAL edges with `hyper_data.knn_in_place = True` (rope: any precision; rigid: "
+                        "fused 16-bit path) and radius INTERNAL edges on the fused 16-bit path (internal_edges='radius', "
+                        "ops.set_precision('bf16')) - otherwise use `update`")
         proj = getattr(self.loss_module, "projection", None)
         if getattr(proj, "entropy_schedule", False):
             raise NotImplementedError("an entropy schedule depends on the host-side step counter, which a captured graph "

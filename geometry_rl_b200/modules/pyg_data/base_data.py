@@ -33,6 +33,7 @@ class BaseData:
     INTERNAL_MODE: str = "knn"
     EDGE_TYPES: Sequence[Tuple[str, str, str]] = ()
     HAS_INFOS: bool = False
+    HAS_NUM_VALID: bool = False  # the particle count varies per sample (`_num_valid`): kNN edge counts are data-dependent
 
     def __init__(self, observation_dim: Dict, observation_names: Dict, full_graph_obs: bool = False,
                  dist_as_pos: bool = False, output_mask_key: Optional[str] = None, training_noise: bool = False,
@@ -85,12 +86,19 @@ class BaseData:
         # Extension (BASELINE configs[3], SURVEY 3.4): rebuild the kNN / task topology from the CURRENT positions on every
         # `build_data` call instead of re-using the placeholder of the first batch (rope_tasks_data.py:224-225,251 builds
         # once).  Off by default - parity runs use the reference's build-once rule.  Two ways (see `refresh_in_place`):
-        #   * in place: radius INTERNAL edges, consumed by the fused 16-bit path - the placeholder of the batch size is
-        #     kept and its position- / num_valid-dependent edge types are rewritten on the device, no host sync, so a
-        #     captured CUDA graph (Learner.capture) rebuilds the topology on every replay;
-        #   * eagerly (any other combination, kNN included): the placeholder is dropped and rebuilt at exact size, with
-        #     host syncs - not capturable.
+        #   * in place: radius INTERNAL edges consumed by the fused 16-bit path, or kNN INTERNAL edges with `knn_in_place`
+        #     - the placeholder of the batch size is kept and its position- / num_valid-dependent edge types are rewritten
+        #     on the device, no host sync, so a captured CUDA graph (Learner.capture, capture_act) rebuilds the topology on
+        #     every replay;
+        #   * eagerly (any other combination): the placeholder is dropped and rebuilt at exact size, with host syncs - not
+        #     capturable.
         self.rebuild_every_call = False
+        # Opt-in, with rebuild_every_call: rebuild kNN INTERNAL edges in place (ops.refresh_knn_edge_set).  Without
+        # num_valid (rope) the set stays exact-size, so every precision and edge path consumes it; with num_valid (rigid)
+        # it has a fixed capacity and needs the fused 16-bit path.  As with radius edges, pruning then keeps every row of
+        # the node type and an edge type without edges still runs its convolution; the eager rebuild recomputes the
+        # live rows per topology and skips such an edge type, as the reference does.
+        self.knn_in_place = False
         # set by the policy wrapper: True when the model consumes fixed-capacity edge sets (HEPi)
         self.consumer_accepts_capacity = False
         self._placeholders: Dict[int, GraphBatch] = {}
@@ -112,10 +120,15 @@ class BaseData:
 
     # ---- public entry point (base_data.py:45-55) ----------------------------------------------------
     def refresh_in_place(self) -> bool:
-        """True when `rebuild_every_call` rewrites the topology in place on the device (capturable): radius INTERNAL
-        edges, edges built, a model that accepts fixed-capacity edge sets, and the fused 16-bit edge path."""
-        return (self.rebuild_every_call and self.internal_edges == "radius" and self.build_edges
-                and self.consumer_accepts_capacity and ops.fused_edge_enabled())
+        """True when `rebuild_every_call` rewrites the topology in place on the device (capturable): edges built, a model
+        that accepts refreshed edge sets (HEPi), and either radius INTERNAL edges on the fused 16-bit edge path or kNN
+        INTERNAL edges with `knn_in_place`, exact-size without num_valid, on the fused 16-bit path with it."""
+        if not (self.rebuild_every_call and self.build_edges and self.consumer_accepts_capacity):
+            return False
+        if self.internal_edges == "radius":
+            return ops.fused_edge_enabled()
+        return (self.knn_in_place and self.INTERNAL_MODE == "knn"
+                and (not self.HAS_NUM_VALID or ops.fused_edge_enabled()))
 
     def build_data(self, *args, **kwargs):
         inputs = self._preprocess_input(*args, **kwargs)
@@ -188,8 +201,11 @@ class BaseData:
             src, _, dst = et
             if src not in kept or dst not in kept or not self.build_edges:
                 continue
-            # fixed capacity for what depends on the positions (INTERNAL) or on num_valid (TASK of the rigid tasks)
+            # rewritten in place: what depends on the positions (INTERNAL) or on num_valid (TASK of the rigid tasks)
             refreshed = refresh and (et == e_int or (et == e_task and num_valid is not None))
+            if et == e_int and refreshed and self.internal_edges == "knn":
+                g.add_edge_set(et, ops.knn_edge_set(pts, num_valid, self.knn_k), refreshed=True)
+                continue
             if et == e_int:
                 if self.INTERNAL_MODE == "knn" and self.internal_edges == "radius":
                     coo, ptr = self._radius_edges(pts, num_valid, refreshed)
@@ -205,7 +221,7 @@ class BaseData:
                     ptr = torch.zeros(B + 1, dtype=torch.int64, device=device)
             else:
                 coo, ptr = ops.dense_edges(1, B, P, A, device, num_valid=num_valid, capacity=refreshed)
-            g.add_edge_type(et, coo, ptr, refreshed=refreshed)
+            g.add_edge_type(et, coo, ptr, refreshed=refreshed, exact=not refreshed)
         for t in kept:  # HeteroNodeCategorical: one-hot over the PRE-subgraph type list (transforms.py:43-76)
             oh = torch.zeros(B * npg[t], len(self.ALL_NODE_TYPES), device=device)
             oh[:, list(self.ALL_NODE_TYPES).index(t)] = 1
@@ -232,6 +248,9 @@ class BaseData:
         e_int = self.EDGE_TYPES[0]
         pts = position_vectors[self.PARTICLE_TYPE]
         for et in g.refreshed_edge_types:
+            if et == e_int and self.internal_edges == "knn":
+                ops.refresh_knn_edge_set(g.edge_sets[et], pts, num_valid, self.knn_k)
+                continue
             if et == e_int:
                 coo, ptr = self._radius_edges(pts, num_valid, True)
             else:

@@ -66,8 +66,8 @@ class GraphBatch:
         self.output_mask_key: Optional[str] = None
         self.output_mask: slice = slice(None)
         self.homo_batch = None
-        # edge types held in fixed-capacity sets that the data builder refreshes in place from every batch's positions
-        # (BaseData.rebuild_every_call with radius edges on the fused 16-bit path); their row sets never enter pruning
+        # edge types whose sets the data builder refreshes in place from every batch's positions (BaseData.refresh_in_place:
+        # radius edges, or kNN edges with knn_in_place); their row sets never enter pruning
         self.refreshed_edge_types: set = set()
         self._homo_cache: Dict[str, ops.EdgeSet] = {}  # shared by every shallow copy of this topology
 
@@ -94,12 +94,17 @@ class GraphBatch:
             off += self.nodes_per_graph[t]
         return out
 
-    def add_edge_type(self, et: EdgeType, coo: torch.Tensor, edge_ptr: torch.Tensor, refreshed: bool = False):
-        """`refreshed`: `coo` is a fixed-capacity buffer and the data builder rewrites the edge set in place later."""
+    def add_edge_type(self, et: EdgeType, coo: torch.Tensor, edge_ptr: torch.Tensor, refreshed: bool = False,
+                      exact: bool = True):
+        """`exact=False`: `coo` is a fixed-capacity buffer.  `refreshed`: see `add_edge_set`."""
         src, _, dst = et
+        self.add_edge_set(et, ops.build_edge_set(coo, edge_ptr, self.num_graphs, self.nodes_per_graph[src],
+                                                 self.nodes_per_graph[dst], exact=exact), refreshed)
+
+    def add_edge_set(self, et: EdgeType, es: ops.EdgeSet, refreshed: bool = False):
+        """`refreshed`: the data builder rewrites `es` in place from every batch (exact-size or fixed-capacity)."""
         self.edge_types.append(et)
-        self.edge_sets[et] = ops.build_edge_set(coo, edge_ptr, self.num_graphs, self.nodes_per_graph[src],
-                                                self.nodes_per_graph[dst], exact=not refreshed)
+        self.edge_sets[et] = es
         if refreshed:
             self.refreshed_edge_types.add(et)
 

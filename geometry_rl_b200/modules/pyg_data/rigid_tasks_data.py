@@ -34,6 +34,7 @@ class RigidTasksData(BaseData):
     EDGE_TYPES = (("object_geometry", "internal", "object_geometry"), ("grippers", "agent", "grippers"),
                   ("object_geometry", "task", "grippers"))
     HAS_INFOS = True
+    HAS_NUM_VALID = True
 
     def _kept_node_types(self):
         # rigid_tasks_data.py:91: every node type except TARGET

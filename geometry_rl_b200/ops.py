@@ -199,6 +199,49 @@ def knn_graph(pos: torch.Tensor, num_valid: Optional[torch.Tensor], k: int):
     return coo[:, :E], edge_ptr
 
 
+def knn_edge_set(pos: torch.Tensor, num_valid: Optional[torch.Tensor], k: int, capacity: Optional[int] = None) -> EdgeSet:
+    """The kNN graph of `knn_graph` as a complete `EdgeSet` (src-sorted pairs included), written by one kernel
+    (grl_knn_topology) with no host read; every array equals what knn_graph -> build_edge_set -> src_sorted_pairs
+    yield.  `refresh_knn_edge_set` rewrites it in place from new positions, inside a CUDA-graph capture too.
+
+    `capacity=None`: exact size when `num_valid` is None (n_edges = B*P*min(k, P-1), known from the shapes), otherwise a
+    fixed-capacity set (`exact=False`) of B*P*k edges, which no num_valid can overflow.  An explicit `capacity` gives a
+    fixed-capacity set of that size (at least B*P*min(k, P-1)).  Unlike knn_graph, non-finite positions are accepted: a
+    NaN distance ranks as +inf (see grl_knn_topology)."""
+    B, P, _ = pos.shape
+    kk = max(0, min(k, P - 1))
+    exact = capacity is None and num_valid is None
+    if capacity is None:
+        capacity = B * P * kk if exact else B * P * k
+    elif capacity < B * P * kk:
+        raise ValueError(f"knn_edge_set: capacity {capacity} < B*P*min(k,P-1) = {B * P * kk}")
+    E, dev = int(capacity), pos.device
+    i32 = lambda n: torch.empty(n, dtype=torch.int32, device=dev)  # noqa: E731
+    coo = torch.empty(2, max(E, 1), dtype=torch.int64, device=dev)[:, :E]
+    es = EdgeSet(B * P, B * P, E, coo, torch.empty(B + 1, dtype=torch.int64, device=dev), i32(B * P + 1),
+                 i32(max(E, 1))[:E], i32(max(E, 1))[:E], i32(max(E, 1))[:E], i32(B * P + 1), i32(max(E, 1))[:E],
+                 s_src=i32(max(E, 1))[:E], s_dst=i32(max(E, 1))[:E], exact=exact)
+    refresh_knn_edge_set(es, pos, num_valid, k)
+    return es
+
+
+def refresh_knn_edge_set(es: EdgeSet, pos: torch.Tensor, num_valid: Optional[torch.Tensor], k: int) -> None:
+    """Rewrite a `knn_edge_set` in place (same tensors) from new positions / num_valid: grl_knn_edge_ptr, then
+    grl_knn_topology.  Device work only, so valid inside a CUDA-graph capture."""
+    pos = _f32c(pos)
+    B, P, _ = pos.shape
+    assert es.n_dst == es.n_src == B * P and es.edge_ptr.numel() == B + 1 and es.s_src is not None
+    if es.exact and num_valid is not None:
+        raise ValueError("refresh_knn_edge_set: an exact-size kNN set has every point valid; pass num_valid=None or "
+                         "build a fixed-capacity set")
+    if num_valid is not None:
+        num_valid = num_valid.to(torch.int32).clamp(0, P).contiguous()
+    L.call("grl_knn_edge_ptr", L.ptr(num_valid), B, P, k, L.ptr(es.edge_ptr))
+    L.call("grl_knn_topology", L.ptr(pos), L.ptr(num_valid), L.ptr(es.edge_ptr), B, P, k, es.n_edges, L.ptr_any(es.coo),
+           es.coo.stride(0), L.ptr(es.rowptr_dst), L.ptr(es.edge_src), L.ptr(es.edge_dst), L.ptr(es.eid_coo),
+           L.ptr(es.rowptr_src), L.ptr(es.src_eid), L.ptr(es.s_src), L.ptr(es.s_dst))
+
+
 def radius_neighbors(pos: torch.Tensor, num_valid: Optional[torch.Tensor], radius: float, max_neighbors: int):
     pos = _f32c(pos)
     B, P, _ = pos.shape

@@ -69,6 +69,21 @@ int grl_knn_edge_ptr(const int32_t* num_valid, int B, int P, int k, int64_t* edg
 int grl_knn_graph(const float* pos, const int32_t* num_valid, const int64_t* edge_ptr, int B, int P, int k,
                   int64_t* coo, int64_t coo_row_stride, grl_stream_t stream);
 
+/* Every layout of the kNN edge set of grl_knn_graph in one launch, with no host read (usable inside a CUDA graph):
+ * the coalesced COO (coo [2][capacity], coo_row_stride >= capacity), the dst-sorted CSR (rowptr_dst [B*P+1], edge_src,
+ * edge_dst, eid_coo) and the src-sorted CSR (rowptr_src [B*P+1], src_eid, and, when non-NULL, the src-sorted endpoint
+ * pairs s_src / s_dst), exactly as grl_knn_graph -> grl_csr_build (both keys) -> gathers lay them out.  edge_ptr comes
+ * from grl_knn_edge_ptr with the same num_valid and k.  capacity >= B*P*min(k,P-1); entries [edge_ptr[B], capacity)
+ * hold 0 in coo, edge_src, eid_coo and src_eid, and in edge_dst, s_src and s_dst the node ids a gather through those
+ * zeros reads (coo[1][0], edge_src[0], edge_dst[0]).  Candidates are ranked by (squared distance, index) with a NaN
+ * distance ranked as +inf, so every valid centre gets exactly min(k, P_b-1) neighbours and the edges written always
+ * equal edge_ptr, whatever the positions hold; for finite distances the neighbours are those of grl_knn_graph.
+ * With capacity 0 the per-edge arrays may be NULL. */
+int grl_knn_topology(const float* pos, const int32_t* num_valid, const int64_t* edge_ptr, int B, int P, int k,
+                     int64_t capacity, int64_t* coo, int64_t coo_row_stride, int32_t* rowptr_dst, int32_t* edge_src,
+                     int32_t* edge_dst, int32_t* eid_coo, int32_t* rowptr_src, int32_t* src_eid, int32_t* s_src,
+                     int32_t* s_dst, grl_stream_t stream);
+
 /* Radius graph (extension, no reference counterpart; SURVEY §3.4): neighbours within `radius`,
  * at most max_neighbors nearest, same output convention but into a PADDED buffer:
  * nbr[B][P][max_neighbors] (local index or -1), cnt[B][P]. */
