@@ -97,6 +97,14 @@ class GrlReadoutDesc(C.Structure):
                 ("grad_latent", _fp), ("grad_partials", _fp), ("n_partials", _i32)]
 
 
+class GrlHomoPart(C.Structure):
+    _fields_ = [("coo", _fp), ("edge_ptr", _fp), ("coo_row_stride", C.c_int64), ("n_src", _i32), ("n_dst", _i32),
+                ("off_src", _i32), ("off_dst", _i32)]
+
+
+HOMO_MAX_PARTS = 8  # GRL_MAX_HOMO_PARTS
+
+
 class GrlActDesc(C.Structure):
     _fields_ = [("batch", _i32), ("num_rows", _i32), ("action_dim", _i32), ("hidden_dim", _i32), ("post_fc", _i32),
                 ("contextual_std", _i32), ("use_tanh_mean", _i32), ("deterministic", _i32), ("rank", _i32),
@@ -133,6 +141,9 @@ SIGNATURES = {
     "grl_radius_graph": (C.c_int, [_fp, _fp, _fp, C.c_int, C.c_int, C.c_int, _fp, C.c_int64, C.c_int64, _fp]),
     "grl_dense_edges": (C.c_int, [C.c_int, _fp, _fp, C.c_int, C.c_int, C.c_int, _fp, C.c_int64, _fp]),
     "grl_csr_build": (C.c_int, [_fp, C.c_int64, _fp, C.c_int, C.c_int, C.c_int, _fp, _fp, _fp, _fp]),
+    "grl_homo_merge": (C.c_int, [C.POINTER(GrlHomoPart), C.c_int, C.c_int, C.c_int, C.c_int64, _fp, _fp, C.c_int64, _fp]),
+    "grl_sub_edge_set": (C.c_int, [_fp, _fp, _fp, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int64, _fp, _fp, _fp,
+                                   _fp, _fp, _fp, _fp, _fp, C.c_int64, _fp]),
     "grl_embed_fwd": (C.c_int, [C.POINTER(GrlEmbedDesc), _fp]),
     "grl_embed_bwd": (C.c_int, [C.POINTER(GrlEmbedDesc), _fp]),
     "grl_edge_basis_fwd": (C.c_int, [C.POINTER(GrlBasisDesc), _fp]),

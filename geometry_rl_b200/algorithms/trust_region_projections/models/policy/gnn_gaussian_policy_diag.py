@@ -51,6 +51,7 @@ class GNNGaussianPolicyDiag(nn.Module):
         self.gnn = gnn
         # fixed-capacity, in-place refreshed topology (BaseData.refresh_in_place) only for a model that consumes it
         hyper_data.consumer_accepts_capacity = bool(getattr(gnn, "accepts_capacity_edge_sets", False))
+        hyper_data.consumer_accepts_homogeneous_capacity = bool(getattr(gnn, "accepts_capacity_homogeneous_view", False))
 
     # ---- forward ---------------------------------------------------------------------------------
     def gnn_forward(self, *args, train=True):

@@ -153,11 +153,11 @@ class PolicyOperator(nn.Module):
         if hd.rebuild_every_call and not hd.refresh_in_place():
             raise ValueError(
                 "capture_act: the data builder rebuilds its topology eagerly on every call (rebuild_every_call with kNN "
-                "edges without knn_in_place, a task with num_valid on the fp32 or unfused path, or a model other than "
-                "HEPi), which reads sizes on the host and cannot be replayed; a captured act rebuilds kNN INTERNAL edges "
-                "with `hyper_data.knn_in_place = True` (rope: any precision; rigid: fused 16-bit path) and radius "
-                "INTERNAL edges on the fused 16-bit path (internal_edges='radius', ops.set_precision('bf16')) - "
-                "otherwise use `act`")
+                "edges without knn_in_place, a task with num_valid or an EMPN policy on the fp32 or unfused path, radius "
+                "edges with EMPN, or a model other than HEPi and EMPN), which reads sizes on the host and cannot be "
+                "replayed; a captured act rebuilds kNN INTERNAL edges with `hyper_data.knn_in_place = True` (HEPi rope: "
+                "any precision; HEPi rigid and EMPN: fused 16-bit path) and, for HEPi, radius INTERNAL edges on the "
+                "fused 16-bit path (internal_edges='radius', ops.set_precision('bf16')) - otherwise use `act`")
         self._act_static = [td_get(example_td, k).clone() for k in self.in_keys]
         with torch.no_grad():
             self.get_dist(dict(zip(self.in_keys, self._act_static)))  # the one-time calibration, if still pending

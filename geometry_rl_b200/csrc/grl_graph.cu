@@ -463,6 +463,130 @@ __global__ void __launch_bounds__(128) csr_build_kernel(const int64_t* __restric
   }
 }
 
+struct HomoParts {
+  GrlHomoPart p[GRL_MAX_HOMO_PARTS];
+  int n;
+};
+
+__device__ __forceinline__ int64_t homo_ptr(const HomoParts& hp, int b) {
+  int64_t s = 0;
+  for (int t = 0; t < hp.n; ++t) s += hp.p[t].edge_ptr[b];
+  return s;
+}
+
+// One thread per output position p of the merged COO (grid-stride): the graph b owning p is found by a binary search
+// over the merged edge_ptr (summed from the parts on the fly), then the part and the edge inside it by walking the
+// parts' counts of graph b.  Threads p <= B also write edge_ptr[p].
+__global__ void __launch_bounds__(256) homo_merge_kernel(HomoParts hp, int B, int n_tot, int64_t capacity,
+                                                         int64_t* __restrict__ edge_ptr, int64_t* __restrict__ coo,
+                                                         int64_t row_stride) {
+  const int64_t e_end = homo_ptr(hp, B);
+  const int64_t n = capacity > (int64_t)B + 1 ? capacity : (int64_t)B + 1;
+  for (int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; p < n; p += (int64_t)gridDim.x * blockDim.x) {
+    if (p <= B) edge_ptr[p] = homo_ptr(hp, (int)p);
+    if (p >= capacity) continue;
+    if (p >= e_end) {
+      coo[p] = 0;
+      coo[row_stride + p] = 0;
+      continue;
+    }
+    int lo = 0, hi = B - 1;  // largest b with homo_ptr(b) <= p
+    while (lo < hi) {
+      const int mid = (lo + hi + 1) / 2;
+      if (homo_ptr(hp, mid) <= p) lo = mid; else hi = mid - 1;
+    }
+    const int b = lo;
+    int64_t r = p - homo_ptr(hp, b);
+    for (int t = 0; t < hp.n; ++t) {
+      const GrlHomoPart& q = hp.p[t];
+      const int64_t e0 = q.edge_ptr[b], c = q.edge_ptr[b + 1] - e0;
+      if (r >= c) {
+        r -= c;
+        continue;
+      }
+      const int64_t e = e0 + r, base = (int64_t)b * n_tot;
+      coo[p] = base + q.off_src + (q.coo[e] - (int64_t)b * q.n_src);
+      coo[row_stride + p] = base + q.off_dst + (q.coo[q.coo_row_stride + e] - (int64_t)b * q.n_dst);
+      break;
+    }
+  }
+}
+
+// sub_edge_ptr / sub_rowptr_dst of grl_sub_edge_set: the output rows of graph b are contiguous in the parent, so their
+// edges are the parent's edge range [rowptr_dst[b*n_tot+out_off], rowptr_dst[b*n_tot+out_off+n_out]).  One CTA,
+// sequential chunks of graphs per thread, like knn_edge_ptr_kernel.
+__global__ void sub_edge_ptr_kernel(const int32_t* __restrict__ rowptr_dst, int B, int n_tot, int out_off, int n_out,
+                                    int64_t* __restrict__ sub_edge_ptr, int32_t* __restrict__ sub_rowptr_dst) {
+  __shared__ long long part[1024];
+  const int tid = threadIdx.x, nt = blockDim.x;
+  const int per = (B + nt - 1) / nt;
+  const int b0 = tid * per, b1 = min(b0 + per, B);
+  auto row = [&](int b, int a) { return (long long)rowptr_dst[(size_t)b * n_tot + out_off + a]; };
+  long long s = 0;
+  for (int b = b0; b < b1; ++b) s += row(b, n_out) - row(b, 0);
+  part[tid] = s;
+  __syncthreads();
+  if (tid == 0) {
+    long long run = 0;
+    for (int i = 0; i < nt; ++i) { const long long t = part[i]; part[i] = run; run += t; }
+    sub_edge_ptr[B] = run;
+    sub_rowptr_dst[(size_t)B * n_out] = (int32_t)run;
+  }
+  __syncthreads();
+  long long run = part[tid];
+  for (int b = b0; b < b1; ++b) {
+    sub_edge_ptr[b] = run;
+    const long long base = row(b, 0);
+    for (int a = 0; a < n_out; ++a) sub_rowptr_dst[(size_t)b * n_out + a] = (int32_t)(run + row(b, a) - base);
+    run += row(b, n_out) - base;
+  }
+}
+
+struct SubEdgeOut {
+  int64_t* eids;
+  int32_t *eids32, *edge_src, *edge_dst, *edge_dst_parent;
+  int64_t* pairs;
+  int64_t pairs_row_stride;
+};
+
+__device__ __forceinline__ int out_rank(int32_t node, int n_tot, int out_off, int n_out) {
+  const int g = node / n_tot, l = node - g * n_tot - out_off;
+  return (l >= 0 && l < n_out) ? g * n_out + l : -1;
+}
+
+// Per-edge arrays of grl_sub_edge_set, one thread per sub edge q and per parent edge (grid-stride over the larger).
+__global__ void __launch_bounds__(256) sub_edges_kernel(const int32_t* __restrict__ rowptr_dst,
+                                                        const int32_t* __restrict__ edge_src,
+                                                        const int32_t* __restrict__ edge_dst, int64_t n_edges, int B,
+                                                        int n_tot, int out_off, int n_out, int64_t capacity,
+                                                        const int64_t* __restrict__ sub_edge_ptr, SubEdgeOut o) {
+  const int64_t e_par = rowptr_dst[(size_t)B * n_tot], e_sub = sub_edge_ptr[B];
+  const int64_t n = capacity > n_edges ? capacity : n_edges;
+  auto rank = [&](int64_t e) { return e < e_par ? out_rank(edge_dst[e], n_tot, out_off, n_out) : -1; };
+  for (int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; q < n; q += (int64_t)gridDim.x * blockDim.x) {
+    if (q < n_edges) o.edge_dst_parent[q] = rank(q);
+    if (q >= capacity) continue;
+    int64_t e = 0;
+    int32_t src = 0;
+    if (q < e_sub) {
+      int lo = 0, hi = B - 1;  // largest b with sub_edge_ptr[b] <= q
+      while (lo < hi) {
+        const int mid = (lo + hi + 1) / 2;
+        if (sub_edge_ptr[mid] <= q) lo = mid; else hi = mid - 1;
+      }
+      e = rowptr_dst[(size_t)lo * n_tot + out_off] + (q - sub_edge_ptr[lo]);
+      src = edge_src[e];
+    }
+    const int dst = rank(e);
+    o.eids[q] = e;
+    o.eids32[q] = (int32_t)e;
+    o.edge_src[q] = src;
+    o.edge_dst[q] = dst;
+    o.pairs[q] = src;
+    o.pairs[o.pairs_row_stride + q] = dst;
+  }
+}
+
 }  // namespace grl
 
 extern "C" {
@@ -563,6 +687,52 @@ int grl_csr_build(const int64_t* coo, int64_t coo_row_stride, const int64_t* edg
   grl::csr_build_kernel<<<grid, 128, (n_key + 1) * sizeof(int), (cudaStream_t)stream>>>(coo, coo_row_stride, edge_ptr, B,
                                                                                        n_key, key_row, rowptr, other, eid);
   return grl::check_launch("grl_csr_build");
+}
+
+int grl_homo_merge(const GrlHomoPart* parts, int n_parts, int B, int n_tot, int64_t capacity, int64_t* edge_ptr,
+                   int64_t* coo, int64_t coo_row_stride, grl_stream_t stream) {
+  GRL_REQUIRE(parts && edge_ptr && B > 0 && n_tot > 0 && capacity >= 0 && (capacity == 0 || coo) &&
+                  coo_row_stride >= capacity,
+              GRL_EINVAL, "grl_homo_merge: bad arguments");
+  GRL_REQUIRE(n_parts >= 0 && n_parts <= GRL_MAX_HOMO_PARTS, GRL_EUNSUPPORTED, "grl_homo_merge: n_parts=%d not in [0,%d]",
+              n_parts, GRL_MAX_HOMO_PARTS);
+  grl::HomoParts hp{};
+  hp.n = n_parts;
+  for (int t = 0; t < n_parts; ++t) {
+    const GrlHomoPart& q = parts[t];
+    GRL_REQUIRE(q.edge_ptr && q.n_src > 0 && q.n_dst > 0 && q.off_src >= 0 && q.off_dst >= 0 &&
+                    q.off_src + q.n_src <= n_tot && q.off_dst + q.n_dst <= n_tot,
+                GRL_EINVAL, "grl_homo_merge: bad part %d", t);
+    hp.p[t] = q;
+  }
+  const int64_t n = std::max<int64_t>(capacity, (int64_t)B + 1);
+  const int grid = (int)std::min<int64_t>((n + 255) / 256, 16LL * grl::sm_count());
+  grl::homo_merge_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(hp, B, n_tot, capacity, edge_ptr, coo, coo_row_stride);
+  return grl::check_launch("grl_homo_merge");
+}
+
+int grl_sub_edge_set(const int32_t* rowptr_dst, const int32_t* edge_src, const int32_t* edge_dst, int64_t n_edges, int B,
+                     int n_tot, int out_off, int n_out, int64_t capacity, int64_t* sub_edge_ptr, int32_t* sub_rowptr_dst,
+                     int64_t* eids, int32_t* eids32, int32_t* sub_edge_src, int32_t* sub_edge_dst,
+                     int32_t* edge_dst_parent, int64_t* pairs, int64_t pairs_row_stride, grl_stream_t stream) {
+  GRL_REQUIRE(rowptr_dst && sub_edge_ptr && sub_rowptr_dst && B > 0 && n_tot > 0 && n_out > 0 && out_off >= 0 &&
+                  out_off + n_out <= n_tot && n_edges >= 0 && capacity >= 0 && pairs_row_stride >= capacity &&
+                  (n_edges == 0 || (edge_src && edge_dst && edge_dst_parent)) &&
+                  (capacity == 0 || (eids && eids32 && sub_edge_src && sub_edge_dst && pairs)),
+              GRL_EINVAL, "grl_sub_edge_set: bad arguments");
+  GRL_REQUIRE((int64_t)B * n_tot < INT32_MAX && n_edges <= INT32_MAX && capacity <= INT32_MAX, GRL_EUNSUPPORTED,
+              "grl_sub_edge_set: sizes exceed the int32 node / edge ids");
+  grl::sub_edge_ptr_kernel<<<1, 1024, 0, (cudaStream_t)stream>>>(rowptr_dst, B, n_tot, out_off, n_out, sub_edge_ptr,
+                                                                 sub_rowptr_dst);
+  int rc = grl::check_launch("grl_sub_edge_set");
+  if (rc != GRL_OK) return rc;
+  const int64_t n = std::max(capacity, n_edges);
+  if (n == 0) return GRL_OK;
+  const int grid = (int)std::min<int64_t>((n + 255) / 256, 16LL * grl::sm_count());
+  grl::SubEdgeOut o{eids, eids32, sub_edge_src, sub_edge_dst, edge_dst_parent, pairs, pairs_row_stride};
+  grl::sub_edges_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(rowptr_dst, edge_src, edge_dst, n_edges, B, n_tot, out_off,
+                                                                n_out, capacity, sub_edge_ptr, o);
+  return grl::check_launch("grl_sub_edge_set");
 }
 
 }  // extern "C"

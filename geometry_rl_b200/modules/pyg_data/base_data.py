@@ -101,6 +101,9 @@ class BaseData:
         self.knn_in_place = False
         # set by the policy wrapper: True when the model consumes fixed-capacity edge sets (HEPi)
         self.consumer_accepts_capacity = False
+        # set by the policy wrapper: True when the model reads only the homogeneous views of GraphBatch (EMPN), which are
+        # then merged on the device from fixed-capacity edge sets and refreshed with them
+        self.consumer_accepts_homogeneous_capacity = False
         self._placeholders: Dict[int, GraphBatch] = {}
         self._example_data: Optional[GraphBatch] = None
 
@@ -122,8 +125,14 @@ class BaseData:
     def refresh_in_place(self) -> bool:
         """True when `rebuild_every_call` rewrites the topology in place on the device (capturable): edges built, a model
         that accepts refreshed edge sets (HEPi), and either radius INTERNAL edges on the fused 16-bit edge path or kNN
-        INTERNAL edges with `knn_in_place`, exact-size without num_valid, on the fused 16-bit path with it."""
-        if not (self.rebuild_every_call and self.build_edges and self.consumer_accepts_capacity):
+        INTERNAL edges with `knn_in_place`, exact-size without num_valid, on the fused 16-bit path with it.  A model that
+        reads the homogeneous view (EMPN) needs kNN INTERNAL edges with `knn_in_place` on the fused 16-bit path."""
+        if not (self.rebuild_every_call and self.build_edges):
+            return False
+        if self.consumer_accepts_homogeneous_capacity and not self.consumer_accepts_capacity:
+            return (self.knn_in_place and self.internal_edges == "knn" and self.INTERNAL_MODE == "knn"
+                    and ops.fused_edge_enabled())
+        if not self.consumer_accepts_capacity:
             return False
         if self.internal_edges == "radius":
             return ops.fused_edge_enabled()
@@ -257,6 +266,7 @@ class BaseData:
                 coo, ptr = ops.dense_edges(1, batch_size, pts.shape[1], position_vectors[self.ACTUATOR_TYPE].shape[1],
                                            device, num_valid=num_valid, capacity=True)
             ops.refresh_edge_set(g.edge_sets[et], coo, ptr)
+        g.refresh_homogeneous()
 
     def _update_placeholders(self, position_vectors, norm_position_vectors, device, **ignored) -> GraphBatch:
         data = self._example_data.shallow_copy()

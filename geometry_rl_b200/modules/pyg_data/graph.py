@@ -36,9 +36,11 @@ class PrunedHomo:
     latent row never reaches an output, so neither the forward values read by anybody nor any gradient change.
     The edge order (dst-sorted, ties in COO order) is that of the full set: the renumbering is monotone.
     `sub` is the bipartite set "live nodes -> output nodes" of the LAST layer, whose result is only read at the
-    output nodes (ponita_gcn.py:132-146 slices `output_mask` out of the last latent)."""
-    live_ids: torch.Tensor  # [n_live] int64: full (padded) node index of every live node, ascending
-    live_ids32: torch.Tensor  # the same as int32 (GrlEmbedDesc.node_ids)
+    output nodes (ponita_gcn.py:132-146 slices `output_mask` out of the last latent).
+    With refreshed edge types (see `homogeneous`) every row is live: `es` is the full homogeneous set, `live_ids` and
+    `live_ids32` are None (identity renumbering), and only `sub` restricts the last layer; both follow every refresh."""
+    live_ids: Optional[torch.Tensor]  # [n_live] int64: full (padded) node index of every live node, ascending
+    live_ids32: Optional[torch.Tensor]  # the same as int32 (GrlEmbedDesc.node_ids)
     es: ops.EdgeSet  # n_src = n_dst = n_live, all E edges, compact node ids
     sub: ops.SubEdgeSet
 
@@ -123,7 +125,14 @@ class GraphBatch:
     def homogeneous(self) -> ops.EdgeSet:
         """All edge types merged into one graph whose nodes are the node types concatenated per graph
         (node_types order); per graph the edges keep edge-type insertion order, as to_homogeneous()
-        yields them, so the segmented sums see the same edge order as the reference."""
+        yields them, so the segmented sums see the same edge order as the reference.
+
+        With refreshed edge types the view is merged on the device (ops.homogeneous_edge_set, no host read): sized for
+        the sum of the edge types' capacities, exact only when every edge type is, and rewritten in place by
+        `refresh_homogeneous` after each refresh of the edge types."""
+        if "homo" not in self._homo_cache and self.refreshed_edge_types:
+            self._homo_cache["homo"] = ops.homogeneous_edge_set(self._homo_parts(), self.num_graphs,
+                                                                sum(self.nodes_per_graph.values()))
         if "homo" not in self._homo_cache:
             for es in self.edge_sets.values():
                 ops.require_exact(es, "GraphBatch.homogeneous")
@@ -152,8 +161,26 @@ class GraphBatch:
             self._homo_cache["homo"] = ops.build_edge_set(coo[:, :E], homo_ptr, B, n_tot, n_tot)
         return self._homo_cache["homo"]
 
+    def _homo_parts(self):
+        offs = self.node_offsets
+        return [(self.edge_sets[et], offs[et[0]], offs[et[2]]) for et in self.edge_types]
+
+    def _output_rows(self):
+        """(first output row, output rows, sub-edge capacity) per graph: output rows are one contiguous range of the
+        concatenated node types, and the capacity sums the edge types that end in it."""
+        n_tot = sum(self.nodes_per_graph.values())
+        start, stop, _ = self.output_mask.indices(n_tot)
+        offs = self.node_offsets
+        cap = sum(es.n_edges for (_, _, dst), es in self.edge_sets.items() if start <= offs[dst] < stop)
+        return start, stop - start, cap
+
     def homogeneous_pruned(self) -> PrunedHomo:
-        """See PrunedHomo.  Derived from `homogeneous()` with a handful of torch index ops, once per topology."""
+        """See PrunedHomo.  Derived from `homogeneous()` with a handful of torch index ops, once per topology; with
+        refreshed edge types, every row is kept and the last layer's sub set is derived on the device."""
+        if "pruned" not in self._homo_cache and self.refreshed_edge_types:
+            es = self.homogeneous()
+            start, n_out, cap = self._output_rows()
+            self._homo_cache["pruned"] = PrunedHomo(None, None, es, ops.sub_edge_set(es, start, n_out, cap))
         if "pruned" not in self._homo_cache:
             es = self.homogeneous()
             B, dev = self.num_graphs, self.device
@@ -178,6 +205,17 @@ class GraphBatch:
             sub = ops.build_sub_edge_set(compact, out_ids)
             self._homo_cache["pruned"] = PrunedHomo(live_ids, live_ids.to(torch.int32).contiguous(), compact, sub)
         return self._homo_cache["pruned"]
+
+    def refresh_homogeneous(self) -> None:
+        """Rewrite the homogeneous views built so far (`homogeneous`, `homogeneous_pruned`) from the refreshed edge
+        types, in place, on the device.  The data builder calls it after every in-place refresh of the edge types."""
+        homo = self._homo_cache.get("homo")
+        if homo is None or not self.refreshed_edge_types:
+            return
+        ops.refresh_homogeneous_edge_set(homo, self._homo_parts())
+        pruned = self._homo_cache.get("pruned")
+        if pruned is not None:
+            ops.refresh_sub_edge_set(pruned.sub, homo, self._output_rows()[0])
 
     # -- heterogeneous view without dead rows (HEPi) ---------------------------------------------------
     def hetero_pruned(self) -> PrunedHetero:

@@ -136,6 +136,9 @@ class SeparableFiberBundleConvNext(nn.Module):
 
     @torch.no_grad()
     def _callibration_factors(self, x, kernel_basis, fk_op, edge_set):
+        if not edge_set.exact:  # fixed-capacity topology: statistics over the real edges only (one count read)
+            edge_set = ops.exact_edge_set(edge_set)
+            kernel_basis = kernel_basis.on(edge_set) if isinstance(kernel_basis, ops.BasisSpec) else kernel_basis
         x1 = ops.aggregate_messages(x, kernel_basis, self.conv.kernel.weight, edge_set)
         x2 = torch.einsum("boc,opc->bpc", x1, fk_op) / 16
         std_in, std_1, std_2 = ops.calibration_std(x), ops.calibration_std(x1), ops.calibration_std(x2)

@@ -9,6 +9,10 @@ from .ponita.ponita import Ponita
 
 
 class PonitaGCN(torch.nn.Module):
+    # reads only GraphBatch.homogeneous() / homogeneous_pruned(), which are derived on the device from fixed-capacity,
+    # in-place refreshed edge sets (BaseData.refresh_in_place)
+    accepts_capacity_homogeneous_view = True
+
     def __init__(self, input_dim_node, output_dim, output_dim_vec, num_layers=2, hidden_dim=64, dropout=0.1, num_ori=20,
                  degree=2, widening_factor=4, attention=False, ponita_dim=3, only_upper_hemisphere=False, **ignored):
         super().__init__()
@@ -48,7 +52,7 @@ class PonitaGCN(torch.nn.Module):
             sc, vc, pos = sc.reshape(B * n_per_graph, -1), vc.reshape(B * n_per_graph, -1), pos.reshape(-1, 3)
             # the one-time calibration (ponita.py:178-192) takes statistics over ALL rows: that call runs dense
             pruned = graph.homogeneous_pruned() if (self.prune_dead_rows and not self.ponita.calibration_pending()) else None
-            if pruned is not None:
+            if pruned is not None and pruned.live_ids is not None:
                 pos = pos[pruned.live_ids]  # the embed kernel reads sc / vc rows in place through live_ids32
             else:
                 edge_set = graph.homogeneous()

@@ -137,6 +137,11 @@ class SubEdgeSet:
     edge_dst_parent: torch.Tensor  # [E_parent] int32: dst rank (0..n_dst-1) of every parent edge, -1 outside the subset
     s_src: Optional[torch.Tensor] = None  # [E_sub] int32: source (parent node id) of the q-th src-sorted sub-edge (lazy)
     s_dst: Optional[torch.Tensor] = None  # [E_sub] int32: destination rank of the q-th src-sorted sub-edge
+    edge_ptr: Optional[torch.Tensor] = None  # [B+1] int64: sub-edges of graph b (sets of `sub_edge_set` only)
+    # False: a fixed-capacity set (`sub_edge_set` of a fixed-capacity parent, rewritten in place by refresh_sub_edge_set).
+    # The real count is rowptr_dst[-1]; past it eids, eids32, edge_src hold 0 and edge_dst, src_eid_parent, s_src, s_dst
+    # what a gather through those zeros reads; edge_dst_parent is -1 past the parent's real count.
+    exact: bool = True
 
 
 def src_sorted_pairs(es: "EdgeSet", sub: Optional[SubEdgeSet] = None):
@@ -350,9 +355,15 @@ def refresh_edge_set(es: EdgeSet, coo: torch.Tensor, edge_ptr: torch.Tensor) -> 
     the same shape, cached src-sorted pairs included.  Device work only (no host sync): valid inside a CUDA-graph
     capture, whose replays then rebuild the topology from whatever the inputs hold."""
     assert not es.exact and tuple(coo.shape) == tuple(es.coo.shape) and edge_ptr.shape == es.edge_ptr.shape
-    B = es.edge_ptr.numel() - 1
     es.coo.copy_(coo)
     es.edge_ptr.copy_(edge_ptr)
+    _refresh_layouts(es, coo)
+
+
+def _refresh_layouts(es: EdgeSet, coo: torch.Tensor) -> None:
+    """Rewrite both CSRs (and the cached src-sorted pairs) of `es` from its COO and edge_ptr, in place; `coo` is a
+    [2, n_edges] int64 scratch buffer (row stride 1) that is overwritten."""
+    B = es.edge_ptr.numel() - 1
     _csr(es.coo, es.edge_ptr, B, es.n_dst // B, 1, (es.rowptr_dst, es.edge_src, es.eid_coo))
     torch.index_select(es.coo[1], 0, es.eid_coo.long(), out=coo[1])  # coo is a scratch buffer from here on
     es.edge_dst.copy_(coo[1])
@@ -363,6 +374,81 @@ def refresh_edge_set(es: EdgeSet, coo: torch.Tensor, edge_ptr: torch.Tensor) -> 
         idx = es.src_eid.long()
         torch.index_select(es.edge_src, 0, idx, out=es.s_src)
         torch.index_select(es.edge_dst, 0, idx, out=es.s_dst)
+
+
+def homogeneous_edge_set(parts, B: int, n_tot: int) -> EdgeSet:
+    """The edge types of a batched heterogeneous graph merged into one homogeneous `EdgeSet` on the device, with no host
+    read (grl_homo_merge, then the CSRs of build_edge_set).  `parts`: (EdgeSet, offset of its source node type, offset of
+    its destination node type) per edge type in insertion order; nodes are the node types concatenated per graph, n_tot
+    per graph.  The capacity is the sum of the parts' `n_edges`: for exact parts that is the merged count and the set is
+    exact, equal to what GraphBatch.homogeneous builds with torch ops; with any fixed-capacity part it is a
+    fixed-capacity set (`exact=False`).  `refresh_homogeneous_edge_set` rewrites it in place, inside a CUDA-graph capture
+    too."""
+    E, dev = sum(p.n_edges for p, _, _ in parts), parts[0][0].edge_ptr.device
+    i32 = lambda n: torch.empty(n, dtype=torch.int32, device=dev)  # noqa: E731
+    z32 = lambda n: torch.zeros(n, dtype=torch.int32, device=dev)  # noqa: E731
+    coo = torch.empty(2, max(E, 1), dtype=torch.int64, device=dev)[:, :E]
+    es = EdgeSet(B * n_tot, B * n_tot, E, coo, torch.empty(B + 1, dtype=torch.int64, device=dev), z32(B * n_tot + 1),
+                 i32(max(E, 1))[:E], i32(max(E, 1))[:E], i32(max(E, 1))[:E], z32(B * n_tot + 1), i32(max(E, 1))[:E],
+                 s_src=i32(max(E, 1))[:E], s_dst=i32(max(E, 1))[:E], exact=all(p.exact for p, _, _ in parts))
+    refresh_homogeneous_edge_set(es, parts)
+    return es
+
+
+def refresh_homogeneous_edge_set(es: EdgeSet, parts) -> None:
+    """Rewrite a `homogeneous_edge_set` in place (same tensors) from the current contents of its parts.  Device work
+    only, so valid inside a CUDA-graph capture."""
+    B = es.edge_ptr.numel() - 1
+    n_tot = es.n_dst // B
+    assert len(parts) <= L.HOMO_MAX_PARTS and es.n_edges == sum(p.n_edges for p, _, _ in parts)
+    desc = (L.GrlHomoPart * max(1, len(parts)))()
+    for i, (p, off_src, off_dst) in enumerate(parts):
+        assert p.edge_ptr.numel() == B + 1 and (p.n_edges == 0 or p.coo.stride(1) == 1)
+        desc[i] = L.GrlHomoPart(coo=L.ptr_any(p.coo) if p.n_edges > 0 else None, edge_ptr=L.ptr(p.edge_ptr),
+                                coo_row_stride=p.coo.stride(0), n_src=p.n_src // B, n_dst=p.n_dst // B, off_src=off_src,
+                                off_dst=off_dst)
+    L.call("grl_homo_merge", desc, len(parts), B, n_tot, es.n_edges, L.ptr(es.edge_ptr), L.ptr_any(es.coo),
+           es.coo.stride(0))
+    if es.n_edges > 0:
+        _refresh_layouts(es, torch.empty(2, es.n_edges, dtype=torch.int64, device=es.coo.device))
+
+
+def sub_edge_set(es: EdgeSet, out_off: int, n_out: int, capacity: int) -> SubEdgeSet:
+    """`build_sub_edge_set` on the device, with no host read, for output rows [out_off, out_off + n_out) of every graph
+    (graph-major) of a homogeneous `es` (grl_sub_edge_set, then grl_csr_build keyed on the source and gathers).
+    `capacity` bounds the sub-edges: the sum of the `n_edges` of the edge types that end in the output rows.  For an
+    exact `es` it must be the real count; the set is then exact and equals build_sub_edge_set(es, out_ids).  Otherwise it
+    is a fixed-capacity set (`exact=False`).  `refresh_sub_edge_set` rewrites it in place, inside a capture too."""
+    B = es.edge_ptr.numel() - 1
+    n_tot, E, dev = es.n_dst // B, int(capacity), es.edge_src.device
+    i32 = lambda n: torch.empty(n, dtype=torch.int32, device=dev)  # noqa: E731
+    out_ids = (torch.arange(B, device=dev)[:, None] * n_tot + out_off + torch.arange(n_out, device=dev)).reshape(-1)
+    sub = SubEdgeSet(es.n_src, B * n_out, E, out_ids, torch.empty(max(E, 1), dtype=torch.int64, device=dev)[:E],
+                     i32(max(E, 1))[:E], i32(B * n_out + 1), i32(max(E, 1))[:E], i32(max(E, 1))[:E],
+                     torch.zeros(es.n_src + 1, dtype=torch.int32, device=dev), i32(max(E, 1))[:E],
+                     i32(max(es.n_edges, 1))[:es.n_edges], s_src=i32(max(E, 1))[:E], s_dst=i32(max(E, 1))[:E],
+                     edge_ptr=torch.empty(B + 1, dtype=torch.int64, device=dev), exact=es.exact)
+    refresh_sub_edge_set(sub, es, out_off)
+    return sub
+
+
+def refresh_sub_edge_set(sub: SubEdgeSet, es: EdgeSet, out_off: int) -> None:
+    """Rewrite a `sub_edge_set` in place (same tensors) from the current contents of its parent `es`.  Device work only."""
+    B = es.edge_ptr.numel() - 1
+    n_tot, E, dev = es.n_dst // B, sub.n_edges, es.edge_src.device
+    assert sub.edge_ptr is not None and sub.n_src == es.n_src and sub.edge_dst_parent.numel() == es.n_edges
+    pairs = torch.empty(2, max(E, 1), dtype=torch.int64, device=dev)[:, :E]
+    L.call("grl_sub_edge_set", L.ptr(es.rowptr_dst), L.ptr(es.edge_src), L.ptr(es.edge_dst), es.n_edges, B, n_tot,
+           out_off, sub.n_dst // B, E, L.ptr(sub.edge_ptr), L.ptr(sub.rowptr_dst), L.ptr(sub.eids), L.ptr(sub.eids32),
+           L.ptr(sub.edge_src), L.ptr(sub.edge_dst), L.ptr(sub.edge_dst_parent), L.ptr_any(pairs), pairs.stride(0))
+    if E == 0:
+        return
+    eid = torch.empty(E, dtype=torch.int32, device=dev)
+    _csr(pairs, sub.edge_ptr, B, n_tot, 0, (sub.rowptr_src, torch.empty(E, dtype=torch.int32, device=dev), eid))
+    idx = eid.long()
+    torch.index_select(sub.eids32, 0, idx, out=sub.src_eid_parent)
+    torch.index_select(sub.edge_src, 0, idx, out=sub.s_src)
+    torch.index_select(sub.edge_dst, 0, idx, out=sub.s_dst)
 
 
 # ------------------------------------------------------------------------------------------------

@@ -118,6 +118,44 @@ int grl_dense_edges(int mode, const int32_t* num_valid, const int64_t* edge_ptr,
 int grl_csr_build(const int64_t* coo, int64_t coo_row_stride, const int64_t* edge_ptr, int B, int n_key, int key_row,
                   int32_t* rowptr, int32_t* other, int32_t* eid, grl_stream_t stream);
 
+/* One edge type of a batched heterogeneous graph as grl_homo_merge reads it: its graph-major COO (exact-size or
+ * fixed-capacity; only edges [edge_ptr[b], edge_ptr[b+1]) of each graph are read, so `coo` may be NULL for a type
+ * without edges), nodes per graph of its source / destination type, and the offsets of those node types in the
+ * per-graph concatenation of all node types. */
+typedef struct {
+  const int64_t* coo;      /* [2][coo_row_stride] */
+  const int64_t* edge_ptr; /* [B+1] */
+  int64_t coo_row_stride;
+  int32_t n_src, n_dst;
+  int32_t off_src, off_dst;
+} GrlHomoPart;
+#define GRL_MAX_HOMO_PARTS 8
+
+/* Merge the edge types into one homogeneous graph whose nodes are the node types concatenated per graph (n_tot per
+ * graph), with no host read (usable inside a CUDA graph).  `parts` is a HOST array of n_parts descriptors in edge-type
+ * insertion order.  Writes edge_ptr[b] = sum over parts of their edge_ptr[b], and the COO [2][capacity]
+ * (coo_row_stride >= capacity): graph b's edges at [edge_ptr[b], edge_ptr[b+1]), part blocks in order, each keeping its
+ * COO order, ids remapped to b*n_tot + offset + local id; entries [edge_ptr[B], capacity) are 0.  capacity must be at
+ * least the merged edge count (the sum of the parts' capacities always is). */
+int grl_homo_merge(const GrlHomoPart* parts, int n_parts, int B, int n_tot, int64_t capacity, int64_t* edge_ptr,
+                   int64_t* coo, int64_t coo_row_stride, grl_stream_t stream);
+
+/* Forward arrays of the sub edge set "every node -> output rows" of a homogeneous edge set (B graphs of n_tot nodes,
+ * dst-sorted CSR rowptr_dst [B*n_tot+1], edge_src / edge_dst [n_edges] in edge order) whose output rows are the
+ * n_out rows [out_off, out_off + n_out) of every graph, graph-major; no host read.  Writes
+ *   sub_edge_ptr [B+1] and sub_rowptr_dst [B*n_out+1] (the exclusive prefix of the output rows' in-degrees);
+ *   for sub edge q < capacity: eids / eids32 (position in the parent's edge order), sub_edge_src (parent node id),
+ *   sub_edge_dst (rank of the destination among the output rows), and pairs [2][pairs_row_stride] = (sub_edge_src,
+ *   sub_edge_dst) as int64, the COO grl_csr_build sorts by source for the backward half;
+ *   edge_dst_parent [n_edges]: the rank of every parent edge's destination, -1 when it is not an output row or the
+ *   edge lies past the parent's real count rowptr_dst[B*n_tot].
+ * Past the real sub count: eids, eids32 and sub_edge_src hold 0, sub_edge_dst holds edge_dst_parent[0] (-1 without
+ * parent edges).  capacity must be at least the real sub count. */
+int grl_sub_edge_set(const int32_t* rowptr_dst, const int32_t* edge_src, const int32_t* edge_dst, int64_t n_edges, int B,
+                     int n_tot, int out_off, int n_out, int64_t capacity, int64_t* sub_edge_ptr, int32_t* sub_rowptr_dst,
+                     int64_t* eids, int32_t* eids32, int32_t* sub_edge_src, int32_t* sub_edge_dst,
+                     int32_t* edge_dst_parent, int64_t* pairs, int64_t pairs_row_stride, grl_stream_t stream);
+
 /* ------------------------------------------------------------------------------------------
  * K2  fused equivariant message passing (forward and backward)
  * replaces hepi.py:109-123,136-171 / ponita/conv.py:71-149 / ponita/ponita.py:149-185,219-230:

@@ -7,6 +7,9 @@ every step, for rope (rope_shaping_hepi_trpl_cfg) and rigid insertion (rigid_ins
   rebuild_only_graphed   the in-place refresh alone (build_data of the policy graph), captured and replayed
   knn_rebuild_graphed_fp32  rope only: the in-place rebuild on the strict fp32 path (exact-size set, replay)
 
+and for the EMPN policy (rigid_pushing_multi_empn_trpl_cfg), whose in-place rebuild also merges the homogeneous view and
+the last layer's sub set on the device (GraphBatch.refresh_homogeneous), the first four.
+
 Prints one JSON object (card name and power limit included) and writes it to --out.  Single process; data-parallel runs
 are not covered here.  Usage: python tools/knn_rebuild_bench.py --out profiles/r04_knn_rebuild.json"""
 import argparse
@@ -20,7 +23,8 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 
 from tools.radius_rebuild_bench import card, timed  # noqa: E402
 
-WORKLOADS = {"rope_shaping_hepi_trpl_cfg": 2048, "rigid_insertion_multi_hepi_trpl_cfg": 8192}
+WORKLOADS = {"rope_shaping_hepi_trpl_cfg": 2048, "rigid_insertion_multi_hepi_trpl_cfg": 8192,
+             "rigid_pushing_multi_empn_trpl_cfg": 4096}
 
 
 def run_variant(name, B, steps, rebuild, in_place, graphed, precision, dev):
@@ -79,6 +83,7 @@ def main():
     ap.add_argument("--steps", type=int, default=50)
     ap.add_argument("--rope-minibatch", type=int, default=WORKLOADS["rope_shaping_hepi_trpl_cfg"])
     ap.add_argument("--rigid-minibatch", type=int, default=WORKLOADS["rigid_insertion_multi_hepi_trpl_cfg"])
+    ap.add_argument("--empn-minibatch", type=int, default=WORKLOADS["rigid_pushing_multi_empn_trpl_cfg"])
     ap.add_argument("--out", default=None)
     args = ap.parse_args()
     if not torch.cuda.is_available():
@@ -89,7 +94,8 @@ def main():
     variants = {"knn_build_once": (False, False, True, "bf16"), "knn_rebuild_graphed": (True, True, True, "bf16"),
                 "knn_rebuild_eager": (True, False, False, "bf16")}
     for name, B in (("rope_shaping_hepi_trpl_cfg", args.rope_minibatch),
-                    ("rigid_insertion_multi_hepi_trpl_cfg", args.rigid_minibatch)):
+                    ("rigid_insertion_multi_hepi_trpl_cfg", args.rigid_minibatch),
+                    ("rigid_pushing_multi_empn_trpl_cfg", args.empn_minibatch)):
         cur = res[f"{name}@{B}"] = {}
         todo = dict(variants)
         if name.startswith("rope"):
