@@ -69,7 +69,8 @@ ENCODER_GRAD_FLOATS = 192 * 64 + 192 + 3 * (64 * 64 + 64) + 4 * 64
 class GrlCriticDesc(C.Structure):
     _fields_ = [("n_graphs", _i32), ("n_tokens", _i32), ("n_feat", _i32), ("n_partials", _i32), ("eps", C.c_float),
                 ("count", C.c_double), ("x", _fp), ("w1", _fp), ("b1", _fp), ("gamma", _fp), ("beta", _fp), ("stats", _fp),
-                ("stat_partials", _fp), ("ysum", _fp), ("grad_ysum", _fp), ("bstats", _fp), ("grad_partials", _fp)]
+                ("stat_partials", _fp), ("ysum", _fp), ("grad_ysum", _fp), ("bstats", _fp), ("grad_partials", _fp),
+                ("n_groups", _i32)]
 
 
 CRITIC_GRAD_FLOATS = 3 * 64 + 64 * 16

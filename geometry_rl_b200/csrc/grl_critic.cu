@@ -1,6 +1,7 @@
 // DeepSets critic, inner per-token MLP up to the pooled sum (deepsets.py:34-53 with PyG MLP / LayerNorm(mode='graph')):
 //   h    = x W1^T + b1                                  x: [B][N][F] tokens (F <= 16), W1: [64][F]
-//   y    = relu((h - mean) / (std + eps) * gamma + beta)  mean / biased std over the WHOLE [B][N][64] tensor (one group)
+//   y    = relu((h - mean) / (std + eps) * gamma + beta)  mean / biased std over the WHOLE [B][N][64] tensor, or per group
+//                                                        of Bg = B / n_groups consecutive graphs (forward only)
 //   ysum = sum_n y[b][n]                                  [B][64]
 // (the second Linear of the inner MLP commutes with the token sum: sum_n (y W2^T + b2) = ysum W2^T + N b2, a [B][64] GEMM the
 // host applies with torch.)
@@ -13,6 +14,11 @@
 // One CTA works on one graph at a time (persistent, contiguous graph ranges): 256 threads = 16 token lanes x 16 channel
 // groups of 4; token lane p owns tokens p, p + 16, ...  Cross-thread sums use fixed-order shared-memory trees; cross-CTA sums
 // are per-CTA partial slots reduced in slot order: deterministic, no atomics.  Statistics are accumulated in fp64.
+//
+// Groups (the time steps of the advantage phase, whose per-step statistics the reference computes in a Python loop): graphs
+// are group-major, group g = graphs [g Bg, (g + 1) Bg).  The n_partials CTAs split into S = n_partials / n_groups slots per
+// group, so a CTA never spans two groups and its partial slot c = g S + s belongs to group g alone.  With one group this is
+// the plain contiguous split of the graphs over the grid.
 #include "grl_common.cuh"
 
 namespace grl {
@@ -79,9 +85,12 @@ __device__ __forceinline__ void block_sum_d(double (&v)[NV], double* __restrict_
   }
 }
 
+// graphs [g_lo, g_hi) of this CTA: slot s of group g (n_groups == 1: the contiguous split over the whole grid)
 __device__ __forceinline__ void critic_range(const GrlCriticDesc& d, int& g_lo, int& g_hi) {
-  g_lo = (int)((long long)d.n_graphs * blockIdx.x / gridDim.x);
-  g_hi = (int)((long long)d.n_graphs * (blockIdx.x + 1) / gridDim.x);
+  const int S = d.n_partials / d.n_groups, g = blockIdx.x / S, s = blockIdx.x % S;
+  const long long bg = d.n_graphs / d.n_groups;
+  g_lo = (int)(g * bg + bg * s / S);
+  g_hi = (int)(g * bg + bg * (s + 1) / S);
 }
 
 // ---- forward pass 1: partial (sum h, sum h^2) per CTA --------------------------------------------------------------------
@@ -117,22 +126,28 @@ __global__ void __launch_bounds__(kCrThreads) critic_stats_kernel(const GrlCriti
   }
 }
 
-// out[i] = sum over slots of partials[slot][i] in slot order (n <= 4 doubles per slot)
-__global__ void critic_combine_kernel(const double* __restrict__ partials, int n_slots, int n, double* __restrict__ out) {
-  const int i = threadIdx.x;
-  if (i >= n) return;
+// out[g][i] = sum over the group's slots of partials[g][slot][i] in slot order (n doubles per slot)
+constexpr int kCrCombineThreads = 128;
+__global__ void critic_combine_kernel(const double* __restrict__ partials, int n_groups, int n_slots, int n,
+                                      double* __restrict__ out) {
+  const int j = blockIdx.x * kCrCombineThreads + threadIdx.x;
+  if (j >= n_groups * n) return;
+  const int g = j / n, i = j % n;
+  const double* p = partials + (size_t)g * n_slots * n + i;
   double s = 0.0;
-  for (int k = 0; k < n_slots; ++k) s += partials[(size_t)k * n + i];
-  out[i] = s;
+  for (int k = 0; k < n_slots; ++k) s += p[(size_t)k * n];
+  out[j] = s;
 }
 
 struct CriticNorm {
   float mean, inv, r;  // inv = 1 / (std + eps), r = std / (std + eps)
 };
+// statistics of this CTA's group (`count` = elements of one group over all ranks)
 __device__ __forceinline__ CriticNorm critic_norm(const GrlCriticDesc& d) {
+  const double* st = d.stats + 2 * (blockIdx.x / (d.n_partials / d.n_groups));
   const double n = d.count;
-  const double mean = d.stats[0] / n;
-  double var = d.stats[1] / n - mean * mean;
+  const double mean = st[0] / n;
+  double var = st[1] / n - mean * mean;
   var = var > 0.0 ? var : 0.0;
   const double sd = sqrt(var);
   CriticNorm c;
@@ -329,10 +344,28 @@ static int critic_check(const GrlCriticDesc* d, const char* who) {
   GRL_REQUIRE(d->x && d->w1 && d->b1 && d->gamma && d->beta && d->stats && d->stat_partials, GRL_EINVAL, "%s: null pointer", who);
   GRL_REQUIRE(d->n_partials > 0 && d->n_partials <= d->n_graphs, GRL_EINVAL, "%s: n_partials=%d must be in [1, n_graphs]", who,
               d->n_partials);
+  GRL_REQUIRE(d->n_groups > 0 && d->n_graphs % d->n_groups == 0 && d->n_partials % d->n_groups == 0, GRL_EINVAL,
+              "%s: n_groups=%d must be >= 1 and divide n_graphs=%d and n_partials=%d", who, d->n_groups, d->n_graphs,
+              d->n_partials);
+  return GRL_OK;
+}
+
+// the backward pass has no grouped statistics (the advantage phase that uses groups takes no gradients)
+static int critic_check_bwd(const GrlCriticDesc* d, const char* who) {
+  const int rc = critic_check(d, who);
+  if (rc != GRL_OK) return rc;
+  GRL_REQUIRE(d->n_groups == 1, GRL_EUNSUPPORTED, "%s: n_groups=%d (the backward pass takes one group)", who, d->n_groups);
+  GRL_REQUIRE(d->grad_ysum && d->bstats && d->grad_partials && d->count > 0, GRL_EINVAL, "%s: null pointer", who);
   return GRL_OK;
 }
 
 static int critic_grid(const GrlCriticDesc* d) { return d->n_partials; }
+
+static void critic_combine(const GrlCriticDesc* d, double* out, cudaStream_t stream) {
+  const int n = d->n_groups * 2;
+  grl::critic_combine_kernel<<<(n + grl::kCrCombineThreads - 1) / grl::kCrCombineThreads, grl::kCrCombineThreads, 0, stream>>>(
+      d->stat_partials, d->n_groups, d->n_partials / d->n_groups, 2, out);
+}
 
 int grl_critic_inner_stats(const GrlCriticDesc* d, grl_stream_t stream) {
   const int rc = critic_check(d, "grl_critic_inner_stats");
@@ -341,7 +374,7 @@ int grl_critic_inner_stats(const GrlCriticDesc* d, grl_stream_t stream) {
   if (grl::ensure_dynamic_smem((const void*)grl::critic_stats_kernel, smem) != GRL_OK) return GRL_ECUDA;
   const int grid = critic_grid(d);
   grl::critic_stats_kernel<<<grid, grl::kCrThreads, smem, (cudaStream_t)stream>>>(*d);
-  grl::critic_combine_kernel<<<1, 32, 0, (cudaStream_t)stream>>>(d->stat_partials, grid, 2, d->stats);
+  critic_combine(d, d->stats, (cudaStream_t)stream);
   return grl::check_launch("grl_critic_inner_stats");
 }
 
@@ -356,21 +389,19 @@ int grl_critic_inner_fwd(const GrlCriticDesc* d, grl_stream_t stream) {
 }
 
 int grl_critic_inner_bwd_stats(const GrlCriticDesc* d, grl_stream_t stream) {
-  const int rc = critic_check(d, "grl_critic_inner_bwd_stats");
+  const int rc = critic_check_bwd(d, "grl_critic_inner_bwd_stats");
   if (rc != GRL_OK) return rc;
-  GRL_REQUIRE(d->grad_ysum && d->bstats && d->grad_partials && d->count > 0, GRL_EINVAL, "grl_critic_inner_bwd_stats: null pointer");
   const int smem = (int)sizeof(grl::CriticSmem);
   if (grl::ensure_dynamic_smem((const void*)grl::critic_bwd_stats_kernel, smem) != GRL_OK) return GRL_ECUDA;
   const int grid = critic_grid(d);
   grl::critic_bwd_stats_kernel<<<grid, grl::kCrThreads, smem, (cudaStream_t)stream>>>(*d);
-  grl::critic_combine_kernel<<<1, 32, 0, (cudaStream_t)stream>>>(d->stat_partials, grid, 2, d->bstats);
+  critic_combine(d, d->bstats, (cudaStream_t)stream);
   return grl::check_launch("grl_critic_inner_bwd_stats");
 }
 
 int grl_critic_inner_bwd(const GrlCriticDesc* d, grl_stream_t stream) {
-  const int rc = critic_check(d, "grl_critic_inner_bwd");
+  const int rc = critic_check_bwd(d, "grl_critic_inner_bwd");
   if (rc != GRL_OK) return rc;
-  GRL_REQUIRE(d->grad_ysum && d->bstats && d->grad_partials && d->count > 0, GRL_EINVAL, "grl_critic_inner_bwd: null pointer");
   const int smem = (int)sizeof(grl::CriticSmem);
   if (grl::ensure_dynamic_smem((const void*)grl::critic_bwd_kernel, smem) != GRL_OK) return GRL_ECUDA;
   grl::critic_bwd_kernel<<<critic_grid(d), grl::kCrThreads, smem, (cudaStream_t)stream>>>(*d);

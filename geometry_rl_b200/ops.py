@@ -875,37 +875,52 @@ def aggregate_messages(x_src, basis, wk, es: EdgeSet) -> torch.Tensor:
 # ------------------------------------------------------------------------------------------------
 # V1: DeepSets critic, inner per-token MLP up to the pooled sum
 # ------------------------------------------------------------------------------------------------
+def critic_partials(n_graphs: int, groups: int = 1) -> int:
+    """CTAs (= partial slots) of the critic kernels.  One group: the update step's split, two CTAs per SM.  Several: S
+    slots per group, S = max(1, min(graphs per group, ceil(2 SMs / groups))), so a CTA never spans two groups."""
+    if groups == 1:
+        return _n_partials(n_graphs, 2)
+    return groups * max(1, min(n_graphs // groups, -(-2 * L.sm_count() // groups)))
+
+
 class CriticInnerFn(torch.autograd.Function):
     """x [B,N,F] -> ysum [B,64] = sum_n relu(graph_layer_norm(x W1^T + b1) * gamma + beta)  (deepsets.py:34-53 up to the
     token sum; PyG LayerNorm(mode='graph') statistics over the whole tensor).  Four launches forward + backward, no
-    [B N, 64] activation in HBM.  `all_reduce(double[2])` (data parallel) makes the statistics global."""
+    [B N, 64] activation in HBM.  `all_reduce(double tensor)` (data parallel) makes the statistics global.
+
+    `groups` > 1 (forward only): the graphs are `groups` consecutive blocks of B / groups (the time-major layout of the
+    advantage phase), each normalised with its own statistics, as GraphLayerNorm(groups) does."""
 
     @staticmethod
-    def forward(ctx, x, w1, b1, gamma, beta, eps, all_reduce=None, world_size=1):
+    def forward(ctx, x, w1, b1, gamma, beta, eps, all_reduce=None, world_size=1, groups=1):
         x, w1c, b1c = _f32c(x), _f32c(w1.detach()), _f32c(b1.detach())
         gc, bc = _f32c(gamma.detach()), _f32c(beta.detach())
         B, N, Fdim = x.shape
         assert tuple(w1c.shape) == (64, Fdim) and Fdim <= 16, f"critic inner layer {tuple(w1c.shape)} on {Fdim} features"
+        assert groups >= 1 and B % groups == 0, f"{B} graphs in {groups} groups"
         dev = x.device
-        n_p = _n_partials(B, 2)
-        stats = torch.empty(2, dtype=torch.float64, device=dev)
+        Bg = B // groups
+        n_p = critic_partials(B, groups)
+        stats = torch.empty(groups, 2, dtype=torch.float64, device=dev)
         sp = torch.empty(n_p, 2, dtype=torch.float64, device=dev)
         ysum = torch.empty(B, 64, dtype=torch.float32, device=dev)
         d = L.GrlCriticDesc(n_graphs=B, n_tokens=N, n_feat=Fdim, n_partials=n_p, eps=float(eps),
-                            count=float(B) * N * 64 * world_size, x=L.ptr(x), w1=L.ptr(w1c), b1=L.ptr(b1c), gamma=L.ptr(gc),
-                            beta=L.ptr(bc), stats=L.ptr_any(stats), stat_partials=L.ptr_any(sp), ysum=L.ptr(ysum))
+                            count=float(Bg) * N * 64 * world_size, x=L.ptr(x), w1=L.ptr(w1c), b1=L.ptr(b1c), gamma=L.ptr(gc),
+                            beta=L.ptr(bc), stats=L.ptr_any(stats), stat_partials=L.ptr_any(sp), ysum=L.ptr(ysum),
+                            n_groups=groups)
         L.call("grl_critic_inner_stats", C.byref(d), shape=(B * N, B, 0))
         if all_reduce is not None:
             all_reduce(stats)
         L.call("grl_critic_inner_fwd", C.byref(d), shape=(B * N, B, 0))
         ctx.save_for_backward(x, w1c, b1c, gc, bc, stats)
-        ctx.meta = (float(eps), all_reduce, world_size, n_p)
+        ctx.meta = (float(eps), all_reduce, world_size, n_p, groups)
         return ysum
 
     @staticmethod
     def backward(ctx, g_ysum):
         x, w1c, b1c, gc, bc, stats = ctx.saved_tensors
-        eps, all_reduce, world_size, n_p = ctx.meta
+        eps, all_reduce, world_size, n_p, groups = ctx.meta
+        assert groups == 1, "the fused critic kernels have no grouped backward pass"
         B, N, Fdim = x.shape
         dev = x.device
         g_ysum = _f32c(g_ysum)
@@ -915,18 +930,18 @@ class CriticInnerFn(torch.autograd.Function):
         d = L.GrlCriticDesc(n_graphs=B, n_tokens=N, n_feat=Fdim, n_partials=n_p, eps=eps, count=float(B) * N * 64 * world_size,
                             x=L.ptr(x), w1=L.ptr(w1c), b1=L.ptr(b1c), gamma=L.ptr(gc), beta=L.ptr(bc), stats=L.ptr_any(stats),
                             stat_partials=L.ptr_any(sp), grad_ysum=L.ptr(g_ysum), bstats=L.ptr_any(bstats),
-                            grad_partials=L.ptr(part))
+                            grad_partials=L.ptr(part), n_groups=1)
         L.call("grl_critic_inner_bwd_stats", C.byref(d), shape=(B * N, B, 0))
         if all_reduce is not None:
             all_reduce(bstats)
         L.call("grl_critic_inner_bwd", C.byref(d), shape=(B * N, B, 0))
         g = _reduce(part)
         g_w1 = g[192:].view(64, 16)[:, :Fdim].contiguous()
-        return None, g_w1, g[128:192], g[0:64], g[64:128], None, None, None
+        return None, g_w1, g[128:192], g[0:64], g[64:128], None, None, None, None
 
 
-def critic_inner(x, w1, b1, gamma, beta, eps, all_reduce=None, world_size=1):
-    return CriticInnerFn.apply(x, w1, b1, gamma, beta, eps, all_reduce, world_size)
+def critic_inner(x, w1, b1, gamma, beta, eps, all_reduce=None, world_size=1, groups=1):
+    return CriticInnerFn.apply(x, w1, b1, gamma, beta, eps, all_reduce, world_size, groups)
 
 
 # ------------------------------------------------------------------------------------------------

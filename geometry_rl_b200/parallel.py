@@ -42,6 +42,51 @@ class _GraphNormStats(torch.autograd.Function):
 
 SIDE_STREAM_RESERVED_SMS = 4
 
+_split_capture = None  # set while a SegmentedGraph records: DataParallel.all_reduce then ends the current segment
+
+
+class SegmentedGraph:
+    """A CUDA graph split at every `DataParallel.all_reduce` the captured function issues.  Each collective runs between
+    the replays of two segments, on the static tensor the first one wrote, so the replay works with any backend (gloo
+    cannot be captured, and ranks that share one GPU cannot use NCCL).  The segments share one memory pool and always
+    replay in capture order.  A function without collectives gives one segment: a plain CUDA graph."""
+
+    def capture(self, fn):
+        global _split_capture
+        pool = torch.cuda.graph_pool_handle()
+        parts, cur = [], [None]
+
+        def begin():
+            g = torch.cuda.CUDAGraph()
+            g.capture_begin(pool=pool)
+            cur[0] = g
+
+        def split(dp, t, op):
+            cur[0].capture_end()
+            parts.append((cur[0], dp, t, op))
+            begin()
+
+        torch.cuda.synchronize()
+        stream = torch.cuda.Stream()
+        stream.wait_stream(torch.cuda.current_stream())
+        with torch.cuda.stream(stream):
+            begin()
+            _split_capture = split
+            try:
+                out = fn()
+            finally:
+                _split_capture = None
+                cur[0].capture_end()
+        torch.cuda.current_stream().wait_stream(stream)
+        self.parts, self.last = parts, cur[0]
+        return out
+
+    def replay(self):
+        for g, dp, t, op in self.parts:
+            g.replay()
+            dp.all_reduce(t, op)
+        self.last.replay()
+
 
 class DataParallel:
     def __init__(self, group=None, side_group: bool = False):
@@ -66,6 +111,9 @@ class DataParallel:
             _lib.reserve_sms(SIDE_STREAM_RESERVED_SMS)
 
     def all_reduce(self, t: torch.Tensor, op=dist.ReduceOp.SUM) -> torch.Tensor:
+        if _split_capture is not None:  # recorded by a SegmentedGraph: the collective runs between its segments
+            _split_capture(self, t, op)
+            return t
         dist.all_reduce(t, op=op, group=self.group)
         self.collectives += 1
         return t

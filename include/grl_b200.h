@@ -339,22 +339,29 @@ int grl_reduce_partials(const float* partials, int n_partials, int64_t n_floats,
  *   forward : grl_critic_inner_stats (-> stats = (sum h, sum h^2)), [all-reduce], grl_critic_inner_fwd (-> ysum)
  *   backward: grl_critic_inner_bwd_stats (-> bstats = (sum g_xhat, sum g_xhat xhat), g_gamma, g_beta partials),
  *             [all-reduce], grl_critic_inner_bwd (-> g_b1, g_W1 partials)
+ * n_groups > 1 (forward only: the advantage phase's time steps, each with its own statistics): the graphs are group-major,
+ * group g = graphs [g Bg, (g + 1) Bg) with Bg = n_graphs / n_groups; `stats` is [n_groups][2], `count` the element count of
+ * ONE group over all ranks, and each of the S = n_partials / n_groups CTAs of a group covers graphs of that group only.
+ * n_groups must divide n_graphs and n_partials; 0 is rejected (GRL_EINVAL), and the backward entry points return
+ * GRL_EUNSUPPORTED for n_groups != 1.
  * ------------------------------------------------------------------------------------------ */
 typedef struct {
   int32_t n_graphs, n_tokens, n_feat, n_partials; /* n_feat <= 16; n_partials <= n_graphs CTAs, one partial slot each    */
   float eps;
-  double count;            /* number of elements of the [B][N][64] tensor over ALL ranks                              */
+  double count;            /* number of elements of one group's [Bg][N][64] tensor over ALL ranks                     */
   const float* x;          /* [B][N][F]                                                                                */
   const float* w1;         /* [64][F] row-major (mlp_inner.lins.0.weight)                                              */
   const float* b1;         /* [64]                                                                                     */
   const float* gamma;      /* [64] mlp_inner.norms.0.weight                                                            */
   const float* beta;       /* [64] mlp_inner.norms.0.bias                                                              */
-  double* stats;           /* [2] (sum h, sum h^2): written by _stats for this rank's rows, read by the other passes   */
-  double* stat_partials;   /* [n_partials][2] workspace                                                                */
+  double* stats;           /* [n_groups][2] (sum h, sum h^2): written by _stats for this rank's rows, read by the other
+                              passes                                                                                   */
+  double* stat_partials;   /* [n_groups][S][2] = [n_partials][2] workspace                                             */
   float* ysum;             /* [B][64]                                                                                  */
   const float* grad_ysum;  /* [B][64]                                                                                  */
   double* bstats;          /* [2] (S1, S2): written by _bwd_stats, read by _bwd                                        */
   float* grad_partials;    /* [n_partials][GRL_CRITIC_GRAD_FLOATS]                                                     */
+  int32_t n_groups;        /* >= 1 independent statistics groups of consecutive graphs (1: the whole tensor)           */
 } GrlCriticDesc;
 /* partial layout: g_gamma[64] | g_beta[64] | g_b1[64] | g_W1[64][16] (columns >= F are zero) */
 #define GRL_CRITIC_GRAD_FLOATS (3 * 64 + 64 * 16)
