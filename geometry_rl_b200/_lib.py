@@ -115,6 +115,22 @@ class GrlActDesc(C.Structure):
 
 
 ACT_MAX_K = 32  # GRL_ACT_MAX_K
+
+
+class GrlVecNormKey(C.Structure):
+    _fields_ = [("batch", C.c_int64), ("feat", _i32), ("comps", _i32), ("x", _fp), ("out", _fp), ("sum", _fp),
+                ("ssq", _fp), ("count", _fp)]
+
+
+VECNORM_MAX_KEYS = 8  # GRL_VECNORM_MAX_KEYS
+VECNORM_MAX_COMPS = 64  # GRL_VECNORM_MAX_COMPS
+VECNORM_ROWS_PER_SLOT = 512  # GRL_VECNORM_ROWS_PER_SLOT
+VECNORM_MAX_SLOTS = 1024  # GRL_VECNORM_MAX_SLOTS
+
+
+class GrlVecNormDesc(C.Structure):
+    _fields_ = [("n_keys", _i32), ("world", _i32), ("decay", C.c_float), ("eps", C.c_float),
+                ("key", GrlVecNormKey * VECNORM_MAX_KEYS), ("partials", _fp), ("inc", _fp)]
 READOUT_MAX_OUT = 8
 MAX_KNN = 8  # GRL_MAX_KNN: k of grl_knn_graph, max_neighbors of the radius graph
 LOSS_TERMS = 8
@@ -177,6 +193,9 @@ SIGNATURES = {
     "grl_gae_scan": (C.c_int, [_fp, _fp, _fp, _fp, C.c_float, C.c_float, C.c_int, C.c_int, _fp, _fp, _fp]),
     "grl_gaussian_act": (C.c_int, [C.POINTER(GrlActDesc), _fp]),
     "grl_act_advance": (C.c_int, [_fp, _fp]),
+    "grl_vecnorm_stats": (C.c_int, [C.POINTER(GrlVecNormDesc), _fp]),
+    "grl_vecnorm_update": (C.c_int, [C.POINTER(GrlVecNormDesc), _fp]),
+    "grl_vecnorm_apply": (C.c_int, [C.POINTER(GrlVecNormDesc), _fp]),
     "grl_trpl_fwd": (C.c_int, [C.POINTER(GrlProjDesc), _fp]),
     "grl_trpl_bwd": (C.c_int, [C.POINTER(GrlProjDesc), _fp]),
     "grl_tc_selftest_gemm": (C.c_int, [_fp, _fp, _fp, C.c_int, C.c_int, _fp]),

@@ -10,6 +10,7 @@ import torch
 from torch import nn
 
 from .... import ops
+from ....parallel import SegmentedGraph
 
 LOG_2PI = math.log(2.0 * math.pi)
 
@@ -142,13 +143,19 @@ class PolicyOperator(nn.Module):
         body, with noise from the device stream (`deterministic`: action = loc, nothing drawn)."""
         return self._write_act(td, self._act([td_get(td, k) for k in self.in_keys], deterministic), copy=False)
 
-    def capture_act(self, example_td, *, seed: int, deterministic: bool = False, warmup: int = 2):
+    def capture_act(self, example_td, *, seed: int, deterministic: bool = False, warmup: int = 2, obs_norm=None):
         """Record `build_data -> body -> grl_gaussian_act -> advance` into one CUDA graph on static copies of the
         example's observation keys (the batch size of every later `act_graphed` call), and start the noise stream at
         (seed, 0).  A pending one-time FiberBundleConv calibration runs eagerly on the example first.  The graph holds the
         topology of this batch size: re-capture after `hyper_data.invalidate()`.  With `hyper_data.rebuild_every_call`
         the data builder must refresh its topology in place (`refresh_in_place()`): every replay then rebuilds the kNN or
-        radius graph from the static positions; any other rebuild mode is refused."""
+        radius graph from the static positions; any other rebuild mode is refused.
+
+        `obs_norm` (an `NDVecNorm`): the graph starts from the RAW observation groups the normaliser reads and runs its
+        device kernels (`NDVecNorm.apply_device`) into the static `norm_*` tensors the body reads; `act_graphed` then also
+        writes copies of the `norm_*` keys.  Capture leaves the statistics as they were.  A normaliser frozen at capture
+        gives a graph with no update (and no collective); replaying after its `frozen` flag changed raises.  Under data
+        parallelism (`obs_norm.dp`) the graph is split at the statistics all-reduce (`parallel.SegmentedGraph`)."""
         hd = self.policy.hyper_data
         if hd.rebuild_every_call and not hd.refresh_in_place():
             raise ValueError(
@@ -158,6 +165,9 @@ class PolicyOperator(nn.Module):
                 "replayed; a captured act rebuilds kNN INTERNAL edges with `hyper_data.knn_in_place = True` (HEPi rope: "
                 "any precision; HEPi rigid and EMPN: fused 16-bit path) and, for HEPi, radius INTERNAL edges on the "
                 "fused 16-bit path (internal_edges='radius', ops.set_precision('bf16')) - otherwise use `act`")
+        if obs_norm is not None:
+            return self._capture_act_norm(example_td, seed, deterministic, warmup, obs_norm)
+        self._act_norm = None
         self._act_static = [td_get(example_td, k).clone() for k in self.in_keys]
         with torch.no_grad():
             self.get_dist(dict(zip(self.in_keys, self._act_static)))  # the one-time calibration, if still pending
@@ -175,9 +185,57 @@ class PolicyOperator(nn.Module):
         self._captured_topology = hd.example_data
         return self
 
+    def _capture_act_norm(self, example_td, seed, deterministic, warmup, obs_norm):
+        raw = {k: td_get(example_td, k).clone() for k in obs_norm.in_keys if td_get(example_td, k) is not None}
+        if not raw:
+            raise ValueError(f"capture_act: the example holds none of the normaliser's keys {obs_norm.in_keys}")
+        normed = {ok: torch.empty_like(raw[k]) for k, ok in zip(obs_norm.in_keys, obs_norm.out_keys) if k in raw}
+        static = {**raw, **normed}
+        self._act_static = [static[k] if k in static else td_get(example_td, k).clone() for k in self.in_keys]
+        # what act_graphed copies in: the raw groups and every policy input the normaliser does not write
+        self._act_copy_in = list(raw.items()) + [(k, s) for k, s in zip(self.in_keys, self._act_static)
+                                                 if k not in static]
+        self._act_norm, self._act_norm_out, self._act_norm_frozen = obs_norm, normed, obs_norm.frozen
+
+        def normalise():
+            obs_norm.apply_device(dict(raw), out=normed)
+
+        obs_norm.ensure_stats(raw)  # no allocation or memset of the state inside the graph
+        saved = obs_norm.state_dict()
+        with torch.no_grad():
+            normalise()
+            self.get_dist(dict(zip(self.in_keys, self._act_static)))  # the one-time calibration, if still pending
+        self.set_act_state(seed, 0)
+        side = torch.cuda.Stream()
+        side.wait_stream(torch.cuda.current_stream())
+        with torch.cuda.stream(side), torch.no_grad():
+            for _ in range(warmup):  # draws without advancing; the statistics are restored below
+                normalise()
+                self.policy.act(*self._act_static, state=self._act_state, deterministic=deterministic, rank=self.act_rank)
+        torch.cuda.current_stream().wait_stream(side)
+        obs_norm.load_state_dict(saved)  # in place: the graph reads these tensors
+
+        def step():
+            normalise()
+            return self._act(self._act_static, deterministic)
+
+        self._act_graph = SegmentedGraph()
+        with torch.no_grad():
+            self._act_graph_out = self._act_graph.capture(step)
+        self._captured_topology = self.policy.hyper_data.example_data
+        return self
+
+    def _check_act_norm(self):
+        norm = getattr(self, "_act_norm", None)
+        if norm is not None and norm.frozen != self._act_norm_frozen:
+            raise RuntimeError(
+                f"act_graphed: the observation normaliser was {'frozen' if self._act_norm_frozen else 'updating'} at "
+                "capture and has changed since; re-capture with capture_act(obs_norm=...)")
+
     def act_static(self, td=None):
         """Replay the captured act on whatever the static inputs hold; with `td`, write the graph's own output tensors
         into it (no copy: the next replay overwrites them).  Returns the outputs keyed like `forward`'s."""
+        self._check_act_norm()
         self._act_graph.replay()
         out = dict(zip(self.out_keys, self._act_graph_out[:4]))
         if td is not None:
@@ -185,10 +243,19 @@ class PolicyOperator(nn.Module):
         return out
 
     def act_graphed(self, td):
-        """Copy td's observation keys into the static inputs, replay the captured act and write copies of its outputs."""
-        for s, k in zip(self._act_static, self.in_keys):
+        """Copy td's observation keys into the static inputs, replay the captured act and write copies of its outputs
+        (and, with a captured `obs_norm`, copies of the `norm_*` keys it computed from td's raw groups)."""
+        if self._act_norm is None:
+            for s, k in zip(self._act_static, self.in_keys):
+                s.copy_(td_get(td, k), non_blocking=True)
+            self._act_graph.replay()
+            return self._write_act(td, self._act_graph_out, copy=True)
+        self._check_act_norm()
+        for k, s in self._act_copy_in:
             s.copy_(td_get(td, k), non_blocking=True)
         self._act_graph.replay()
+        for ok, t in self._act_norm_out.items():
+            td[ok] = t.clone()
         return self._write_act(td, self._act_graph_out, copy=True)
 
 

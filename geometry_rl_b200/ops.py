@@ -1078,6 +1078,53 @@ def act_advance(state) -> None:
 
 
 # ------------------------------------------------------------------------------------------------
+# N4: observation normalisation (NDVecNorm) on the device
+# ------------------------------------------------------------------------------------------------
+def vecnorm_slots(rows: int) -> int:
+    """Partial slots of one key in grl_vecnorm_stats (a function of its row count M only)."""
+    return max(1, min(-(-int(rows) // L.VECNORM_ROWS_PER_SLOT), L.VECNORM_MAX_SLOTS))
+
+
+def vecnorm(xs, *, out, sums, ssqs, counts, decay: float, eps: float, update: bool = True, all_reduce=None,
+            world_size: int = 1):
+    """Standardise every group of `xs` (fp32, any shape whose numel is a multiple of its statistics' numel C) per
+    component into `out` with NDVecNorm's running statistics `sums[i]` / `ssqs[i]` [C], `counts[i]` [1] (fp32, updated in
+    place).  `update=False` is the frozen normaliser: one launch, no statistics.  Otherwise the fp64 increments of every
+    key go through ONE `all_reduce(inc)` (data parallelism: equal shards, count increment M_local * world_size) between
+    grl_vecnorm_stats and grl_vecnorm_update.  No host read: capturable in a CUDA graph."""
+    groups = [xs, out, sums, ssqs, counts]
+    if any(not t.is_cuda for g in groups for t in g):
+        raise RuntimeError("vecnorm: geometry_rl_b200 kernels need CUDA tensors (no CPU path exists)")
+    n = len(xs)
+    if not 1 <= n <= L.VECNORM_MAX_KEYS or any(len(g) != n for g in groups):
+        raise ValueError(f"vecnorm: 1..{L.VECNORM_MAX_KEYS} keys, with one out / sum / ssq / count each")
+    d = L.GrlVecNormDesc(n_keys=n, world=int(world_size), decay=float(decay), eps=float(eps))
+    rows, comps = [], []
+    for i, (x, o, s, q, c) in enumerate(zip(*groups)):
+        if any(t.dtype != torch.float32 for t in (x, o, s, q, c)) or o.shape != x.shape or c.numel() != 1 \
+                or q.shape != s.shape:
+            raise ValueError("vecnorm: fp32 tensors, out shaped like x, ssq like sum, one count")
+        C_ = s.numel()
+        B = x.shape[0] if x.dim() > 0 else 1
+        F = x.numel() // B if B else 0
+        d.key[i] = L.GrlVecNormKey(batch=B, feat=F, comps=C_, x=L.ptr(x), out=L.ptr(o), sum=L.ptr(s), ssq=L.ptr(q),
+                                   count=L.ptr(c))
+        rows.append(B * F // C_ if C_ and F % C_ == 0 else 0)
+        comps.append(C_)
+    if update:
+        partials = torch.empty(sum(vecnorm_slots(m) * c for m, c in zip(rows, comps)) * 2, dtype=torch.float64,
+                               device=xs[0].device)
+        inc = torch.empty(sum(comps) * 2, dtype=torch.float64, device=xs[0].device)
+        d.partials, d.inc = L.ptr(partials), L.ptr(inc)
+        L.call("grl_vecnorm_stats", C.byref(d), shape=(sum(rows), n, 0))
+        if all_reduce is not None:
+            all_reduce(inc)
+        L.call("grl_vecnorm_update", C.byref(d), shape=(sum(rows), n, 0))
+    L.call("grl_vecnorm_apply", C.byref(d), shape=(sum(rows), n, 0))
+    return out
+
+
+# ------------------------------------------------------------------------------------------------
 # K4: trust-region projection
 # ------------------------------------------------------------------------------------------------
 class TrplProjectFn(torch.autograd.Function):

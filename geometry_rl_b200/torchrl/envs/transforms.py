@@ -52,8 +52,10 @@ class NDVecNorm:
     every leading dimension (environments, points) is summed over and counted (`_count_left`, transforms.py:62-68)."""
 
     def __init__(self, in_keys: Sequence[str], out_keys: Optional[Sequence[str]] = None, shapes: Optional[Sequence] = None,
-                 decay: float = 0.9999, eps: float = 1e-4, **ignored):
+                 decay: float = 0.9999, eps: float = 1e-4, *, dp=None, **ignored):
+        """`dp`: a `parallel.DataParallel` handle; `apply_device` then takes its statistics over every rank's rows."""
         self.in_keys = list(in_keys)
+        self.dp = dp
         self.out_keys = list(out_keys) if out_keys is not None else list(self.in_keys)
         if shapes is not None and len(shapes) != len(self.in_keys):
             raise ValueError("shapes must have one entry per in_key")
@@ -101,11 +103,60 @@ class NDVecNorm:
         return {f"{k}_{n}": t.clone() for k, st in self._stats.items() for n, t in st.items()}
 
     def load_state_dict(self, sd: Mapping[str, torch.Tensor]):
+        """Copies into the existing state tensors when they have the checkpoint's shapes (a CUDA graph captured with
+        `PolicyOperator.capture_act(obs_norm=...)` keeps reading them), else installs clones."""
         for k in self.in_keys:
             if f"{k}_sum" in sd:
-                self._stats[k] = {n: sd[f"{k}_{n}"].clone() for n in ("sum", "ssq", "count")}
+                new = {n: sd[f"{k}_{n}"] for n in ("sum", "ssq", "count")}
+                st = self._stats.get(k)
+                if st is not None and all(st[n].shape == new[n].shape and st[n].dtype == new[n].dtype for n in new):
+                    for n, t in new.items():
+                        st[n].copy_(t)
+                else:
+                    self._stats[k] = {n: t.clone() for n, t in new.items()}
 
     def freeze(self):
         """Evaluation mode (`VecNorm.freeze()`): standardise with the current statistics without updating them."""
         self.frozen = True
         return self
+
+    # ---- the device path (csrc/grl_obsnorm.cu) ---------------------------------------------------------------------
+    def ensure_stats(self, td: Mapping[str, torch.Tensor]):
+        """Create (zeros) or move the statistics of every present in_key to its tensor's device, as fp32 contiguous
+        tensors.  `apply_device` does this itself; a CUDA graph capture calls it first so that no allocation or memset of
+        the state is recorded."""
+        for i, k in enumerate(self.in_keys):
+            if k not in td:
+                continue
+            v = td[k]
+            shape = self.shapes[i] if self.shapes is not None else tuple(v.shape[1:])
+            st = self._stats.get(k)
+            if st is None:
+                z = lambda: torch.zeros(shape, dtype=torch.float32, device=v.device)
+                self._stats[k] = {"sum": z(), "ssq": z(), "count": torch.zeros(1, dtype=torch.float32, device=v.device)}
+            elif any(t.device != v.device or t.dtype != torch.float32 or not t.is_contiguous() for t in st.values()):
+                self._stats[k] = {n: t.to(device=v.device, dtype=torch.float32).contiguous() for n, t in st.items()}
+        return self
+
+    @torch.no_grad()
+    def apply_device(self, td: MutableMapping[str, torch.Tensor], out: Optional[Mapping[str, torch.Tensor]] = None):
+        """What `__call__` computes, on the device kernels (`ops.vecnorm`), for every present in_key at once, on the same
+        state tensors.  The input keeps its layout: a flat [B, F] group is read as B F / C rows of the C statistics
+        components (ReshapeTransform is a view), and td[out_key] has x's shape.  `out` (out_key -> tensor) names the
+        output tensors; otherwise new ones are allocated.  With `dp` the increments are summed over all ranks (equal
+        shards) before the update, so every rank holds bit-identical statistics."""
+        from ...ops import vecnorm
+        keys = [(k, ok) for k, ok in zip(self.in_keys, self.out_keys) if k in td]
+        if not keys:
+            return td
+        self.ensure_stats(td)
+        xs = [td[k] for k, _ in keys]
+        outs = [out[ok] if out is not None else torch.empty_like(x) for (_, ok), x in zip(keys, xs)]
+        st = [self._stats[k] for k, _ in keys]
+        vecnorm(xs, out=outs, sums=[s["sum"] for s in st], ssqs=[s["ssq"] for s in st], counts=[s["count"] for s in st],
+                decay=self.decay, eps=self.eps, update=not self.frozen,
+                all_reduce=self.dp.all_reduce if self.dp is not None else None,
+                world_size=self.dp.world_size if self.dp is not None else 1)
+        for (_, ok), o in zip(keys, outs):
+            td[ok] = o
+        return td

@@ -476,6 +476,48 @@ int grl_gaussian_act(const GrlActDesc* d, grl_stream_t stream);
 int grl_act_advance(int64_t* state, grl_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------
+ * N4  Observation normalisation of the collector: replaces the eager NDVecNorm call (torchrl/envs/transforms.py:135-171
+ * on torchrl 0.3.1 VecNorm._update) that writes the norm_* keys every policy and the critic read.  Every key of one
+ * call is handled by the same launches.  Key i is a flat [B][F] fp32 group read as M = B F / C rows of C components
+ * (ReshapeTransform is a view); its running state is the fp32 sum[C], ssq[C], count[1] of NDVecNorm._stats.
+ *   grl_vecnorm_stats   per-component sums of x and x^2 in fp64: S(M) CTAs per key write partial slots, a second launch
+ *                       sums them in slot order into inc[key] (no atomics, no host read).  S(M) depends on M only:
+ *                       S = max(1, min(ceil(M / GRL_VECNORM_ROWS_PER_SLOT), GRL_VECNORM_MAX_SLOTS)), slot s covers rows
+ *                       [s P, min(M, (s + 1) P)) with P = ceil(M / S).
+ *   [all-reduce of inc]  under data parallelism (sum over ranks; then count_inc = max(1, M) * world).
+ *   grl_vecnorm_update  one CTA per key, torch's fp32 arithmetic with two roundings (no FMA):
+ *                       sum <- fl(fl(decay sum) + fl32(inc_sum)), ssq likewise, count <- fl(fl(decay count) + count_inc)
+ *   grl_vecnorm_apply   mean = sum / count, std = sqrt(max(ssq / count - mean^2, eps)), out = (x - mean) / max(std, eps)
+ *                       in the op order of transforms.py:86-88 (with the same state: torch's result bit for bit; a NaN
+ *                       passes the clamps as in torch.clamp_min).  The frozen normaliser calls this alone.
+ * ------------------------------------------------------------------------------------------ */
+#define GRL_VECNORM_MAX_KEYS 8
+#define GRL_VECNORM_MAX_COMPS 64
+#define GRL_VECNORM_ROWS_PER_SLOT 512
+#define GRL_VECNORM_MAX_SLOTS 1024
+typedef struct {
+  int64_t batch;           /* B >= 0                                                                              */
+  int32_t feat;            /* F >= 0, a multiple of comps                                                          */
+  int32_t comps;           /* C in [1, GRL_VECNORM_MAX_COMPS]: the statistics' numel                               */
+  const float* x;          /* [B][F]                                                                              */
+  float* out;              /* [B][F] (apply)                                                                      */
+  float* sum;              /* [C] running state                                                                   */
+  float* ssq;              /* [C]                                                                                 */
+  float* count;            /* [1]                                                                                 */
+} GrlVecNormKey;
+typedef struct {
+  int32_t n_keys;          /* 1 .. GRL_VECNORM_MAX_KEYS                                                           */
+  int32_t world;           /* ranks whose rows inc sums (count_inc = max(1, M) * world); 1 without data parallelism */
+  float decay, eps;
+  GrlVecNormKey key[GRL_VECNORM_MAX_KEYS];
+  double* partials;        /* [sum_i S(M_i) C_i][2] workspace (stats)                                               */
+  double* inc;             /* [sum_i C_i][2] (sum x, sum x^2) per key and component: written by stats, read by update */
+} GrlVecNormDesc;
+int grl_vecnorm_stats(const GrlVecNormDesc* d, grl_stream_t stream);
+int grl_vecnorm_update(const GrlVecNormDesc* d, grl_stream_t stream);
+int grl_vecnorm_apply(const GrlVecNormDesc* d, grl_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------
  * K4  TRPL projection of a diagonal Gaussian (mean + "std := cov" diagonal v):
  * replaces projections/kl_projection_layer.py:15-111,162-204 (ITPAL cpp_projection on the CPU),
  * projections/w2_projection_layer.py:15-68, base_projection_layer.py:71-100.
