@@ -80,7 +80,18 @@ class GrlProjDesc(C.Structure):
     _fields_ = [("batch", _i32), ("k", _i32), ("proj_type", _i32), ("eps_mean", C.c_float), ("eps_cov", C.c_float),
                 ("mean", _fp), ("v", _fp), ("old_mean", _fp), ("old_v", _fp), ("proj_mean", _fp), ("proj_v", _fp),
                 ("eta", _fp), ("grad_proj_mean", _fp), ("grad_proj_v", _fp), ("grad_mean", _fp), ("grad_v", _fp),
-                ("grad_mean_add", _fp), ("grad_v_add", _fp)]
+                ("grad_mean_add", _fp), ("grad_v_add", _fp), ("entropy_mode", _i32), ("entropy_first", _i32),
+                ("entropy_beta", _fp), ("entropy_alpha", _fp)]
+
+
+ENTROPY_MODE = {"ineq": 1, "eq": 2}  # GRL_ENTROPY_INEQ / _EQ (0 = off)
+ENTROPY_SCHEDULE = {"linear": 1, "exp": 2}  # GRL_ENTROPY_LINEAR / _EXP
+
+
+class GrlEntropyBoundDesc(C.Structure):
+    _fields_ = [("batch", _i32), ("k", _i32), ("schedule", _i32), ("stage", _i32), ("total_train_steps", C.c_int64),
+                ("target_entropy", C.c_double), ("temperature", C.c_double), ("old_v", _fp), ("step", _fp), ("sums", _fp),
+                ("state", _fp)]
 
 
 class GrlLossDesc(C.Structure):
@@ -198,6 +209,7 @@ SIGNATURES = {
     "grl_vecnorm_apply": (C.c_int, [C.POINTER(GrlVecNormDesc), _fp]),
     "grl_trpl_fwd": (C.c_int, [C.POINTER(GrlProjDesc), _fp]),
     "grl_trpl_bwd": (C.c_int, [C.POINTER(GrlProjDesc), _fp]),
+    "grl_trpl_entropy_bound": (C.c_int, [C.POINTER(GrlEntropyBoundDesc), _fp]),
     "grl_tc_selftest_gemm": (C.c_int, [_fp, _fp, _fp, C.c_int, C.c_int, _fp]),
     "grl_tc_selftest_gemm_ts": (C.c_int, [_fp, _fp, _fp, C.c_int, _fp]),
     "grl_tc_debug_mma": (C.c_int, [_fp, C.c_int, _fp, C.c_int, _fp, C.c_int, C.c_int] + [C.c_uint32] * 8 + [_fp]),

@@ -42,6 +42,11 @@ class TRPLLoss(nn.Module):
         self.register_buffer("clip_epsilon", torch.tensor(clip_epsilon))
         self.projection = projection
         self._global_steps = 0
+        # entropy control on the fused path reads the step from this int64 device tensor.  A Learner owns and advances it
+        # on the device (`steps_on_device`), so captured updates see the right step; otherwise every call writes
+        # `_global_steps` into it.
+        self.step_counter = None
+        self.steps_on_device = False
         # data-parallel hooks (None = single process): see geometry_rl_b200/parallel.py
         self.dp = None
         # projection + every actor-side loss term and metric in a handful of kernel launches (ops.trpl_loss) instead
@@ -93,7 +98,7 @@ class TRPLLoss(nn.Module):
     def _can_fuse(self, policy) -> bool:
         pr = self.projection
         return (self.fused and getattr(pr, "KERNEL_TYPE", None) in ("kl", "w2")
-                and not pr.has_entropy_control and (pr.KERNEL_TYPE != "w2" or pr.scale_prec)
+                and (pr.KERNEL_TYPE != "w2" or pr.scale_prec)
                 and getattr(policy, "contextual_std", True) and td_is_cuda(policy))
 
     def _forward_fused(self, td, with_critic: bool) -> dict:
@@ -102,7 +107,14 @@ class TRPLLoss(nn.Module):
         previous_dist = self.actor_network.build_dist_from_params(td)
         current_dist = self.actor_network.get_dist(td)
         pr = self.projection
-        if pr.initial_entropy is None:  # base_projection_layer.py:202-203
+        entropy = None
+        if pr.has_entropy_control:  # the initial entropy is latched on the device, with the bound
+            if self.step_counter is None:
+                self.step_counter = torch.zeros((), dtype=torch.int64, device=current_dist.mean.device)
+            if not self.steps_on_device:
+                self.step_counter.fill_(self._global_steps)
+            entropy = pr.entropy_control(self.step_counter)
+        elif pr.initial_entropy is None:  # base_projection_layer.py:202-203
             pr.initial_entropy = policy.entropy((previous_dist.mean, previous_dist.var_diag)).mean().detach()
         advantage = td_get(td, "advantage")
         l_obj, l_tr, l_ent, sc = ops.trpl_loss(
@@ -110,7 +122,7 @@ class TRPLLoss(nn.Module):
             td_get(td, "sample_log_prob"), advantage, pr.mean_bound, pr.cov_bound, pr.KERNEL_TYPE,
             self.entropy_coef if self.entropy_bonus else 0.0, pr.trust_region_coeff,
             self.normalize_advantage and advantage.numel() * (1 if self.dp is None else self.dp.world_size) > 1,
-            None if self.dp is None else self.dp.all_gather_small)
+            None if self.dp is None else self.dp.all_gather_small, entropy)
         ix = _lib.LOSS_SCALAR_INDEX
         out = {"loss_objective": l_obj, "loss_trust_region": l_tr}
         if self.entropy_bonus:

@@ -65,7 +65,9 @@ class BaseProjectionLayer(object):
         self.entropy_first = entropy_first
         self.entropy_eq = entropy_eq
         self.temperature = temperature
+        self.total_train_steps = total_train_steps
         self._initial_entropy = None
+        self._entropy_state = None  # fused path: float64 [4] (initial_entropy, latched flag, bound, unused) on the device
 
     # ---- call protocol (base_projection_layer.py:199-273) ------------------------------------------
     def __call__(self, policy, p: Tuple[torch.Tensor, torch.Tensor], q, step, **kwargs):
@@ -105,6 +107,28 @@ class BaseProjectionLayer(object):
     def initial_entropy(self, entropy):
         if self.initial_entropy is None:
             self._initial_entropy = entropy
+
+    def entropy_state(self, device) -> torch.Tensor:
+        """The fused path's entropy-control state, created on first use.  An initial entropy the torch formulation has
+        already latched is carried over; from then on `initial_entropy` is a 0-dim view of the state."""
+        if self._entropy_state is None:
+            s = torch.zeros(4, dtype=torch.float64, device=device)
+            if self._initial_entropy is not None:
+                s[0] = self._initial_entropy.detach().to(device=device, dtype=torch.float64)
+                s[1] = 1.0
+            self._entropy_state = s
+            self._initial_entropy = s[0]
+        return self._entropy_state
+
+    def entropy_control(self, step: torch.Tensor) -> ops.EntropyControl:
+        """Arguments of ops.trpl_loss's entropy control; `step` is the int64 device step counter."""
+        return ops.EntropyControl(self.entropy_state(step.device), step, self._entropy_schedule_type, self.total_train_steps,
+                                  float(self.target_entropy), float(self.temperature), self.entropy_eq, self.entropy_first)
+
+    @property
+    def entropy_bound(self):
+        """Entropy bound of the latest fused call (0-dim device view, for logging); None before one has run."""
+        return None if self._entropy_state is None else self._entropy_state[2]
 
     def trust_region_value(self, policy, p, q):
         return gaussian_kl(policy, p, q)

@@ -12,6 +12,30 @@
 namespace grl {
 
 constexpr int kMaxK = GRL_MAX_ACTION_DIM;
+constexpr double kLog2Pi = 1.8378770664093454835606594728112;
+
+// Entropy projection of one sample (base_projection_layer.py:14-68): alpha = exp((beta - H(v)) / k) with
+// H(v) = 0.5 (k (1 + log 2pi) + 2 sum log v) ("std := v"), where H < beta (inequality) or always (equality); 1 elsewhere.
+__device__ __forceinline__ double entropy_alpha(const float* v, int k, int mode, double beta) {
+  double slog = 0.0;
+#pragma unroll
+  for (int i = 0; i < kMaxK; ++i)
+    if (i < k) slog += log((double)v[i]);
+  const double H = 0.5 * (k * (1.0 + kLog2Pi) + 2.0 * slog);
+  return (mode == GRL_ENTROPY_EQ || H < beta) ? exp((beta - H) / k) : 1.0;
+}
+
+// Vector-Jacobian product of v' = alpha(v) v: g_j <- alpha (g_j - sum_i g_i x_i / (k x_j)).  With x = v this is
+// alpha g_j - alpha / (k v_j) sum_i g_i v_i; x = v' gives the same value (alpha cancels).  beta is a constant.
+__device__ __forceinline__ void entropy_vjp(double* g, const double* x, int k, double alpha) {
+  double s = 0.0;
+#pragma unroll
+  for (int i = 0; i < kMaxK; ++i)
+    if (i < k) s += g[i] * x[i];
+#pragma unroll
+  for (int i = 0; i < kMaxK; ++i)
+    if (i < k) g[i] = alpha * (g[i] - s / (k * x[i]));
+}
 
 struct KlEval {
   double kl, dkl;
@@ -43,6 +67,8 @@ __device__ __forceinline__ KlEval kl_eval(const KlInv& q, int k, double eta) {
   return r;
 }
 
+// ENT: entropy control (d.entropy_mode != 0); the <false> instantiation is the plain trust-region projection.
+template <bool ENT>
 __global__ void __launch_bounds__(128) trpl_fwd_kernel(const GrlProjDesc d) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= d.batch) return;
@@ -58,6 +84,15 @@ __global__ void __launch_bounds__(128) trpl_fwd_kernel(const GrlProjDesc d) {
     } else {
       m[i] = mo[i] = 0.f;
       v[i] = vo[i] = 1.f;
+    }
+  }
+  double alpha = 1.0;
+  if constexpr (ENT) {
+    if (d.entropy_first) {  // the trust-region projection then starts from the entropy-projected v
+      alpha = entropy_alpha(v, k, d.entropy_mode, *d.entropy_beta);
+#pragma unroll
+      for (int i = 0; i < kMaxK; ++i)
+        if (i < k) v[i] = (float)(alpha * (double)v[i]);
     }
   }
   // ---- mean part ---------------------------------------------------------------------------
@@ -130,8 +165,21 @@ __global__ void __launch_bounds__(128) trpl_fwd_kernel(const GrlProjDesc d) {
     for (int i = 0; i < kMaxK; ++i)
       if (i < k) d.proj_v[(size_t)b * k + i] = active ? (v[i] + eta * vo[i]) / (1.0f + eta + 1e-16f) : v[i];
   }
+  if constexpr (ENT) {
+    if (!d.entropy_first) {  // entropy projection of the trust-region output (this thread's own stores)
+      float pv[kMaxK];
+#pragma unroll
+      for (int i = 0; i < kMaxK; ++i) pv[i] = i < k ? d.proj_v[(size_t)b * k + i] : 1.f;
+      alpha = entropy_alpha(pv, k, d.entropy_mode, *d.entropy_beta);
+#pragma unroll
+      for (int i = 0; i < kMaxK; ++i)
+        if (i < k) d.proj_v[(size_t)b * k + i] = (float)(alpha * (double)pv[i]);
+    }
+    d.entropy_alpha[b] = alpha;
+  }
 }
 
+template <bool ENT>
 __global__ void __launch_bounds__(128) trpl_bwd_kernel(const GrlProjDesc d) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= d.batch) return;
@@ -155,6 +203,30 @@ __global__ void __launch_bounds__(128) trpl_bwd_kernel(const GrlProjDesc d) {
     } else {
       m[i] = mo[i] = gm[i] = gv[i] = 0.0;
       v[i] = vo[i] = 1.0;
+    }
+  }
+  // ENT: gq = gradient w.r.t. the trust-region projection's input v, before grad_v_add
+  double alpha = 1.0, v_in[kMaxK], gq[kMaxK];
+  bool ent_active = false;
+  if constexpr (ENT) {
+    alpha = d.entropy_alpha[b];
+    ent_active = d.entropy_mode == GRL_ENTROPY_EQ || alpha > 1.0;  // inequality: alpha > 1 exactly where H < beta
+#pragma unroll
+    for (int i = 0; i < kMaxK; ++i) {
+      v_in[i] = v[i];
+      gq[i] = 0.0;
+    }
+    if (d.entropy_first) {
+      // the trust-region projection saw v' = alpha v, rounded as the forward rounded it
+#pragma unroll
+      for (int i = 0; i < kMaxK; ++i)
+        if (i < k) v[i] = (double)(float)(alpha * v[i]);
+    } else if (ent_active) {
+      // gradient reaching the trust-region output pv0 through pv = alpha(pv0) pv0 (evaluated at pv)
+      double pv[kMaxK];
+#pragma unroll
+      for (int i = 0; i < kMaxK; ++i) pv[i] = i < k ? (double)d.proj_v[(size_t)b * k + i] : 1.0;
+      entropy_vjp(gv, pv, k, alpha);
     }
   }
   // ---- mean: pm = (m + w mo) / (1 + w), w = sqrt(M / eps) - 1, M = scale * sum ((m - mo) / vo)^2
@@ -208,13 +280,17 @@ __global__ void __launch_bounds__(128) trpl_bwd_kernel(const GrlProjDesc d) {
       for (int i = 0; i < kMaxK; ++i)
         if (i < k) {
           const double gc = gct[i] * dct_dc[i] - num * (dkl_dct[i] * dct_dc[i]) / den;
-          d.grad_v[(size_t)b * k + i] = (float)(gc * 2.0 * v[i] + av[i]);
+          if constexpr (ENT) gq[i] = gc * 2.0 * v[i];
+          else d.grad_v[(size_t)b * k + i] = (float)(gc * 2.0 * v[i] + av[i]);
         }
     } else {
       // identity: pv = sqrt(v^2) = v
 #pragma unroll
       for (int i = 0; i < kMaxK; ++i)
-        if (i < k) d.grad_v[(size_t)b * k + i] = (float)(gv[i] + av[i]);
+        if (i < k) {
+          if constexpr (ENT) gq[i] = gv[i];
+          else d.grad_v[(size_t)b * k + i] = (float)(gv[i] + av[i]);
+        }
     }
   } else {
     if (eta > 0.0) {
@@ -226,14 +302,27 @@ __global__ void __launch_bounds__(128) trpl_bwd_kernel(const GrlProjDesc d) {
       const double deta_dS = 1.0 / (2.0 * (double)d.eps_cov * (1.0 + eta));
 #pragma unroll
       for (int i = 0; i < kMaxK; ++i)
-        if (i < k)
-          d.grad_v[(size_t)b * k + i] =
-              (float)(gv[i] / (1.0 + eta) + dot * deta_dS * 2.0 * (v[i] / vo[i] - 1.0) / vo[i] + av[i]);
+        if (i < k) {
+          if constexpr (ENT) gq[i] = gv[i] / (1.0 + eta) + dot * deta_dS * 2.0 * (v[i] / vo[i] - 1.0) / vo[i];
+          else
+            d.grad_v[(size_t)b * k + i] =
+                (float)(gv[i] / (1.0 + eta) + dot * deta_dS * 2.0 * (v[i] / vo[i] - 1.0) / vo[i] + av[i]);
+        }
     } else {
 #pragma unroll
       for (int i = 0; i < kMaxK; ++i)
-        if (i < k) d.grad_v[(size_t)b * k + i] = (float)(gv[i] + av[i]);
+        if (i < k) {
+          if constexpr (ENT) gq[i] = gv[i];
+          else d.grad_v[(size_t)b * k + i] = (float)(gv[i] + av[i]);
+        }
     }
+  }
+  if constexpr (ENT) {
+    // entropy first: chain through v' = alpha(v) v at the original v; grad_v_add reaches the original v after it
+    if (d.entropy_first && ent_active) entropy_vjp(gq, v_in, k, alpha);
+#pragma unroll
+    for (int i = 0; i < kMaxK; ++i)
+      if (i < k) d.grad_v[(size_t)b * k + i] = (float)(gq[i] + av[i]);
   }
 }
 
@@ -242,8 +331,6 @@ __global__ void __launch_bounds__(128) trpl_bwd_kernel(const GrlProjDesc d) {
 // Loss terms around the projection (objectives/trpl.py:231-321, base_projection_layer.py:292-384).
 // terms[b] = { log_w, tr_mean, tr_cov, kl_mean + kl_cov, H_dist(proj), H_policy(p), H_policy(proj), advantage }
 // ---------------------------------------------------------------------------------------------------
-constexpr double kLog2Pi = 1.8378770664093454835606594728112;
-
 __global__ void __launch_bounds__(128) trpl_loss_terms_kernel(const GrlLossDesc d) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= d.batch) return;
@@ -304,6 +391,33 @@ __device__ __forceinline__ double block_max(double x, double* sh) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) x = fmax(x, __shfl_xor_sync(0xffffffffu, x, o));
   return x;
+}
+
+// Scheduled entropy bound (see grl_trpl_entropy_bound in grl_b200.h).  Stage 1 needs the whole CTA (block_sum);
+// stage 2 is one thread.  The sum runs over samples in a fixed order, so the bound is bit-reproducible.
+__global__ void __launch_bounds__(kLossThreads) trpl_entropy_bound_kernel(const GrlEntropyBoundDesc d) {
+  __shared__ double sh[32];
+  const int B = d.batch, k = d.k, tid = threadIdx.x;
+  if (d.stage != 2) {
+    double s = 0.0;
+    for (int b = tid; b < B; b += blockDim.x) {
+      double slog = 0.0;
+      for (int i = 0; i < k; ++i) slog += log((double)d.old_v[(size_t)b * k + i]);
+      s += 0.5 * (k * (1.0 + kLog2Pi) + 2.0 * slog);  // policy.entropy(q), gnn_gaussian_policy_diag.py:116-122
+    }
+    s = block_sum(s, sh);
+    if (tid == 0) { d.sums[0] = s; d.sums[1] = (double)B; }
+  }
+  if (d.stage != 1 && tid == 0) {
+    double* S = d.state;
+    if (S[1] == 0.0) {  // base_projection_layer.py:202-203: latched on the first call, detached
+      S[0] = d.sums[0] / d.sums[1];
+      S[1] = 1.0;
+    }
+    const double ie = S[0], te = d.target_entropy, step = (double)*d.step, T = (double)d.total_train_steps;
+    S[2] = d.schedule == GRL_ENTROPY_LINEAR ? step * (te - ie) / T + ie
+                                            : k * te + (ie - k * te) * pow(d.temperature, 10.0 * step / T);
+  }
 }
 
 // Data parallel: out[i] = sum_r gathered[r][i] (i < n_sum) | max_r gathered[r][i] (i >= n_sum), ranks visited in rank
@@ -455,21 +569,52 @@ static int check_proj(const GrlProjDesc* d, const char* who, bool bwd) {
   GRL_REQUIRE(d->mean && d->v && d->old_mean && d->old_v && d->eta, GRL_EINVAL, "%s: null pointer", who);
   if (bwd) GRL_REQUIRE(d->grad_proj_mean && d->grad_proj_v && d->grad_mean && d->grad_v, GRL_EINVAL, "%s: null grad pointer", who);
   else GRL_REQUIRE(d->proj_mean && d->proj_v, GRL_EINVAL, "%s: null output pointer", who);
+  GRL_REQUIRE(d->entropy_mode >= GRL_ENTROPY_OFF && d->entropy_mode <= GRL_ENTROPY_EQ, GRL_EUNSUPPORTED,
+              "%s: entropy_mode=%d", who, d->entropy_mode);
+  GRL_REQUIRE(d->entropy_first == 0 || (d->entropy_first == 1 && d->entropy_mode != GRL_ENTROPY_OFF), GRL_EINVAL,
+              "%s: entropy_first=%d with entropy_mode=%d", who, d->entropy_first, d->entropy_mode);
+  if (d->entropy_mode != GRL_ENTROPY_OFF) {
+    GRL_REQUIRE(d->entropy_alpha && (bwd || d->entropy_beta), GRL_EINVAL, "%s: null entropy pointer", who);
+    if (bwd && !d->entropy_first) GRL_REQUIRE(d->proj_v, GRL_EINVAL, "%s: entropy projection after: null proj_v", who);
+  }
   return GRL_OK;
 }
 
 int grl_trpl_fwd(const GrlProjDesc* d, grl_stream_t stream) {
   const int rc = check_proj(d, "grl_trpl_fwd", false);
   if (rc != GRL_OK) return rc;
-  grl::trpl_fwd_kernel<<<(d->batch + 127) / 128, 128, 0, (cudaStream_t)stream>>>(*d);
+  if (d->entropy_mode == GRL_ENTROPY_OFF)
+    grl::trpl_fwd_kernel<false><<<(d->batch + 127) / 128, 128, 0, (cudaStream_t)stream>>>(*d);
+  else
+    grl::trpl_fwd_kernel<true><<<(d->batch + 127) / 128, 128, 0, (cudaStream_t)stream>>>(*d);
   return grl::check_launch("grl_trpl_fwd");
 }
 
 int grl_trpl_bwd(const GrlProjDesc* d, grl_stream_t stream) {
   const int rc = check_proj(d, "grl_trpl_bwd", true);
   if (rc != GRL_OK) return rc;
-  grl::trpl_bwd_kernel<<<(d->batch + 127) / 128, 128, 0, (cudaStream_t)stream>>>(*d);
+  if (d->entropy_mode == GRL_ENTROPY_OFF)
+    grl::trpl_bwd_kernel<false><<<(d->batch + 127) / 128, 128, 0, (cudaStream_t)stream>>>(*d);
+  else
+    grl::trpl_bwd_kernel<true><<<(d->batch + 127) / 128, 128, 0, (cudaStream_t)stream>>>(*d);
   return grl::check_launch("grl_trpl_bwd");
+}
+
+int grl_trpl_entropy_bound(const GrlEntropyBoundDesc* d, grl_stream_t stream) {
+  const char* who = "grl_trpl_entropy_bound";
+  GRL_REQUIRE(d, GRL_EINVAL, "%s: null descriptor", who);
+  GRL_REQUIRE(d->batch > 0 && d->k > 0, GRL_EINVAL, "%s: batch=%d k=%d", who, d->batch, d->k);
+  GRL_REQUIRE(d->k <= GRL_MAX_ACTION_DIM, GRL_EUNSUPPORTED, "%s: k=%d > %d", who, d->k, GRL_MAX_ACTION_DIM);
+  GRL_REQUIRE(d->schedule == GRL_ENTROPY_LINEAR || d->schedule == GRL_ENTROPY_EXP, GRL_EUNSUPPORTED,
+              "%s: schedule=%d", who, d->schedule);
+  GRL_REQUIRE(d->stage >= 0 && d->stage <= 2, GRL_EINVAL, "%s: stage=%d", who, d->stage);
+  GRL_REQUIRE(d->total_train_steps > 0, GRL_EINVAL, "%s: total_train_steps=%lld", who, (long long)d->total_train_steps);
+  GRL_REQUIRE(d->schedule != GRL_ENTROPY_EXP || d->temperature > 0.0, GRL_EINVAL, "%s: temperature=%g for exp", who,
+              d->temperature);
+  GRL_REQUIRE(d->step && d->sums && d->state && (d->stage == 2 || d->old_v), GRL_EINVAL, "%s: null pointer", who);
+  const int threads = d->stage == 2 ? 32 : grl::kLossThreads;
+  grl::trpl_entropy_bound_kernel<<<1, threads, 0, (cudaStream_t)stream>>>(*d);
+  return grl::check_launch(who);
 }
 
 static int check_loss(const GrlLossDesc* d, const char* who, bool bwd) {

@@ -72,8 +72,9 @@ def policy_in_keys(cfg: PathConfig):
     return keys
 
 
-def build_agent(cfg: PathConfig, device, proj_type: str = "kl", seed: int = 0):
-    """-> (actor PolicyOperator, critic ValueOperator, projection, loss_module, adv_module)."""
+def build_agent(cfg: PathConfig, device, proj_type: str = "kl", seed: int = 0, projection_kwargs=None):
+    """-> (actor PolicyOperator, critic ValueOperator, projection, loss_module, adv_module).  `projection_kwargs` override
+    the projection layer's keywords, e.g. dict(entropy_schedule="linear", target_entropy=-2.0) for entropy control."""
     torch.manual_seed(seed)
     m, _ = _task_module(cfg)
     body = make_policy_body(cfg, device)
@@ -90,11 +91,12 @@ def build_agent(cfg: PathConfig, device, proj_type: str = "kl", seed: int = 0):
     critic_net = BaseCritic(vf).to(device)
     actor = PolicyOperator(policy, policy_in_keys(cfg))
     critic = ValueOperator(critic_net, obs_keys(cfg))
-    projection = get_projection_layer(proj_type=proj_type, mean_bound=cfg.mean_bound, cov_bound=cfg.cov_bound,
-                                      trust_region_coeff=cfg.trust_region_coeff, scale_prec=True,
-                                      entropy_schedule=False, target_entropy=0.0, temperature=0.5, entropy_eq=False,
-                                      entropy_first=False, action_dim=cfg.total_action_dim, total_train_steps=1000,
-                                      cpu=False, dtype=torch.float32)
+    pkw = dict(mean_bound=cfg.mean_bound, cov_bound=cfg.cov_bound, trust_region_coeff=cfg.trust_region_coeff,
+               scale_prec=True, entropy_schedule=False, target_entropy=0.0, temperature=0.5, entropy_eq=False,
+               entropy_first=False, action_dim=cfg.total_action_dim, total_train_steps=1000, cpu=False,
+               dtype=torch.float32)
+    pkw.update(projection_kwargs or {})
+    projection = get_projection_layer(proj_type=proj_type, **pkw)
     loss_module = TRPLLoss(actor, critic, projection=projection, clip_epsilon=0.2, entropy_bonus=True,
                            entropy_coef=cfg.entropy_coef, critic_coef=cfg.critic_coef, loss_critic_type="l2",
                            normalize_advantage=True, clip_value=cfg.clip_value)
@@ -132,6 +134,18 @@ class Learner:
         if dp is not None:
             dp.attach(loss_module)
             dp.sync_module_state(actor, critic)  # replicas start bit-identical whatever each rank's RNG did
+        # entropy control: the step the bound is scheduled on lives on the device and every update advances it there, so
+        # a captured update replays with the right step; `num_network_updates` is its host mirror
+        self._step = None
+        if getattr(loss_module.projection, "has_entropy_control", False):
+            self._step = torch.zeros((), dtype=torch.int64, device=self._params[0].device)
+            loss_module.step_counter, loss_module.steps_on_device = self._step, True
+
+    def set_step(self, n: int):
+        """Resume at `n` network updates (host counter and the device step of the entropy bound)."""
+        self.num_network_updates = int(n)
+        if self._step is not None:
+            self._step.fill_(int(n))
 
     def compute_losses(self, batch) -> Dict[str, torch.Tensor]:
         self.loss_module._global_steps = self.num_network_updates
@@ -181,6 +195,8 @@ class Learner:
         self.critic_optim.step()
         self.actor_optim.zero_grad()
         self.critic_optim.zero_grad()
+        if self._step is not None:
+            self._step.add_(1)
         return loss
 
 
@@ -212,6 +228,8 @@ class Learner:
         self.critic_optim.step()
         self.actor_optim.zero_grad()
         self.critic_optim.zero_grad()
+        if self._step is not None:
+            self._step.add_(1)
         return loss
 
     # ---- CUDA-graph replay of the whole update (launch-bound glue: ~500 launches per step) -----------------------
@@ -222,7 +240,10 @@ class Learner:
         parameters and optimiser state are put back afterwards, so the first replayed minibatch is the first update the
         networks see, as in the reference loop (train.py:259-316).  The one-time calibration runs BEFORE the snapshot:
         it belongs to the first forward, not to the warm-up.  The captured graph bakes in Python-side scalars (Adam's lr,
-        `loss_module._global_steps`): lr annealing or an entropy schedule would be frozen, so capture refuses them.
+        `loss_module._global_steps`): lr annealing would be frozen.  An entropy schedule is captured on the fused loss
+        path, which reads the step from the learner's device counter; `restore` then also puts back that counter and the
+        projection's latched initial entropy, so the first replayed minibatch latches it.  The torch formulation reads the
+        host step and is refused.
         The graph also holds the topology tensors of this batch size: re-capture after `hyper_data.invalidate()`.  With
         `hyper_data.rebuild_every_call` the data builder must refresh its topology in place (`refresh_in_place()`): every
         replay then rebuilds the kNN or radius graph from the static inputs' positions; any other rebuild mode is refused."""
@@ -238,10 +259,10 @@ class Learner:
                         "`hyper_data.knn_in_place = True` (HEPi rope: any precision; HEPi rigid and EMPN: fused 16-bit "
                         "path) and, for HEPi, radius INTERNAL edges on the fused 16-bit path (internal_edges='radius', "
                         "ops.set_precision('bf16')) - otherwise use `update`")
-        proj = getattr(self.loss_module, "projection", None)
-        if getattr(proj, "entropy_schedule", False):
-            raise NotImplementedError("an entropy schedule depends on the host-side step counter, which a captured graph "
-                                      "freezes; use the eager `update`")
+        proj = self.loss_module.projection
+        if self._step is not None and not self.loss_module._can_fuse(self.actor.get_submodule("0").module):
+            raise NotImplementedError("an entropy schedule on the torch loss formulation depends on the host-side step "
+                                      "counter, which a captured graph freezes; use the fused loss or the eager `update`")
         # data-parallel: the NCCL all-reduces of the step are captured too (torch's ProcessGroupNCCL records them on the
         # capture stream); every rank must capture and replay in lock-step
         self._static = {k: v.clone() for k, v in example_batch.items() if torch.is_tensor(v)}
@@ -252,6 +273,8 @@ class Learner:
             import copy
             saved_opt = [copy.deepcopy(o.state_dict()) for o in (self.actor_optim, self.critic_optim)]
             saved_n = self.num_network_updates
+            if self._step is not None:
+                saved_ent = [t.clone() for t in (self._step, proj.entropy_state(self._step.device))]
         side = torch.cuda.Stream()
         side.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(side):
@@ -273,6 +296,9 @@ class Learner:
                             if torch.is_tensor(v):
                                 v.zero_()
             self.num_network_updates = saved_n
+            if self._step is not None:
+                for t, s_ in zip((self._step, proj.entropy_state(self._step.device)), saved_ent):
+                    t.copy_(s_)
         self._graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self._graph):
             self._graph_out = self.update(self._static)

@@ -7,7 +7,7 @@ eager fallback — tensors must live on a CUDA device.
 import ctypes as C
 import os
 from dataclasses import dataclass
-from typing import Optional
+from typing import NamedTuple, Optional
 
 import torch
 
@@ -1219,17 +1219,30 @@ class TrplLossFn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, mean, v, old_mean, old_v, action, prev_log_prob, advantage, eps_mean, eps_cov, proj_type,
-                entropy_coef, trust_region_coeff, normalize_advantage, all_reduce=None):
+                entropy_coef, trust_region_coeff, normalize_advantage, all_reduce=None, entropy=None):
         mean, v, old_mean, old_v = _f32c(mean), _f32c(v), _f32c(old_mean), _f32c(old_v)
         action, prev_log_prob, advantage = _f32c(action), _f32c(prev_log_prob).reshape(-1), _f32c(advantage).reshape(-1)
         B, k = mean.shape
         assert action.shape == (B, k) and prev_log_prob.numel() == B and advantage.numel() == B
         dev = mean.device
+        make_global = None
+        if all_reduce is not None:
+            # data parallel: `all_reduce` is the hook `gather(tensor[n]) -> [world, n]` (one all-gather); the slice is then
+            # combined in rank order by grl_dp_combine (sums first, maxima last): ONE collective per stage, deterministic
+            def make_global(buf, lo, hi, n_sum):
+                g = all_reduce(buf[lo:hi])
+                L.call("grl_dp_combine", L.ptr_any(g), g.shape[0], hi - lo, n_sum, buf[lo:hi].data_ptr())
         pm, pv = torch.empty_like(mean), torch.empty_like(v)
         eta = torch.empty(B, 2, dtype=torch.float64, device=dev)
         d = L.GrlProjDesc(batch=B, k=k, proj_type=proj_type, eps_mean=float(eps_mean), eps_cov=float(eps_cov),
                           mean=L.ptr(mean), v=L.ptr(v), old_mean=L.ptr(old_mean), old_v=L.ptr(old_v), proj_mean=L.ptr(pm),
                           proj_v=L.ptr(pv), eta=L.ptr_any(eta))
+        alpha = None
+        if entropy is not None:
+            alpha = torch.empty(B, dtype=torch.float64, device=dev)
+            d.entropy_mode = entropy_bound(entropy, old_v, make_global)
+            d.entropy_first = int(bool(entropy.first))
+            d.entropy_beta, d.entropy_alpha = L.ptr_any(entropy.state[2:3]), L.ptr(alpha)
         L.call("grl_trpl_fwd", C.byref(d))
         terms = torch.empty(B, L.LOSS_TERMS, dtype=torch.float64, device=dev)
         stats = torch.empty(L.LOSS_STATS, dtype=torch.float64, device=dev)
@@ -1243,11 +1256,6 @@ class TrplLossFn(torch.autograd.Function):
         if all_reduce is None:
             L.call("grl_trpl_loss_fwd", C.byref(ld))
         else:
-            # data parallel: `all_reduce` is the hook `gather(tensor[n]) -> [world, n]` (one all-gather); the slice is then
-            # combined in rank order by grl_dp_combine (sums first, maxima last): ONE collective per stage, deterministic
-            def make_global(buf, lo, hi, n_sum):
-                g = all_reduce(buf[lo:hi])
-                L.call("grl_dp_combine", L.ptr_any(g), g.shape[0], hi - lo, n_sum, buf[lo:hi].data_ptr())
             ld.stage = 1
             L.call("grl_trpl_loss_fwd", C.byref(ld))
             make_global(stats, 0, 4, 3)
@@ -1256,15 +1264,16 @@ class TrplLossFn(torch.autograd.Function):
             make_global(sums, 3, 12, 7)
             ld.stage = 3
             L.call("grl_trpl_loss_fwd", C.byref(ld))
-        ctx.save_for_backward(mean, v, old_mean, old_v, action, pm, pv, eta, terms, stats)
-        ctx.meta = (float(eps_mean), float(eps_cov), proj_type, float(entropy_coef), float(trust_region_coeff))
+        ctx.save_for_backward(mean, v, old_mean, old_v, action, pm, pv, eta, terms, stats, alpha)
+        ctx.meta = (float(eps_mean), float(eps_cov), proj_type, float(entropy_coef), float(trust_region_coeff),
+                    d.entropy_mode, d.entropy_first)
         ctx.mark_non_differentiable(scalars)
         return scalars[0].clone(), scalars[1].clone(), scalars[2].clone(), scalars
 
     @staticmethod
     def backward(ctx, g_obj, g_tr, g_ent, _g_scalars):
-        mean, v, old_mean, old_v, action, pm, pv, eta, terms, stats = ctx.saved_tensors
-        eps_mean, eps_cov, proj_type, entropy_coef, trust_region_coeff = ctx.meta
+        mean, v, old_mean, old_v, action, pm, pv, eta, terms, stats, alpha = ctx.saved_tensors
+        eps_mean, eps_cov, proj_type, entropy_coef, trust_region_coeff, ent_mode, ent_first = ctx.meta
         B, k = mean.shape
         dev = mean.device
         zero = torch.zeros((), dtype=torch.float32, device=dev)
@@ -1282,15 +1291,50 @@ class TrplLossFn(torch.autograd.Function):
                           v=L.ptr(v), old_mean=L.ptr(old_mean), old_v=L.ptr(old_v), eta=L.ptr_any(eta),
                           grad_proj_mean=L.ptr(g_pm), grad_proj_v=L.ptr(g_pv), grad_mean=L.ptr(gm), grad_v=L.ptr(gv),
                           grad_mean_add=L.ptr(g_md), grad_v_add=L.ptr(g_vd))
+        if ent_mode:
+            d.entropy_mode, d.entropy_first, d.entropy_alpha, d.proj_v = ent_mode, ent_first, L.ptr(alpha), L.ptr(pv)
         L.call("grl_trpl_bwd", C.byref(d))
-        return (gm, gv) + (None,) * 12
+        return (gm, gv) + (None,) * 13
+
+
+class EntropyControl(NamedTuple):
+    """TRPL entropy control on the fused path (base_projection_layer.py:14-68,199-273, projection_utils.py:252-280)."""
+    state: torch.Tensor  # float64 [4] (initial_entropy, latched flag, bound of the latest call, unused), on the device
+    step: torch.Tensor  # int64 0-dim device tensor: network updates so far
+    schedule: str  # "linear" | "exp"
+    total_train_steps: int
+    target_entropy: float
+    temperature: float
+    equality: bool  # entropy_eq: project onto H = beta; otherwise only where H < beta
+    first: bool  # entropy_first: entropy projection before the trust-region projection
+
+
+def entropy_bound(ent: EntropyControl, old_v, make_global=None) -> int:
+    """Latch ent.state[0] = mean policy.entropy(old) on the first call and write this step's bound to ent.state[2], on the
+    device (grl_trpl_entropy_bound).  `make_global(buf, lo, hi, n_sum)`: the data-parallel combine of the entropy sum
+    between the two stages.  Returns the GrlProjDesc.entropy_mode of `ent`."""
+    if ent.state.dtype != torch.float64 or ent.state.numel() != 4 or ent.step.dtype != torch.int64 or ent.step.numel() != 1:
+        raise ValueError("entropy control: state must be float64 [4] and step an int64 scalar")
+    old_v = _f32c(old_v)
+    sums = torch.empty(2, dtype=torch.float64, device=old_v.device)
+    d = L.GrlEntropyBoundDesc(batch=old_v.shape[0], k=old_v.shape[1], schedule=L.ENTROPY_SCHEDULE.get(ent.schedule, 0),
+                              stage=0 if make_global is None else 1, total_train_steps=int(ent.total_train_steps),
+                              target_entropy=float(ent.target_entropy), temperature=float(ent.temperature),
+                              old_v=L.ptr(old_v), step=L.ptr_any(ent.step), sums=L.ptr(sums), state=L.ptr(ent.state))
+    L.call("grl_trpl_entropy_bound", C.byref(d))
+    if make_global is not None:
+        make_global(sums, 0, 2, 2)
+        d.stage = 2
+        L.call("grl_trpl_entropy_bound", C.byref(d))
+    return L.ENTROPY_MODE["eq" if ent.equality else "ineq"]
 
 
 def trpl_loss(mean, v, old_mean, old_v, action, prev_log_prob, advantage, eps_mean, eps_cov, proj_type, entropy_coef,
-              trust_region_coeff, normalize_advantage=True, all_reduce=None):
+              trust_region_coeff, normalize_advantage=True, all_reduce=None, entropy: Optional[EntropyControl] = None):
     """-> (loss_objective, loss_trust_region, loss_entropy, scalars) with scalars indexed by _lib.LOSS_SCALAR_INDEX.
     `all_reduce` (data parallel, equal shards) = the hook `gather(tensor[n]) -> [world, n]`: advantage statistics, ESS and
-    metrics become global, the three losses are this rank's share (local sum / global count)."""
+    metrics become global, the three losses are this rank's share (local sum / global count).
+    `entropy`: entropy control; the bound is computed on the device before the projection (global under `all_reduce`)."""
     code = {"kl": 0, "w2": 1}[proj_type]
     return TrplLossFn.apply(mean, v, old_mean, old_v, action, prev_log_prob, advantage, eps_mean, eps_cov, code,
-                            entropy_coef, trust_region_coeff, normalize_advantage, all_reduce)
+                            entropy_coef, trust_region_coeff, normalize_advantage, all_reduce, entropy)

@@ -540,9 +540,44 @@ typedef struct {
   float* grad_v;               /* [B][k]                                                        */
   const float* grad_mean_add;  /* optional [B][k]: added to grad_mean (gradient reaching `mean` directly)   */
   const float* grad_v_add;     /* optional [B][k]: added to grad_v                                          */
+  /* entropy control (base_projection_layer.py:14-68,199-273); all zero = off, the launch is the plain projection.
+   * alpha = exp((beta - H(v)) / k), H(v) = 0.5 (k (1 + log 2 pi) + 2 sum log v), v <- alpha v, mean unchanged.
+   * Applied after the trust-region projection, or before it with entropy_first.  The backward reads alpha and,
+   * when entropy_first is 0, proj_v. */
+  int32_t entropy_mode;        /* GRL_ENTROPY_OFF | _INEQ (only where H < beta) | _EQ (always)                      */
+  int32_t entropy_first;       /* 0 | 1 (needs entropy_mode != 0)                                                  */
+  const double* entropy_beta;  /* device scalar: the bound (grl_trpl_entropy_bound state[2]); forward only          */
+  double* entropy_alpha;       /* [B] forward writes alpha (1 where inactive), backward reads it                    */
 } GrlProjDesc;
+#define GRL_ENTROPY_OFF 0
+#define GRL_ENTROPY_INEQ 1
+#define GRL_ENTROPY_EQ 2
 int grl_trpl_fwd(const GrlProjDesc* d, grl_stream_t stream);
 int grl_trpl_bwd(const GrlProjDesc* d, grl_stream_t stream);
+
+/* Scheduled entropy bound (base_projection_layer.py:199-203, utils/projection_utils.py:252-280) on the device.
+ *   stage 1  sums[0] = sum_b H(old_v_b) (fp64, fixed order, no atomics), sums[1] = batch
+ *   stage 2  first call only (state[1] == 0): state[0] = sums[0] / sums[1], state[1] = 1; then with s = *step,
+ *            T = total_train_steps, ie = state[0], te = target_entropy:
+ *              linear  state[2] = s (te - ie) / T + ie
+ *              exp     state[2] = k te + (ie - k te) temperature^(10 s / T)
+ *   stage 0  both.  Data parallel: all-gather sums between the stages and grl_dp_combine them (n = n_sum = 2), so
+ *            every rank latches the global mean and holds a bit-identical bound. */
+#define GRL_ENTROPY_LINEAR 1
+#define GRL_ENTROPY_EXP 2
+typedef struct {
+  int32_t batch, k;
+  int32_t schedule;           /* GRL_ENTROPY_LINEAR | GRL_ENTROPY_EXP                                     */
+  int32_t stage;              /* 0 = stages 1 and 2, else 1 | 2                                           */
+  int64_t total_train_steps;  /* > 0                                                                      */
+  double target_entropy;
+  double temperature;         /* > 0 for exp                                                              */
+  const float* old_v;         /* [B][k] old policy's "std" diagonal                                       */
+  const int64_t* step;        /* device scalar: network updates so far                                    */
+  double* sums;               /* [2] (sum H, n) workspace between the stages                             */
+  double* state;              /* [4] (initial_entropy, latched flag, bound, unused): owned by the caller  */
+} GrlEntropyBoundDesc;
+int grl_trpl_entropy_bound(const GrlEntropyBoundDesc* d, grl_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------
  * L1/P3  TRPL loss terms around the projection: replaces the ~170 elementwise / reduction launches of
