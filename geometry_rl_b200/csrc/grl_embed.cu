@@ -189,7 +189,8 @@ int grl_embed_fwd(const GrlEmbedDesc* d, grl_stream_t stream) {
 int grl_embed_bwd(const GrlEmbedDesc* d, grl_stream_t stream) {
   const int rc = check_embed(d, "grl_embed_bwd");
   if (rc != GRL_OK) return rc;
-  GRL_REQUIRE(d->grad_x && d->grad_weight_partials && d->n_partials > 0, GRL_EINVAL, "grl_embed_bwd: null pointer");
+  GRL_REQUIRE(d->grad_x && d->grad_weight_partials && d->n_partials > 0, GRL_EINVAL,
+              "grl_embed_bwd: null pointer or n_partials=%d", d->n_partials);
   const int fq = (d->n_scalars + d->n_vectors + 3) / 4;
   cudaStream_t st = (cudaStream_t)stream;
   if (fq == 1) grl::embed_bwd_kernel<1><<<d->n_partials, grl::kThreads, 0, st>>>(*d);

@@ -23,6 +23,15 @@ __device__ __forceinline__ float warp_sum(float v) {
   return v;
 }
 
+// mean_o ori[o][d], the factor of b_j in the vector readout.  On a symmetric grid (the 2-D circle) the mean is ~1e-8
+// while the partial sums of an fp32 loop reach ~5 and leave ~1e-7 of rounding, which b_j * mean would add to every
+// output and bias gradient; summed in double, the mean is the float nearest the exact one.
+__device__ __forceinline__ float orientation_mean(const float (&ori)[kO][3], int d) {
+  double a = 0.0;
+  for (int o = 0; o < kO; ++o) a += ori[o][d];
+  return (float)(a / kO);
+}
+
 struct ReadoutRow {
   float2 hid;     // hidden of channels 2l, 2l+1
   float2 V[3];    // V[c][d]
@@ -51,11 +60,7 @@ __global__ void __launch_bounds__(256) readout_fwd_kernel(const GrlReadoutDesc d
   __shared__ float s_obar[3];
   if (threadIdx.x < kO * 3) s_ori[threadIdx.x / 3][threadIdx.x % 3] = d.ori[threadIdx.x];
   __syncthreads();
-  if (threadIdx.x < 3) {
-    float a = 0.f;
-    for (int o = 0; o < kO; ++o) a += s_ori[o][threadIdx.x];
-    s_obar[threadIdx.x] = a / kO;
-  }
+  if (threadIdx.x < 3) s_obar[threadIdx.x] = orientation_mean(s_ori, threadIdx.x);
   __syncthreads();
   float ori[kO][3];
 #pragma unroll
@@ -99,11 +104,7 @@ __global__ void __launch_bounds__(256) readout_bwd_kernel(const GrlReadoutDesc d
   if (threadIdx.x < kO * 3) s_ori[threadIdx.x / 3][threadIdx.x % 3] = d.ori[threadIdx.x];
   for (int i = threadIdx.x; i < 8 * (kMaxJ * kC + kMaxJ); i += blockDim.x) (&s_gw[0][0])[i] = 0.f;
   __syncthreads();
-  if (threadIdx.x < 3) {
-    float a = 0.f;
-    for (int o = 0; o < kO; ++o) a += s_ori[o][threadIdx.x];
-    s_obar[threadIdx.x] = a / kO;
-  }
+  if (threadIdx.x < 3) s_obar[threadIdx.x] = orientation_mean(s_ori, threadIdx.x);
   __syncthreads();
   float ori[kO][3];
 #pragma unroll
@@ -191,7 +192,9 @@ static int check_readout(const GrlReadoutDesc* d, const char* who, bool bwd) {
               GRL_EUNSUPPORTED, "%s: od=%d odv=%d (need od == odv or od == 1, od + odv <= %d)", who, d->od, d->odv,
               GRL_READOUT_MAX_OUT);
   GRL_REQUIRE(d->latent && d->weight && d->bias && d->ori, GRL_EINVAL, "%s: null pointer", who);
-  if (bwd) GRL_REQUIRE(d->grad_out && d->grad_latent && d->grad_partials && d->n_partials > 0, GRL_EINVAL, "%s: null grad pointer", who);
+  if (bwd)
+    GRL_REQUIRE(d->grad_out && d->grad_latent && d->grad_partials && d->n_partials > 0, GRL_EINVAL,
+                "%s: null grad pointer or n_partials=%d", who, d->n_partials);
   else GRL_REQUIRE(d->out && d->hidden, GRL_EINVAL, "%s: null output pointer", who);
   return GRL_OK;
 }
